@@ -5,6 +5,7 @@
     python bench.py --workload c3|c4|c5 [...]                       # the other BASELINE.json configs
     python bench.py --scaling strong [...]                          # c2/c5: ONE sequence split over the ranks
     python bench.py --impl reference [...]                          # the reference's CPU path, host cores
+    python bench.py --dump-outputs DIR [...]                        # also write the last timed step's outputs
 
 Workloads (BASELINE.json configs[1..4], made concrete in SURVEY.md §8(d)); inputs are the tensors the
 path sees after the backbone: saliency maps (T,H,W,1) fp32 and NHWC feature maps (T,H/16,W/16,384) fp32.
@@ -93,7 +94,12 @@ def parse():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-eager-baseline", action="store_true")
     ap.add_argument("--no-graph", action="store_true", help="launch the step eagerly instead of replaying a CUDA graph")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/<name>.npy (see dump_outputs); with "
+                         "several ranks: rank 0's frames and the match lists of all ranks gathered on rank 0")
     a = ap.parse_args()
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl b200)")
     w = WORKLOADS[a.workload]
     a.H, a.W, a.kind = w["H"], w["W"], w["kind"]
     a.frames = a.frames or w["frames"]
@@ -266,6 +272,57 @@ def make_inputs(a, plan, pinned=True):
         sal[i, :, :, 0].copy_(torch.sigmoid(lg))
         feat[i].copy_(ft)
     return sal, feat
+
+
+DUMP_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(path, per_frame, per_pair, descriptors):
+    """--dump-outputs: the outputs of the last timed step as <path>/<name>.npy, all float32 (the integer
+    outputs are exact there: |value| < 2**24).  Inputs and weights are seeded, so two builds run with the
+    same arguments can be compared file for file.
+
+    per_frame / per_pair: name -> tensor whose first axis runs over the frames / the pairs;
+    descriptors: (frames, K, D).  The files stay under DUMP_BYTES in all.  The per-pair arrays, then the
+    per-frame arrays, are kept whole when they fit an equal share of what is left; otherwise every array
+    of that group keeps the same fixed, seeded sample of its rows, whose indices go to pair_rows.npy /
+    frame_rows.npy (float64).  The descriptors fill the rest: a seeded sample of the (frame, keypoint)
+    rows of the kept frames, written as descriptors.npy (n, D) with descriptor_rows.npy holding
+    frame * K + keypoint."""
+    import numpy as np
+    import torch
+    os.makedirs(path, exist_ok=True)
+    left = DUMP_BYTES - 256 * (2 * (len(per_frame) + len(per_pair)) + 4)     # room for the .npy headers
+
+    def sample(n, keep):
+        return np.sort(np.random.Generator(np.random.PCG64(0)).choice(n, keep, replace=False))
+
+    def save(name, arr):
+        np.save(os.path.join(path, name + ".npy"), arr)
+        return arr.nbytes
+
+    def put(group, arrays, share):
+        rows = next(iter(arrays.values())).shape[0]
+        row_bytes = sum(4 * t.numel() // max(rows, 1) for t in arrays.values())
+        idx, used = np.arange(rows), 0
+        if rows * row_bytes > share:
+            idx = sample(rows, min(rows, share // (row_bytes + 8)))
+            used += save(group + "_rows", idx.astype(np.float64))
+        sel = torch.from_numpy(idx)
+        for name, t in arrays.items():
+            used += save(name, t.index_select(0, sel.to(t.device)).float().cpu().numpy())
+        return idx, used
+
+    _, used = put("pair", per_pair, left // 3)
+    left -= used
+    frames, used = put("frame", per_frame, left // 2)
+    left -= used
+    F, K, D = descriptors.shape
+    cand = (frames[:, None] * K + np.arange(K)[None, :]).ravel()
+    rows = cand[sample(cand.size, min(cand.size, left // (4 * D + 8)))]
+    save("descriptor_rows", rows.astype(np.float64))
+    flat = descriptors.reshape(F * K, D)
+    save("descriptors", flat.index_select(0, torch.from_numpy(rows).to(flat.device)).float().cpu().numpy())
 
 
 def refiner_module(dev=None):
@@ -465,12 +522,12 @@ def run_b200(a):
         padded = (torch.full((pad_pairs, K, 2), -1, dtype=torch.int32, device=dev),
                   torch.zeros((pad_pairs, K), device=dev), torch.zeros((pad_pairs,), dtype=torch.int32, device=dev))
 
-    last_feats = [g_feats if replay is not None else None]
+    last_feats = [None]                                      # the bank the latest step wrote
 
     def step(timers=None, eager=False):
         if replay is not None and not eager:
             replay()
-            pairs, pscores, counts = g_pairs, g_pscores, g_counts
+            last_feats[0], pairs, pscores, counts = g_feats, g_pairs, g_pscores, g_counts
         else:
             last_feats[0], pairs, pscores, counts = run(timers)
         gathered = None
@@ -521,6 +578,12 @@ def run_b200(a):
     value = pairs_per_step / (ms_step * 1e-3)
     coll = {k: (sum(e0.elapsed_time(e1) for e0, e1 in v) / max(len(v), 1) if v else None) for k, v in coll_ms.items()}
     final_pairs, final_scores, final_counts = (t.clone() for t in out[:3])
+    if a.dump_outputs and rank == 0:
+        # rank 0's frames; with several ranks, the match lists of all ranks as gathered on rank 0
+        f = last_feats[0]
+        lists = out[3] if world > 1 else (final_pairs, final_scores, final_counts)
+        dump_outputs(a.dump_outputs, {"keypoints": f["keypoints_pixel"], "scores": f["scores"]},
+                     dict(zip(("pairs", "pair_scores", "counts"), lists)), f["descriptors"])
 
     # ---- instrumented pass: CUDA events around every kernel launch of the library (per-kernel rooflines)
     ops.profile_enable(True)
