@@ -239,6 +239,41 @@ int sslam_eval_matches(const int32_t* pred, const int32_t* pred_counts, int pred
                        int32_t* scratch, int32_t* out, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
+ * Geometric verification: RANSAC homography over the padded match lists of P pairs at once, in a
+ * fixed number of launches without host synchronisation (capturable in a CUDA graph).
+ *   kpts1 [F1,N,2], kpts2 [F2,M,2] fp32 (x,y); pair p reads sets (a,b) = pair_index[p] (int32 [P,2]) or
+ *   (p,p), as sslam_match_top2 / sslam_nn_points do.  pairs [P,L,2] int32 rows (i,j), pair_scores [P,L],
+ *   counts [P]: the output format of sslam_match_finalize (L = its N); rows k < min(counts[p], L) are used.
+ *   Hypothesis h (0 <= h < iters) of a pair with n rows solves the normalised 4-point DLT (double) on 4
+ *   distinct rows drawn by splitmix64: draw c (< 32, repeats redrawn) is output h*32 + c of the stream
+ *   seeded with `seed`, row = (u >> 32) * n >> 32.  Samples depend on (seed, h, n) only, so a pair gives
+ *   the same result alone or anywhere in a batch.  A sample is degenerate when a pivot of the 8x8 solve or
+ *   h33 is below 1e-8 in magnitude (collinear or repeated points), or when its 4 draws are not distinct.
+ *   Row k is an inlier of H iff ||pi(H.(x1,y1,1)) - (x2,y2)||^2 < threshold^2 (forward transfer error,
+ *   strict), in fp32 with u/w and v/w formed as u*(1/w), v*(1/w).
+ *   The best hypothesis has the most inliers; ties go to the lowest h.  It is refit by least squares
+ *   (normalised DLT over its inliers, smallest eigenvector of the 9x9 normal matrix, double, fixed-order
+ *   reductions) and the refit is kept iff it has at least as many inliers.
+ *   Outputs: H [P,9] double row-major frame1 -> frame2 scaled to h33 = 1 (may be NULL); the inlier rows in
+ *   input order (ascending i is preserved) as out_pairs [P,L,2] int32 (-1 padded), out_scores [P,L] (the
+ *   rows' pair_scores, 0 padded), out_counts [P]; inlier_mask [P,L] uint8 per input row (may be NULL).
+ *   No model — n < 4 or every hypothesis degenerate — is data: out_counts[p] = 0, H[p] all zeros, SSLAM_OK.
+ *   On return the workspace starts with the inlier count of every hypothesis, int32 [P,iters] (-1:
+ *   degenerate), followed at the next 256-byte boundary by the best hypothesis per pair, int32 [P] (-1:
+ *   none), and at the next by the best hypothesis's inlier mask before the refit, uint8 [P,L].
+ * Limits: L <= 16384, 1 <= iters <= 65536, threshold > 0.  Out-of-range keypoint indices in a row make
+ * that row an outlier (and a sample containing it degenerate).
+ */
+size_t sslam_ransac_workspace_bytes(int P, int L, int iters);
+int sslam_ransac_homography(const float* kpts1, int F1, const float* kpts2, int F2,
+                            const int32_t* pair_index, int P, int N, int M,
+                            const int32_t* pairs, const float* pair_scores, const int32_t* counts, int L,
+                            int iters, double threshold, uint64_t seed,
+                            double* H, int32_t* out_pairs, float* out_scores,
+                            int32_t* out_counts, uint8_t* inlier_mask,
+                            void* ws, size_t ws_bytes, void* stream);
+
+/* ---------------------------------------------------------------------------------------------
  * Optional cell-softmax front stage of the decode (north_star "softmax/depth-to-space ... border
  * mask"; OFF by default — the reference code has no such mode, keypoint_selector.py:61-62 is a
  * sigmoid; the vocabulary is papers/pdfs/SuperPoint_DeTone.md:49-58):

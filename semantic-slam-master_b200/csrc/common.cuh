@@ -58,7 +58,7 @@ extern std::atomic<uint64_t> g_launches;
 enum KernelKind {
   KK_DECODE_SCAN = 0, KK_DECODE_TOPK, KK_DECODE_COUNT, KK_DECODE_RESOLVE, KK_NMS, KK_GATHER, KK_L2NORM,
   KK_MATCH_F32, KK_MATCH_TC, KK_SPLIT, KK_UNPACK, KK_FINALIZE, KK_GEMM, KK_LAYERNORM, KK_EVAL, KK_HEATMAP,
-  KK_CONV_HEAD, KK_COUNT
+  KK_CONV_HEAD, KK_RANSAC_HYP, KK_RANSAC_SCORE, KK_RANSAC_REFIT, KK_COUNT
 };
 extern std::atomic<int> g_profile_on;
 void prof_mark(int kind, cudaStream_t stream, bool begin);

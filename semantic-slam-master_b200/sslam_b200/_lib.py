@@ -56,6 +56,11 @@ SIGNATURES = {
     "sslam_selector_head_f32": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int,
                                         c_int, c_int, c_int, c_void_p, c_void_p, c_size_t, c_void_p]),
     "sslam_heatmap_from_cells_f32": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p]),
+    "sslam_ransac_workspace_bytes": (c_size_t, [c_int] * 3),
+    "sslam_ransac_homography": (c_int, [c_void_p, c_int, c_void_p, c_int, c_void_p, c_int, c_int, c_int,
+                                        c_void_p, c_void_p, c_void_p, c_int, c_int, ctypes.c_double, ctypes.c_uint64,
+                                        c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t,
+                                        c_void_p]),
 }
 
 # include/sslam_b200_debug.h (tools only)

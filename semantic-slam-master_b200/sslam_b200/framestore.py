@@ -10,12 +10,13 @@ slots through ``pair_index`` (slot ids), so nothing leaves the device until the 
 
 ``FrameStore``          ring buffer of ``capacity`` slots; ``push`` extracts a batch of frames into it.
 ``match_spacings``      frame t against frame t - s for several spacings s at once (one matcher call).
+``verify_pairs``        RANSAC homography over lists those calls returned, from the resident keypoints.
 ``TrackingCounters``    the counters of track_frame_sequence (:166-199) accumulated on the device.
 """
 
 import torch
 
-from . import matchers, ops
+from . import geometry, matchers, ops
 from .ops import SIM_BF16, SIM_F16X3
 
 
@@ -107,6 +108,17 @@ class FrameStore:
             return fp, torch.empty(0, K, 2, dtype=torch.int32, device=dev), torch.empty(0, K, device=dev), \
                 torch.empty(0, dtype=torch.int32, device=dev)
         return (fp,) + tuple(self.match_pairs(fp, variant, **kw))
+
+    @torch.no_grad()
+    def verify_pairs(self, frame_pairs, pairs, scores, counts, **ransac):
+        """Geometric verification of the lists match_pairs / match_spacings returned for ``frame_pairs``,
+        on the resident keypoints (pixel units).  ``ransac``: threshold, iters, seed, want_mask.
+        Returns geometry.verify_homography_device's (H (P,3,3), pairs, scores, counts[, mask])."""
+        kp = self.bank["keypoints"]
+        if self.fe.grid != "pixel":
+            kp = kp * self.fe.patch + self.fe.patch / 2
+        return geometry.verify_homography_device(kp, kp, pairs, scores, counts, pair_index=self.pair_index(frame_pairs),
+                                                 **ransac)
 
 
 class TrackingCounters:

@@ -364,6 +364,62 @@ def eval_matches(pred_pairs, pred_counts, gt_pairs, gt_counts, num_kpts1):
     return out
 
 
+# ---------------------------------------------------------------------------------- geometric verification
+def ransac_homography(kpts1, kpts2, pairs, pair_scores, counts, pair_index=None, num_pairs=None, threshold=3.0,
+                      iters=1024, seed=0, want_mask=False, workspace=None):
+    """RANSAC homography per padded match list (sslam_ransac_homography).
+
+    kpts1 (F1,N,2), kpts2 (F2,M,2) fp32; pairs (P,L,2) int32, pair_scores (P,L) fp32, counts (P,) int32 as
+    match_finalize returns them; pair_index (P,2) int32 selects (a,b) per pair, default (p,p).
+    Returns (H (P,3,3) float64, h33 = 1, all zeros where there is no model; inlier pairs (P,L,2) int32 in
+    input order, -1 padded; their scores (P,L); counts (P,) int32[; inlier mask (P,L) uint8 per input row])."""
+    lib = _lib.load()
+    _need_cuda(kpts1, kpts2, pairs, pair_scores, counts, pair_index)
+    k1, k2 = kpts1.contiguous(), kpts2.contiguous()
+    if k1.dtype != torch.float32 or k2.dtype != torch.float32:
+        raise RuntimeError("ransac_homography expects fp32 keypoints")
+    pr = pairs.to(torch.int32).contiguous()
+    ps = pair_scores.to(torch.float32).contiguous()
+    cn = counts.to(torch.int32).contiguous()
+    F1, N = k1.shape[0], k1.shape[1]
+    F2, M = k2.shape[0], k2.shape[1]
+    P, L = pr.shape[0], pr.shape[1]
+    if pair_index is not None:
+        pair_index = pair_index.to(torch.int32).contiguous()
+        if pair_index.shape[0] != P:
+            raise RuntimeError("ransac_homography: pair_index must hold one (a, b) row per match list")
+    elif num_pairs is not None and int(num_pairs) != P:
+        raise RuntimeError("ransac_homography: num_pairs differs from the number of match lists")
+    dev = pr.device
+    H = torch.empty(P, 3, 3, dtype=torch.float64, device=dev)
+    out_pairs = torch.empty(P, L, 2, dtype=torch.int32, device=dev)
+    out_scores = torch.empty(P, L, dtype=torch.float32, device=dev)
+    out_counts = torch.empty(P, dtype=torch.int32, device=dev)
+    mask = torch.empty(P, L, dtype=torch.uint8, device=dev) if want_mask else None
+    need = lib.sslam_ransac_workspace_bytes(P, L, int(iters))
+    ws = workspace if workspace is not None else _ws("ransac", need, dev)
+    _lib.check(lib.sslam_ransac_homography(_ptr(k1), F1, _ptr(k2), F2, _ptr(pair_index), P, N, M, _ptr(pr),
+                                           _ptr(ps), _ptr(cn), L, int(iters), float(threshold),
+                                           int(seed) & 0xFFFFFFFFFFFFFFFF, _ptr(H), _ptr(out_pairs),
+                                           _ptr(out_scores), _ptr(out_counts), _ptr(mask), _ptr(ws), ws.numel(),
+                                           _stream()))
+    return (H, out_pairs, out_scores, out_counts) + ((mask,) if want_mask else ())
+
+
+def ransac_workspace_views(workspace, P, L, iters):
+    """Views of what sslam_ransac_homography leaves at the start of its workspace: per-hypothesis inlier
+    counts (P,iters) int32 (-1 degenerate), best hypothesis (P,) int32 (-1 none), and the best
+    hypothesis's inlier mask before the refit (P,L) uint8."""
+    def up(x):
+        return (x + 255) // 256 * 256
+    o_best = up(P * iters * 4)
+    o_mask = o_best + up(P * 4)
+    w = workspace
+    return (w[:P * iters * 4].view(torch.int32).reshape(P, iters),
+            w[o_best:o_best + P * 4].view(torch.int32),
+            w[o_mask:o_mask + P * L].reshape(P, L))
+
+
 # ---------------------------------------------------------------------------------- optional decode front stage (J1)
 def heatmap_from_cells(logits, cell=8, border=0):
     """(B, cell*cell+1, Hc, Wc) fp32 cell logits -> (B, Hc*cell, Wc*cell) heatmap: channel softmax,
