@@ -9,14 +9,6 @@
 extern "C" {
 #endif
 
-/* While buf != NULL (device memory, 4 int64 per CTA of the grid), the MMA thread of every CTA of
- * match_res_kernel writes {total, wait_full, wait_tempty, wait_afull} cycle counters. */
-void sslam_debug_match_stalls(long long* buf);
-
-/* While buf != NULL (device memory, 8 int64 per CTA), gemm_pair_kernel writes {MMA thread: total,
- * wait_full, wait_tempty, wait_weights}. */
-void sslam_debug_gemm_stalls(long long* buf);
-
 /* Host-mapped buffer (device pointer) that receives {block, thread, barrier, parity} records of
  * mbarrier waits that timed out in the GEMM translation unit; returns a cudaError_t value. */
 int sslam_debug_watchdog_gemm(unsigned long long* buf);
@@ -29,7 +21,8 @@ void sslam_debug_decode_stream(int on);
 void sslam_debug_decode_tune(int stages, int band_rows);
 
 /* DescriptorRefiner forward: 0 = one GEMM launch per layer; 1..4 = the layer-fused persistent kernel with
- * that many 256-row strip pairs per chunk (default 3).  Both paths compute bit-identical results. */
+ * that many 256-row strip pairs per chunk (default 3).  Other values are clamped to 0..4.  Both paths
+ * compute bit-identical results. */
 void sslam_debug_refiner_fused(int mode);
 
 #ifdef __cplusplus

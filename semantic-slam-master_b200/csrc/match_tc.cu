@@ -35,8 +35,6 @@ namespace sslam {
 
 using namespace tc;
 
-long long* g_match_dbg = nullptr;   // set by sslam_debug_match_stalls (tools only, not part of the ABI)
-
 namespace {
 
 constexpr int BM = 128, BN = 128;
@@ -52,7 +50,6 @@ template <> struct Cfg<SSLAM_SIM_TF32X3> {
   static constexpr float CROSS_SCALE = 1.0f;
 };
 struct TcParams {
-  long long* dbg;               // optional per-CTA stall counters of the MMA thread (debug aid), or null
   const int32_t* pair_index;
   int P, N, M, D;
   int32_t* nn12;
@@ -428,23 +425,15 @@ match_res_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_consta
       const uint32_t idesc = make_instr_desc(C::FMT, 2 * BM, BN);      // M = 256 across the pair
       int stage = 0; uint32_t phase = 0;
       int tc = 0, it = 0;
-      const bool dbg_on = p.dbg != nullptr;
-      long long w_full = 0, w_tempty = 0, w_afull = 0, t_begin = clock64(), tq = 0;
       for (int item = pair_id; item < nitems; item += npairs, ++it) {
         for (int ct = 0; ct < ntile; ++ct, ++tc) {
           const int acc = tc & 1;
-          if (dbg_on) tq = clock64();
           mbar_wait(&tempty[acc], (((uint32_t)tc >> 1) & 1u) ^ 1u);
-          if (dbg_on) w_tempty += clock64() - tq;
           tcgen05_fence_after();
           const uint32_t tmem_d = tmem_base + acc * C::ACC_COLS;
           for (int kb = 0; kb < nkb; ++kb) {
-            if (dbg_on) tq = clock64();
             if (ct == 0) mbar_wait(&afull[kb], (uint32_t)(it & 1));
-            if (dbg_on) w_afull += clock64() - tq;
-            if (dbg_on) tq = clock64();
             mbar_wait(&full[stage], phase);
-            if (dbg_on) w_full += clock64() - tq;
             tcgen05_fence_after();
             const uint32_t sa = smem_u32(a_res + (kb * C::TERMS) * BLOCK_BYTES);
             const uint32_t sb = smem_u32(b_stages + stage * L::B_STAGE);
@@ -468,10 +457,6 @@ match_res_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_consta
             if (++stage == C::B_STAGES) { stage = 0; phase ^= 1; }
           }
         }
-      }
-      if (p.dbg) {
-        long long* d = p.dbg + 4 * blockIdx.x;
-        d[0] = clock64() - t_begin; d[1] = w_full; d[2] = w_tempty; d[3] = w_afull;
       }
     }
   } else {
@@ -786,7 +771,6 @@ int match_top2_tc(const void* bank1, const void* bank1_lo, int F1, const void* b
                   int dtype, int P, int N, int M, int D, int32_t* nn12, float* best12, float* second12,
                   u64* colkeys, void* ws_extra, size_t ws_extra_bytes, cudaStream_t stream) {
   TcParams tp;
-  tp.dbg = g_match_dbg;
   tp.pair_index = pair_index; tp.P = P; tp.N = N; tp.M = M; tp.D = D;
   tp.nn12 = nn12; tp.best12 = best12; tp.second12 = second12; tp.colkeys = colkeys;
   CUtensorMap a_hi, a_lo, b_hi, b_lo;
@@ -864,7 +848,3 @@ int match_top2_tc(const void* bank1, const void* bank1_lo, int F1, const void* b
 }
 
 }  // namespace sslam
-
-// Debug aid for tools/: per-CTA {total, wait_full, wait_tempty, wait_afull} cycle counters of the MMA
-// thread of match_res_kernel are written to buf (device, 4 * gridDim int64) while buf != NULL.
-extern "C" void sslam_debug_match_stalls(long long* buf) { sslam::g_match_dbg = buf; }

@@ -43,7 +43,6 @@ using namespace tc;
 __device__ unsigned int g_refiner_status = 0;
 constexpr float F16_RANGE_SQ = 65504.0f * 65504.0f;
 
-long long* g_gemm_dbg = nullptr;    // set by sslam_debug_gemm_stalls (tools only, not part of the ABI)
 int g_refiner_fused = 3;            // 0: one launch per layer; 1..4: layer-fused kernel, strip pairs per chunk (sslam_debug_refiner_fused)
 
 namespace {
@@ -85,7 +84,6 @@ struct GemmParams {
   float* out_sum;
   float* out_sq;
   size_t stat_stride;
-  long long* dbg;           // optional per-CTA stall counters (debug aid), or null
 };
 
 // 32 contiguous, 32-byte aligned bytes through the read-only path as one 256-bit load
@@ -364,10 +362,7 @@ gemm_f16x3_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_const
 // tcgen05.commit multicasts `empty` / `tfull` to both CTAs; both epilogues arrive on the leader's
 // `tempty`.
 constexpr int P_STAGES = 3;
-#ifndef SSLAM_P_MAX_KB
-#define SSLAM_P_MAX_KB 6
-#endif
-constexpr int P_MAX_KB = SSLAM_P_MAX_KB;                  // K <= 384
+constexpr int P_MAX_KB = 6;                               // K <= 384
 constexpr int B_HALF = 64 * 128;                          // 64 weight rows x 128 bytes of K
 constexpr int P_STAGE_BYTES = 2 * BLOCK_BYTES;            // A_hi, A_lo
 constexpr int P_SMEM_B = P_MAX_KB * 2 * B_HALF;
@@ -494,24 +489,17 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_consta
       const uint16_t pair_mask = (uint16_t)(3u << leader);        // both CTAs of this pair
       const uint16_t all_mask = (uint16_t)((1u << (2 * ntile)) - 1u);
       int stage = 0; uint32_t phase = 0;
-      const bool dbg_on = p.dbg != nullptr;
-      long long w_full = 0, w_tempty = 0, tq = 0, t_begin = clock64();
       mbar_wait(bfull, 0);
       tcgen05_fence_after();
-      const long long w_b = clock64() - t_begin;
       int tc = 0;
       for (int sp = g; sp < nsp; sp += groups, ++tc) {
         const int acc = tc & 1;
-        if (dbg_on) tq = clock64();
         mbar_wait(&tempty[acc], (((uint32_t)tc >> 1) & 1u) ^ 1u);
-        if (dbg_on) w_tempty += clock64() - tq;
         tcgen05_fence_after();
         const uint32_t tmem_d = tmem_base + acc * 2 * BN;
         const uint32_t tmem_s = tmem_d + BN;
         for (int kb = 0; kb < nkb; ++kb) {
-          if (dbg_on) tq = clock64();
           mbar_wait(&full[stage], phase);
-          if (dbg_on) w_full += clock64() - tq;
           tcgen05_fence_after();
           const uint32_t sa = smem_u32(a_stages + stage * P_STAGE_BYTES);
           const uint32_t sb = smem_u32(bres + kb * 2 * B_HALF);
@@ -531,10 +519,6 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_consta
           if (kb == nkb - 1) tcgen05_commit_pair(&tfull[acc], pair_mask);
           if (++stage == P_STAGES) { stage = 0; phase ^= 1; }
         }
-      }
-      if (p.dbg) {
-        long long* d = p.dbg + 8 * blockIdx.x;
-        d[0] = clock64() - t_begin; d[1] = w_full; d[2] = w_tempty; d[3] = w_b;
       }
     }
   } else {
@@ -755,7 +739,7 @@ constexpr int F_THREADS = NUM_THREADS + 64;               // + the weight produc
 constexpr int F_W_WARP = NUM_THREADS / 32;
 constexpr int F_PUB_WARP = F_W_WARP + 1;
 // Activation stages: F_BK K-elements of the CTA's 128 rows, hi and lo (32 KB).  What bounds the kernel is
-// measured in DESIGN.md 4.5 (tools/fused_probe.py): neither the ring depth nor the request size.
+// measured in DESIGN.md 4.5: neither the ring depth nor the request size.
 constexpr int F_BK = 64;
 // Scratch activations (h, u): per 128-row strip and 64-column block one 32 KB piece = exactly one stage of
 // the A operand, [hi | lo][column / 8 (8 chunks)][row / 8][row % 8][column % 8] — the no-swizzle core-matrix
@@ -773,10 +757,7 @@ constexpr int F_STAGE_BYTES = 2 * F_HALF_BYTES;           // A_hi, A_lo
 // 160 cycles + 1 cycle per 73 bytes, so the feed wants few, large requests)
 static_assert(F_BK == 64, "the stage of the fused kernel is one 64-column block");
 // (a fourth 32 KB stage, tried at K = 320 where it fits: 2.60 instead of 2.62 ms — the ring depth is not the limit)
-#ifndef SSLAM_F_STAGES
-#define SSLAM_F_STAGES 3
-#endif
-constexpr int F_STAGES = SSLAM_F_STAGES;
+constexpr int F_STAGES = 3;
 constexpr int F_SUB = BK / F_BK;                          // stages per 64-element weight k-block
 constexpr int F_SMEM_A = F_STAGES * F_STAGE_BYTES;
 constexpr int F_SMEM_VECS = F_MAX_LAYERS * 2 * BN * 4;    // [layer][bias 128 | s1 128] of the pair's columns
@@ -801,8 +782,6 @@ struct FusedParams {
   float* st_sum[2];                  // partial row sums [2 * ntile][stat_stride]: 0 = of h, 1 = of u
   float* st_sq[2];
   size_t stat_stride;                // = groups * S * 256 scratch rows
-  long long* dbg;                    // optional per-CTA cycle counters (16 int64 per CTA), or null
-  int dbg_flags;
 };
 
 struct LayerInfo {
@@ -867,9 +846,6 @@ struct EpiTile {
   float* out_sum;                    // partial row sums of the output, [2 * ntile][stat_stride]
   float* out_sq;
   size_t stat_stride;
-  long long* dbg_wait;               // debug: per-section cycle counters (null = off)
-  bool nostore;                      // debug: skip the output stores
-  int dbgf;                          // debug flags (128: free-running epilogue, 256: no TMEM loads)
   uint64_t* tfull;
   uint32_t tempty_leader;
 };
@@ -898,19 +874,6 @@ struct EpiFlags { bool ln, res, relu, f32, stats; };
 
 __device__ __forceinline__ void fused_epilogue_tile(const EpiTile& c, const EpiFlags fl, int acc, uint32_t tfull_parity) {
   const int lane = c.lane, q = c.q, half = c.half;
-  long long* const dw = c.dbg_wait;
-  long long t0 = 0;
-#ifdef SSLAM_FUSED_SECTIONS                                // build-time switch of tools/fused_probe.py's section timers
-#if SSLAM_FUSED_SECTIONS == 2                               // coarse: [0] wait for the accumulator, [6] the rest of the tile
-#define SEC(i) do { if (dw && ((i) == 0 || (i) == 6)) { const long long t1_ = clock64(); dw[i] += t1_ - t0; t0 = t1_; } } while (0)
-#else
-#define SEC(i) do { if (dw) { const long long t1_ = clock64(); dw[i] += t1_ - t0; t0 = t1_; } } while (0)
-#endif
-  if (dw) t0 = clock64();
-#else
-#define SEC(i) do { } while (0)
-  (void)dw; (void)t0;
-#endif
   const float lo_clamp = fl.relu ? 0.f : __int_as_float(0xff800000);
   const bool wide = (c.N & 15) == 0;                     // fp32 output rows are 32-byte aligned only when N % 16 == 0
   // scratch arrays (h, u) are stored as 8-row x 16-byte core matrices, [strip][column / 8][row / 8][row % 8][column % 8]:
@@ -926,25 +889,21 @@ __device__ __forceinline__ void fused_epilogue_tile(const EpiTile& c, const EpiF
     if (gc + 8 < c.N) { nh[1] = ld_cg_128(res_h + o + SCR_CHUNK); nl[1] = ld_cg_128(res_l + o + SCR_CHUNK); }
   };
   if (fl.res) load_res(c.col_base + half * 64);          // in flight while the accumulator completes
-  SEC(1);
-  if (!(c.dbgf & 128)) mbar_wait(&c.tfull[acc], tfull_parity);
-  SEC(0);
+  mbar_wait(&c.tfull[acc], tfull_parity);
   tcgen05_fence_after();
   // (-mean, rstd) of this row of the A operand, from the publisher / LayerNorm warp (normally complete a
   // tile ago; never read before lnfull — this warp may get here while other CTAs are still storing the
   // statistics of the strip's previous layer)
   float ar = 1.f, nam = -0.f;
   if (fl.ln) {
-    if (!(c.dbgf & 128)) mbar_wait(c.lnfull, c.ln_parity);
+    mbar_wait(c.lnfull, c.ln_parity);
     const float2 ln = c.ln[q * 32 + lane];
     nam = ln.x; ar = ln.y;
   }
   uint32_t r[UNIT], rs[UNIT];
   const uint32_t tbase = c.tmem_base + ((uint32_t)(q * 32) << 16) + acc * 2 * BN + half * 64;
-  if (!(c.dbgf & 256)) {
-    tmem_ld_32x16(tbase, r);
-    tmem_ld_32x16(tbase + BN, rs);
-  }
+  tmem_ld_32x16(tbase, r);
+  tmem_ld_32x16(tbase + BN, rs);
   // The arithmetic below is the scalar formula of gemm_pair_kernel's epilogue, element for element
   // (same operations, same roundings), issued two elements at a time: FFMA2 / FADD2 / FMUL2 on register
   // pairs, and the fp16 <-> fp32 mixed forms (FHADD, FHFMA) instead of a conversion plus an fp32 operation.
@@ -959,27 +918,21 @@ __device__ __forceinline__ void fused_epilogue_tile(const EpiTile& c, const EpiF
     uint4 rh[2] = {nh[0], nh[1]}, rl[2] = {nl[0], nl[1]};
     if (fl.res && un + 1 < 64 / UNIT) load_res(gc0 + UNIT);
     uint64_t x2[UNIT / 2];
-    SEC(3);
     tmem_ld_wait();
-    SEC(2);
 #pragma unroll
     for (int j = 0; j < UNIT / 2; ++j)                     // fold the cross terms
       x2[j] = ffma2(pack_f32x2(__uint_as_float(rs[2 * j]), __uint_as_float(rs[2 * j + 1])), inv2,
                     pack_f32x2(__uint_as_float(r[2 * j]), __uint_as_float(r[2 * j + 1])));
-    if (un + 1 < 64 / UNIT && !(c.dbgf & 256)) {         // next unit's accumulators: in flight during the math
+    if (un + 1 < 64 / UNIT) {                              // next unit's accumulators: in flight during the math
       tmem_ld_32x16(tbase + (un + 1) * UNIT, r);
       tmem_ld_32x16(tbase + (un + 1) * UNIT + BN, rs);
     }
-    SEC(3);
     if (gc0 >= c.N) continue;
     float v[UNIT];
 #pragma unroll
     for (int j = 0; j < UNIT / 2; j += 2) {
-      float4 b4 = make_float4(0.5f, 0.25f, 0.125f, 1.f), s4 = b4;
-      if (!(c.dbgf & 512)) {
-        b4 = *reinterpret_cast<const float4*>(c.sbias + col0 + 2 * j);
-        s4 = *reinterpret_cast<const float4*>(c.ss1 + col0 + 2 * j);
-      }
+      const float4 b4 = *reinterpret_cast<const float4*>(c.sbias + col0 + 2 * j);
+      const float4 s4 = *reinterpret_cast<const float4*>(c.ss1 + col0 + 2 * j);
       // rho*(acc - mu*s1) + c0
       x2[j] = ffma2(ar2, ffma2(nam2, pack_f32x2(s4.x, s4.y), x2[j]), pack_f32x2(b4.x, b4.y));
       x2[j + 1] = ffma2(ar2, ffma2(nam2, pack_f32x2(s4.z, s4.w), x2[j + 1]), pack_f32x2(b4.z, b4.w));
@@ -1004,11 +957,8 @@ __device__ __forceinline__ void fused_epilogue_tile(const EpiTile& c, const EpiF
       sum2 = fadd2(sum2, x2[j]);
       sq2 = ffma2(x2[j], x2[j], sq2);
     }
-    SEC(3);
     const bool whole = gc0 + UNIT <= c.N;
-    if (c.nostore) {
-      if (v[0] == 1234.5f) c.o_f32[0] = v[3] + v[7] + v[12];
-    } else if (fl.f32) {
+    if (fl.f32) {
       if (c.row_ok) {
         float* dst = c.o_f32 + c.orow * (size_t)c.N + gc0;
         if (whole && wide) {
@@ -1046,7 +996,6 @@ __device__ __forceinline__ void fused_epilogue_tile(const EpiTile& c, const EpiF
         *reinterpret_cast<uint4*>(c.o_lo + o + SCR_CHUNK) = pl[1];
       }
     }
-    SEC(5);
   }
   float rsum, rsq;
   {
@@ -1067,8 +1016,6 @@ __device__ __forceinline__ void fused_epilogue_tile(const EpiTile& c, const EpiF
     c.out_sum[o] = rsum;
     c.out_sq[o] = rsq;
   }
-  SEC(6);
-#undef SEC
 }
 
 __global__ void __launch_bounds__(F_THREADS, 1)
@@ -1124,9 +1071,7 @@ refiner_fused_kernel(const __grid_constant__ FusedMaps tm, const FusedParams p) 
   tcgen05_fence_after();
   const uint32_t tmem_base = *tmem_slot;
 
-  const bool freerun = (p.dbg_flags & 128) != 0;       // debug: only the epilogue warps run, without any barrier
-  if (freerun && (warp < 2 || warp == F_W_WARP || warp == F_PUB_WARP)) {
-  } else if (warp == 0) {
+  if (warp == 0) {
     // ---- activation producer (every CTA): one thread drives the barriers and the TMA.  It never does
     // anything else: with three stages in flight any pause of this thread is a bubble in the tensor pipe.
     if (lane == 0) for (int i = 0; i < 3; ++i) { prefetch_tensormap(&tm.a_hi[i]); prefetch_tensormap(&tm.a_lo[i]); }
@@ -1136,8 +1081,6 @@ refiner_fused_kernel(const __grid_constant__ FusedMaps tm, const FusedParams p) 
     const int scr_kb = (p.Hd + F_BK - 1) / F_BK;                  // 64-column blocks of a scratch strip
     int stage = 0; uint32_t phase = 0;
     int turn = 0, nchunk = 0;
-    const bool dbg_on = p.dbg != nullptr;
-    long long w_ready = 0, w_empty = 0, tq = 0;
     for (int c0 = 0; c0 < cnt; c0 += S, ++nchunk) {
       const int Sc = min(S, cnt - c0);
       for (int l = 0; l < L; ++l) {
@@ -1157,9 +1100,7 @@ refiner_fused_kernel(const __grid_constant__ FusedMaps tm, const FusedParams p) 
               // whole L1 (CCTL.IVALL) and would evict the bias vectors the epilogue reads through it
               // once per tile.  The proxy fence orders the async proxy (TMA) after the wait.
               const uint32_t par = (uint32_t)(nchunk * (L - 1) + l - 1) & 1u;
-              if (dbg_on) tq = clock64();
               mbar_wait(&ready[s], par);
-              if (dbg_on) w_ready += clock64() - tq;
               fence_proxy_async_all();
             }
           }
@@ -1167,9 +1108,7 @@ refiner_fused_kernel(const __grid_constant__ FusedMaps tm, const FusedParams p) 
             const bool pf = (l == L - 1) && (c0 + S + s < cnt);   // next chunk's input rows -> L2
             const int pf_row = (g + (c0 + S + s) * groups) * 2 * BM + (int)rank * BM;
             for (int kb = 0; kb < nkb; ++kb) {
-              if (dbg_on) tq = clock64();
               mbar_wait(&empty[stage], phase ^ 1);
-              if (dbg_on) w_empty += clock64() - tq;
               unsigned char* st = a_stages + stage * F_STAGE_BYTES;
               const uint32_t full_leader = mapa_u32(smem_u32(&full[stage]), leader);
               if (rank == 0) mbar_arrive_expect_tx(&full[stage], 2u * F_STAGE_BYTES);
@@ -1206,7 +1145,6 @@ refiner_fused_kernel(const __grid_constant__ FusedMaps tm, const FusedParams p) 
         mbar_wait(&empty[stage], phase ^ 1);
         if (++stage == F_STAGES) { stage = 0; phase ^= 1; }
       }
-      if (dbg_on) { long long* d = p.dbg + 16 * blockIdx.x; d[4] = w_ready; d[5] = w_empty; }
     }
   } else if (warp == F_W_WARP) {
     if (elect_one()) {                                            // ---- weight producer (every CTA)
@@ -1298,7 +1236,7 @@ refiner_fused_kernel(const __grid_constant__ FusedMaps tm, const FusedParams p) 
           if (l + 1 < L) {                                        // P(l, s)
             if (lane == 0) {
               mbar_wait(&tdone[tcn & 3u], (tcn >> 2) & 1u);
-              if (!(p.dbg_flags & 8192)) asm volatile("fence.release.cluster;" ::: "memory");   // (debug 8192: timing without the fence)
+              asm volatile("fence.release.cluster;" ::: "memory");
               const uint32_t rb = smem_u32(&ready[s]);
               for (uint32_t j = 0; j < ncta; ++j) mbar_arrive_cluster_relaxed(mapa_u32(rb, j));
             }
@@ -1315,9 +1253,6 @@ refiner_fused_kernel(const __grid_constant__ FusedMaps tm, const FusedParams p) 
       const uint16_t all_mask = (uint16_t)((1u << (2 * ntile)) - 1u);
       int stage = 0; uint32_t phase = 0;
       uint32_t tc = 0, n = 0;
-      const bool dbg_on = p.dbg != nullptr;
-      long long w_full = 0, w_tempty = 0, w_w = 0, tq = 0;
-      const long long t_begin = clock64();
       for (int c0 = 0; c0 < cnt; c0 += S) {
         const int Sc = min(S, cnt - c0);
         for (int l = 0; l < L; ++l, ++n) {
@@ -1325,9 +1260,7 @@ refiner_fused_kernel(const __grid_constant__ FusedMaps tm, const FusedParams p) 
           const int nkb = (li.K + BK - 1) / BK;               // weight k-blocks of this layer
           for (int s = 0; s < Sc; ++s, ++tc) {
             const int acc = (int)(tc & 1u);
-            if (dbg_on) tq = clock64();
             mbar_wait(&tempty[acc], ((tc >> 1) & 1u) ^ 1u);
-            if (dbg_on) w_tempty += clock64() - tq;
             tcgen05_fence_after();
             const uint32_t tmem_d = tmem_base + acc * 2 * BN;
             const uint32_t tmem_s = tmem_d + BN;
@@ -1335,11 +1268,8 @@ refiner_fused_kernel(const __grid_constant__ FusedMaps tm, const FusedParams p) 
             const int nst = (li.K + F_BK - 1) / F_BK;             // activation stages of this tile (32 K-elements each)
             for (int ks = 0; ks < nst; ++ks) {
               const int kb = ks / F_SUB, sub = ks % F_SUB;        // weight k-block (64 K-elements) of this stage
-              if (dbg_on) tq = clock64();
               if (s == 0 && sub == 0) mbar_wait(&wfull[kb], n & 1u);     // this layer's weights, k-block kb
-              if (dbg_on) { const long long t1 = clock64(); w_w += t1 - tq; tq = t1; }
               mbar_wait(&full[stage], phase);
-              if (dbg_on) w_full += clock64() - tq;
               tcgen05_fence_after();
               const uint32_t sa = smem_u32(a_stages + stage * F_STAGE_BYTES);
               const uint32_t sb = smem_u32(bres + kb * 2 * B_HALF);
@@ -1355,7 +1285,7 @@ refiner_fused_kernel(const __grid_constant__ FusedMaps tm, const FusedParams p) 
               const uint64_t b_lo = make_smem_desc_sw128(sb + B_HALF) + boff;
               // a pair whose columns lie beyond the layer's width (output projection narrower than the hidden
               // layers) keeps the barrier protocol going but issues no MMAs: its epilogue skips every column
-              if (!(p.dbg_flags & 2) && col_base < li.N)
+              if (col_base < li.N)
 #pragma unroll
               for (int k = 0; k < F_BK / 16; ++k) {
                 const uint64_t adv = (uint64_t)(k * 32 >> 4), aadv = (uint64_t)k * a_step;
@@ -1374,10 +1304,6 @@ refiner_fused_kernel(const __grid_constant__ FusedMaps tm, const FusedParams p) 
           }
         }
       }
-      if (dbg_on) {
-        long long* d = p.dbg + 16 * blockIdx.x;
-        d[0] = clock64() - t_begin; d[1] = w_full; d[2] = w_tempty; d[3] = w_w;
-      }
     }
   } else {
     // ---- epilogue warps 2..9 of both CTAs
@@ -1394,25 +1320,18 @@ refiner_fused_kernel(const __grid_constant__ FusedMaps tm, const FusedParams p) 
     const uint32_t tempty_leader0 = mapa_u32(smem_u32(&tempty[0]), leader);
     const uint32_t tempty_leader1 = mapa_u32(smem_u32(&tempty[1]), leader);
     uint32_t tc = 0;
-#ifdef SSLAM_FUSED_SECTIONS
-    long long sec[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-    const long long t_begin = clock64();
-    c.dbg_wait = (p.dbg && lane == 0 && (warp == 2 || warp == 6)) ? sec : nullptr;
-#else
-    c.dbg_wait = nullptr;
-#endif
-    uint32_t tcn = 0;                                             // tiles handed to the publisher so far
+    uint32_t tcn = 0;                                            // tiles handed to the publisher so far
     int nchunk = 0;
     const size_t scr_strip = (size_t)((p.Hd + F_BK - 1) / F_BK) * SCR_BLOCK;   // elements of one strip of a scratch array
     for (int c0 = 0; c0 < cnt; c0 += S, ++nchunk) {
-      const int Sc = min(S, cnt - c0);
       for (int l = 0; l < L; ++l) {
         const LayerInfo li = layer_info(p, l);
         c.N = li.N; c.K = li.K;
         c.sbias = svec + l * 2 * BN; c.ss1 = c.sbias + BN;
         c.o_hi = p.s_hi[li.dst]; c.o_lo = p.s_lo[li.dst];
         c.out_sum = p.st_sum[li.st_out]; c.out_sq = p.st_sq[li.st_out];
-        for (int s = 0; s < Sc; ++s, ++tc) {
+        // s < min(S, cnt - c0), written so that no chunk count stays live across the tile (168 registers, no spill)
+        for (int s = 0; s < S && c0 + s < cnt; ++s, ++tc) {
           const int srow_w = ((g * S + s) * 2 + (int)rank) * BM + c.q * 32;       // scratch row of lane 0
           const int trow_w = (g + (c0 + s) * groups) * 2 * BM + (int)rank * BM + c.q * 32;
           c.srow = (size_t)(srow_w + lane);
@@ -1422,23 +1341,12 @@ refiner_fused_kernel(const __grid_constant__ FusedMaps tm, const FusedParams p) 
           const int acc = (int)(tc & 1u);
           const uint32_t par = (tc >> 1) & 1u;
           c.tempty_leader = acc ? tempty_leader1 : tempty_leader0;
-          const EpiFlags fl{li.ln && !(p.dbg_flags & 32), li.res && !(p.dbg_flags & 16), li.relu, li.f32, li.stats && !(p.dbg_flags & 64)};
-          c.nostore = (p.dbg_flags & 8) != 0;
-          c.dbgf = p.dbg_flags;
+          const EpiFlags fl{li.ln, li.res, li.relu, li.f32, li.stats};
           c.ln = sln + (tc & 1u) * BM;
           c.lnfull = &lnfull[tc & 1u];
           c.ln_parity = (tc >> 1) & 1u;
-          if (p.dbg_flags & 4) {
-            mbar_wait(&tfull[acc], par);
-            tcgen05_fence_after();
-            tcgen05_fence_before();
-            __syncwarp();
-            if (lane == 0) mbar_arrive_cluster(c.tempty_leader);
-          } else {
-            fused_epilogue_tile(c, fl, acc, par);
-          }
+          fused_epilogue_tile(c, fl, acc, par);
           if (l < L - 1) {                                        // hand the tile to the publisher warp
-            if (p.dbg_flags & 1) __threadfence();
             __syncwarp();
             if (lane == 0) mbar_arrive(&tdone[tcn & 3u]);
             ++tcn;
@@ -1446,13 +1354,6 @@ refiner_fused_kernel(const __grid_constant__ FusedMaps tm, const FusedParams p) 
         }
       }
     }
-#ifdef SSLAM_FUSED_SECTIONS
-    if (c.dbg_wait && warp == 2) {
-      long long* d = p.dbg + 16 * blockIdx.x + 6;
-      d[0] = clock64() - t_begin;
-      for (int i = 0; i < 8; ++i) d[1 + i] = sec[i];
-    }
-#endif
   }
   tcgen05_fence_before();
   cluster_sync_all();
@@ -1547,7 +1448,6 @@ int launch_gemm(Pair a, Pair w, int rows, int N, int K, const float* bias, RowSt
   gp.out_sum = out_stats ? out_stats->sum : nullptr;
   gp.out_sq = out_stats ? out_stats->sq : nullptr;
   gp.stat_stride = stat_stride_of(rows);
-  gp.dbg = g_gemm_dbg;
   if (pair) {
     const int ntile = (N + BN - 1) / BN;
     const int nsp = (rows + 2 * BM - 1) / (2 * BM);
@@ -1647,8 +1547,7 @@ int launch_fused(Pair xs, const FusedLayer* layers, int rows, int C, int Hd, int
   int groups = mcl < nsp ? mcl : nsp;
   const int cap = 160 / (2 * ntile);
   if (groups > cap) groups = cap;
-  int S = g_refiner_fused & 255;
-  if (S > F_MAX_SLOTS) S = F_MAX_SLOTS;
+  int S = g_refiner_fused;                                       // 1..F_MAX_SLOTS (sslam_debug_refiner_fused)
   const int per_cluster = (nsp + groups - 1) / groups;
   if (S > per_cluster) S = per_cluster;                          // short inputs: no unused scratch slots
   const size_t srows = (size_t)groups * S * 2 * BM;
@@ -1672,8 +1571,6 @@ int launch_fused(Pair xs, const FusedLayer* layers, int rows, int C, int Hd, int
   }
   fp.rows = rows; fp.C = C; fp.Hd = Hd; fp.D = D; fp.L = L; fp.S = S; fp.groups = groups; fp.ntile = ntile;
   fp.s_hi[0] = sh.hi; fp.s_lo[0] = sh.lo; fp.s_hi[1] = su.hi; fp.s_lo[1] = su.lo; fp.raw = raw; fp.stat_stride = srows;
-  fp.dbg = g_gemm_dbg;
-  fp.dbg_flags = g_refiner_fused >> 8;
 
   FusedMaps m;
   int rc;
@@ -1861,13 +1758,6 @@ extern "C" int sslam_refiner_forward_f32(const float* const* params, const void*
   return sslam_l2norm_rows(raw, rows, D, eps_norm, out_f32, out_bf16, out_hi, out_lo, stream_);   // :86
 }
 
-// Debug aid for tools/: per-CTA cycle counters of gemm_pair_kernel ({MMA thread: total, wait_full,
-// wait_tempty, wait_weights; epilogue warp 2: total, wait_tfull, wait_store, tiles}, 8 int64 per CTA)
-// are written to buf (device) while buf != NULL.
-extern "C" void sslam_debug_gemm_stalls(long long* buf) { sslam::g_gemm_dbg = buf; }
-
-// Debug aid for tests / tools: 0 = one GEMM launch per layer (gemm_pair_kernel); 1..4 = the layer-fused
-// kernel with that many strip pairs per chunk (default 3).
 extern "C" int sslam_refiner_range_check(void* stream_) {
   int rc = check_device();
   if (rc) return rc;
@@ -1885,7 +1775,11 @@ extern "C" int sslam_refiner_range_check(void* stream_) {
   return SSLAM_OK;
 }
 
-extern "C" void sslam_debug_refiner_fused(int mode) { sslam::g_refiner_fused = mode < 0 ? 0 : mode; }
+// Debug aid for tests / tools: 0 = one GEMM launch per layer (gemm_pair_kernel); 1..4 = the layer-fused
+// kernel with that many strip pairs per chunk (default 3).  Other values are clamped to 0..4.
+extern "C" void sslam_debug_refiner_fused(int mode) {
+  sslam::g_refiner_fused = mode < 0 ? 0 : (mode > sslam::F_MAX_SLOTS ? sslam::F_MAX_SLOTS : mode);
+}
 
 // Debug aid for tools/: host-mapped buffer (device pointer) that receives watchdog records of this
 // translation unit's kernels; see tc_common.cuh.

@@ -65,8 +65,6 @@ SIGNATURES = {
 
 # include/sslam_b200_debug.h (tools only)
 DEBUG_SIGNATURES = {
-    "sslam_debug_match_stalls": (None, [c_void_p]),
-    "sslam_debug_gemm_stalls": (None, [c_void_p]),
     "sslam_debug_watchdog_gemm": (c_int, [c_void_p]),
     "sslam_debug_decode_stream": (None, [c_int]),
     "sslam_debug_refiner_fused": (None, [c_int]),
