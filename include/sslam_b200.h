@@ -274,6 +274,51 @@ int sslam_ransac_homography(const float* kpts1, int F1, const float* kpts2, int 
                             void* ws, size_t ws_bytes, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
+ * Epipolar verification: RANSAC fundamental matrix over the padded match lists of P pairs at once.
+ * The parameters, the launches, the determinism, the outputs' format, the no-model convention and the
+ * limits are those of sslam_ransac_homography; only the model differs.
+ *   Sample s (0 <= s < iters; iters counts samples, as cv2's maxIters does) draws 7 distinct rows with
+ *   the same sampler (draw c < 32 is output s*32 + c, repeats redrawn).  The 7-point solve runs in double
+ *   with correctly rounded operations only: each image's points are normalised (centroid, sqrt(2) / mean
+ *   distance); the 7x9 system of rows [u x, u y, u, v x, v y, v, x, y, 1] (x1 = (x,y), x2 = (u,v)) is
+ *   reduced by Gaussian elimination with full pivoting (largest |entry| of the remaining submatrix,
+ *   lowest (row, column) on ties); the two columns that never pivot, in ascending order, give the null
+ *   vectors f1, f2.  The real roots of det(F2 + lam (F1 - F2)) = c3 lam^3 + c2 lam^2 + c1 lam + c0 are
+ *   taken as lam in [-1, 1] from that cubic, then as mu = 1/lam in (-1, 1) from c0 mu^3 + c1 mu^2 + c2 mu
+ *   + c3 (mu = 0 is F1 - F2); each interval is split at the real critical points and every bracket
+ *   with a sign change is bisected 64 times.  Each root's F is denormalised (T2^T F T1), scaled to unit
+ *   Frobenius norm and signed so that its largest-|entry| element (lowest index on ties) is positive.
+ *   Sample s owns hypothesis slots 3s, 3s+1, 3s+2, filled in root order (the first cubic's roots
+ *   ascending, then the second's); unused slots are degenerate.  A sample is degenerate when n < 7, the
+ *   sampler finds no 7 distinct rows in 32 draws, the 7 points coincide in either image, a pivot is below
+ *   1e-8 in magnitude (7 correspondences related by one homography give a rank-6 system, so an exactly
+ *   planar or purely rotating sample is degenerate) or no root is real.
+ *   Row k is an inlier of F iff both squared point-to-epipolar-line distances (cv2's FM_RANSAC error) are
+ *   < threshold^2, in fp32 with the fp32 hypothesis: a2 = (F0 x1 + F1 y1) + F2, b2 = (F3 x1 + F4 y1) + F5,
+ *   c2 = (F6 x1 + F7 y1) + F8, d2 = (x2 a2 + y2 b2) + c2, e2 = d2 d2 * (1 / (a2 a2 + b2 b2)); e1 likewise
+ *   with F^T and the points' roles swapped.  An undefined line (NaN) makes the row an outlier.
+ *   The best slot has the most inliers (lowest slot on ties).  With at least 8 inliers it is refit by the
+ *   normalised 8-point least squares over them (smallest eigenvector of the 9x9 normal matrix, rank 2
+ *   enforced as F' = Fn - (Fn v3) v3^T with v3 the smallest eigenvector of Fn^T Fn), kept iff it has at
+ *   least as many inliers.
+ *   Outputs: F [P,9] double row-major with x2^T F x1 = 0, unit Frobenius norm (may be NULL); out_pairs,
+ *   out_scores, out_counts and inlier_mask as for the homography.  No model is data: F[p] all zeros, an
+ *   empty list, SSLAM_OK.  On return the workspace starts with the inlier count of every slot, int32
+ *   [P,3*iters] (-1: degenerate), then at the next 256-byte boundary the best slot per pair, int32 [P]
+ *   (-1: none), then the best slot's inlier mask before the refit, uint8 [P,L].
+ * Limits: L <= 16384, 1 <= iters <= 65536, threshold > 0.  The workspace holds 40 bytes per slot, so
+ * 32 640 pairs (all pairs of 256 keyframes) at 1024 samples need about 4.0 GB.
+ */
+size_t sslam_ransac_fundamental_workspace_bytes(int P, int L, int iters);
+int sslam_ransac_fundamental(const float* kpts1, int F1, const float* kpts2, int F2,
+                             const int32_t* pair_index, int P, int N, int M,
+                             const int32_t* pairs, const float* pair_scores, const int32_t* counts, int L,
+                             int iters, double threshold, uint64_t seed,
+                             double* F, int32_t* out_pairs, float* out_scores,
+                             int32_t* out_counts, uint8_t* inlier_mask,
+                             void* ws, size_t ws_bytes, void* stream);
+
+/* ---------------------------------------------------------------------------------------------
  * Optional cell-softmax front stage of the decode (north_star "softmax/depth-to-space ... border
  * mask"; OFF by default — the reference code has no such mode, keypoint_selector.py:61-62 is a
  * sigmoid; the vocabulary is papers/pdfs/SuperPoint_DeTone.md:49-58):

@@ -61,6 +61,11 @@ SIGNATURES = {
                                         c_void_p, c_void_p, c_void_p, c_int, c_int, ctypes.c_double, ctypes.c_uint64,
                                         c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t,
                                         c_void_p]),
+    "sslam_ransac_fundamental_workspace_bytes": (c_size_t, [c_int] * 3),
+    "sslam_ransac_fundamental": (c_int, [c_void_p, c_int, c_void_p, c_int, c_void_p, c_int, c_int, c_int,
+                                         c_void_p, c_void_p, c_void_p, c_int, c_int, ctypes.c_double,
+                                         ctypes.c_uint64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                         c_void_p, c_size_t, c_void_p]),
 }
 
 # include/sslam_b200_debug.h (tools only)

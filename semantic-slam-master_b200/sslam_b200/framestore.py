@@ -10,7 +10,8 @@ slots through ``pair_index`` (slot ids), so nothing leaves the device until the 
 
 ``FrameStore``          ring buffer of ``capacity`` slots; ``push`` extracts a batch of frames into it.
 ``match_spacings``      frame t against frame t - s for several spacings s at once (one matcher call).
-``verify_pairs``        RANSAC homography over lists those calls returned, from the resident keypoints.
+``verify_pairs``        RANSAC homography or fundamental matrix over lists those calls returned, from the
+                        resident keypoints.
 ``TrackingCounters``    the counters of track_frame_sequence (:166-199) accumulated on the device.
 """
 
@@ -110,15 +111,20 @@ class FrameStore:
         return (fp,) + tuple(self.match_pairs(fp, variant, **kw))
 
     @torch.no_grad()
-    def verify_pairs(self, frame_pairs, pairs, scores, counts, **ransac):
+    def verify_pairs(self, frame_pairs, pairs, scores, counts, model="homography", **ransac):
         """Geometric verification of the lists match_pairs / match_spacings returned for ``frame_pairs``,
-        on the resident keypoints (pixel units).  ``ransac``: threshold, iters, seed, want_mask.
-        Returns geometry.verify_homography_device's (H (P,3,3), pairs, scores, counts[, mask])."""
+        on the resident keypoints (pixel units), against a homography (default) or, with
+        ``model="fundamental"``, the epipolar constraint.  ``ransac``: threshold, iters, seed, want_mask.
+        Returns geometry.verify_homography_device's (H (P,3,3), pairs, scores, counts[, mask]), or
+        verify_fundamental_device's with F in place of H."""
+        verify = {"homography": geometry.verify_homography_device,
+                  "fundamental": geometry.verify_fundamental_device}.get(model)
+        if verify is None:
+            raise ValueError(f"verify_pairs: model must be 'homography' or 'fundamental', not {model!r}")
         kp = self.bank["keypoints"]
         if self.fe.grid != "pixel":
             kp = kp * self.fe.patch + self.fe.patch / 2
-        return geometry.verify_homography_device(kp, kp, pairs, scores, counts, pair_index=self.pair_index(frame_pairs),
-                                                 **ransac)
+        return verify(kp, kp, pairs, scores, counts, pair_index=self.pair_index(frame_pairs), **ransac)
 
 
 class TrackingCounters:

@@ -373,11 +373,37 @@ def ransac_homography(kpts1, kpts2, pairs, pair_scores, counts, pair_index=None,
     match_finalize returns them; pair_index (P,2) int32 selects (a,b) per pair, default (p,p).
     Returns (H (P,3,3) float64, h33 = 1, all zeros where there is no model; inlier pairs (P,L,2) int32 in
     input order, -1 padded; their scores (P,L); counts (P,) int32[; inlier mask (P,L) uint8 per input row])."""
+    return _ransac("homography", kpts1, kpts2, pairs, pair_scores, counts, pair_index, num_pairs, threshold, iters,
+                   seed, want_mask, workspace)
+
+
+def ransac_fundamental(kpts1, kpts2, pairs, pair_scores, counts, pair_index=None, num_pairs=None, threshold=3.0,
+                       iters=1024, seed=0, want_mask=False, workspace=None):
+    """RANSAC fundamental matrix per padded match list (sslam_ransac_fundamental): 7-point samples,
+    symmetric epipolar error, 8-point refit.  Arguments as for ransac_homography; ``iters`` counts samples.
+    Returns (F (P,3,3) float64 with x2^T F x1 = 0, unit Frobenius norm, all zeros where there is no model;
+    inlier pairs, scores, counts[, inlier mask]) in ransac_homography's format."""
+    return _ransac("fundamental", kpts1, kpts2, pairs, pair_scores, counts, pair_index, num_pairs, threshold,
+                   iters, seed, want_mask, workspace)
+
+
+_RANSAC_SYMBOLS = {"homography": ("sslam_ransac_homography", "sslam_ransac_workspace_bytes", 1),
+                   "fundamental": ("sslam_ransac_fundamental", "sslam_ransac_fundamental_workspace_bytes", 3)}
+
+
+def ransac_workspace_bytes(P, L, iters, model="homography"):
+    """Workspace bytes ransac_homography / ransac_fundamental need for P lists of stride L."""
+    return getattr(_lib.load(), _RANSAC_SYMBOLS[model][1])(int(P), int(L), int(iters))
+
+
+def _ransac(model, kpts1, kpts2, pairs, pair_scores, counts, pair_index, num_pairs, threshold, iters, seed,
+            want_mask, workspace):
+    name = "ransac_" + model
     lib = _lib.load()
     _need_cuda(kpts1, kpts2, pairs, pair_scores, counts, pair_index)
     k1, k2 = kpts1.contiguous(), kpts2.contiguous()
     if k1.dtype != torch.float32 or k2.dtype != torch.float32:
-        raise RuntimeError("ransac_homography expects fp32 keypoints")
+        raise RuntimeError(f"{name} expects fp32 keypoints")
     pr = pairs.to(torch.int32).contiguous()
     ps = pair_scores.to(torch.float32).contiguous()
     cn = counts.to(torch.int32).contiguous()
@@ -387,35 +413,39 @@ def ransac_homography(kpts1, kpts2, pairs, pair_scores, counts, pair_index=None,
     if pair_index is not None:
         pair_index = pair_index.to(torch.int32).contiguous()
         if pair_index.shape[0] != P:
-            raise RuntimeError("ransac_homography: pair_index must hold one (a, b) row per match list")
+            raise RuntimeError(f"{name}: pair_index must hold one (a, b) row per match list")
     elif num_pairs is not None and int(num_pairs) != P:
-        raise RuntimeError("ransac_homography: num_pairs differs from the number of match lists")
+        raise RuntimeError(f"{name}: num_pairs differs from the number of match lists")
     dev = pr.device
-    H = torch.empty(P, 3, 3, dtype=torch.float64, device=dev)
+    G = torch.empty(P, 3, 3, dtype=torch.float64, device=dev)
     out_pairs = torch.empty(P, L, 2, dtype=torch.int32, device=dev)
     out_scores = torch.empty(P, L, dtype=torch.float32, device=dev)
     out_counts = torch.empty(P, dtype=torch.int32, device=dev)
     mask = torch.empty(P, L, dtype=torch.uint8, device=dev) if want_mask else None
-    need = lib.sslam_ransac_workspace_bytes(P, L, int(iters))
+    fn, ws_fn, _ = _RANSAC_SYMBOLS[model]
+    need = getattr(lib, ws_fn)(P, L, int(iters))
     ws = workspace if workspace is not None else _ws("ransac", need, dev)
-    _lib.check(lib.sslam_ransac_homography(_ptr(k1), F1, _ptr(k2), F2, _ptr(pair_index), P, N, M, _ptr(pr),
-                                           _ptr(ps), _ptr(cn), L, int(iters), float(threshold),
-                                           int(seed) & 0xFFFFFFFFFFFFFFFF, _ptr(H), _ptr(out_pairs),
-                                           _ptr(out_scores), _ptr(out_counts), _ptr(mask), _ptr(ws), ws.numel(),
-                                           _stream()))
-    return (H, out_pairs, out_scores, out_counts) + ((mask,) if want_mask else ())
+    _lib.check(getattr(lib, fn)(_ptr(k1), F1, _ptr(k2), F2, _ptr(pair_index), P, N, M, _ptr(pr),
+                                _ptr(ps), _ptr(cn), L, int(iters), float(threshold),
+                                int(seed) & 0xFFFFFFFFFFFFFFFF, _ptr(G), _ptr(out_pairs),
+                                _ptr(out_scores), _ptr(out_counts), _ptr(mask), _ptr(ws), ws.numel(),
+                                _stream()))
+    return (G, out_pairs, out_scores, out_counts) + ((mask,) if want_mask else ())
 
 
-def ransac_workspace_views(workspace, P, L, iters):
-    """Views of what sslam_ransac_homography leaves at the start of its workspace: per-hypothesis inlier
-    counts (P,iters) int32 (-1 degenerate), best hypothesis (P,) int32 (-1 none), and the best
-    hypothesis's inlier mask before the refit (P,L) uint8."""
+def ransac_workspace_views(workspace, P, L, iters, model="homography"):
+    """Views of what sslam_ransac_homography (model="homography") or sslam_ransac_fundamental
+    (model="fundamental") leaves at the start of its workspace: per-slot inlier counts (P,S) int32 (-1
+    degenerate), S = iters for the homography and 3*iters for the fundamental matrix (slots 3s..3s+2
+    belong to sample s); the best slot (P,) int32 (-1 none); and the best slot's inlier mask before the
+    refit (P,L) uint8."""
     def up(x):
         return (x + 255) // 256 * 256
-    o_best = up(P * iters * 4)
+    S = iters * _RANSAC_SYMBOLS[model][2]
+    o_best = up(P * S * 4)
     o_mask = o_best + up(P * 4)
     w = workspace
-    return (w[:P * iters * 4].view(torch.int32).reshape(P, iters),
+    return (w[:P * S * 4].view(torch.int32).reshape(P, S),
             w[o_best:o_best + P * 4].view(torch.int32),
             w[o_mask:o_mask + P * L].reshape(P, L))
 

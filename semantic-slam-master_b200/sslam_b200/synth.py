@@ -7,9 +7,11 @@ is a crop window sliding over a fixed "world canvas" (TUM fr1/desk-like small mo
 every 8 frames), so consecutive frames overlap and mutual matches exist.
 
 All randomness comes from ``torch.Generator`` objects with the seeds listed in SURVEY.md §8(d);
-identical tensors are handed to the oracle and to the kernels.
+identical tensors are handed to the oracle and to the kernels.  The keypoint-level two-view banks at the
+end (``two_view_bank``, ``two_view_lists``), for epipolar geometry, are drawn with NumPy generators.
 """
 
+import numpy as np
 import torch
 import torch.nn.functional as F
 
@@ -99,3 +101,69 @@ def noisy_permutation_descriptors(n, d=256, noise=0.05, seed=0, m=None):
         b = torch.cat([b, torch.randn(m - n, d, generator=g)], 0)
     b = F.normalize(b, dim=-1)
     return a.contiguous(), b.contiguous(), perm
+
+
+def _rotation(w):
+    """Rodrigues: axis-angle vector (3,) -> rotation matrix (3,3)."""
+    th = float(np.linalg.norm(w))
+    if th == 0.0:
+        return np.eye(3)
+    k = np.asarray(w, dtype=np.float64) / th
+    Kx = np.array([[0, -k[2], k[1]], [k[2], 0, -k[0]], [-k[1], k[0], 0]])
+    return np.eye(3) + np.sin(th) * Kx + (1.0 - np.cos(th)) * (Kx @ Kx)
+
+
+def two_view_bank(num_sets=2, num_points=2048, seed=0, noise=0.0, baseline=(0.2, 0.4), direction=None,
+                  focal=525.0, height=480, width=640):
+    """Keypoint banks of one static 3-D scene seen by a moving pinhole camera (general motion, so the
+    epipolar geometry is identifiable — unlike make_sequence, whose frames are translated crops of a flat
+    canvas).  Point k is drawn at a uniform pixel of set 0 and a depth of 4-10 m; each later camera pose
+    moves by a small random rotation (0.02-0.05 rad) and a translation of ``baseline`` (m, uniform) in a
+    random direction, or along ``direction`` (3,) when given (a sideways motion keeps the epipoles far
+    outside the image, where the epipolar lines constrain every point).
+    Keypoint k of every set is the projection of point k (plus ``noise`` px Gaussian), rounded to fp32.
+
+    Returns (bank (num_sets, num_points, 2) float32 ndarray in the [F,K,2] layout, F (num_sets-1, 3, 3)
+    float64): F[s] is the true fundamental matrix of sets (s, s+1), x_{s+1}^T F x_s = 0, at unit Frobenius
+    norm with its largest-|entry| element positive."""
+    rng = np.random.default_rng(seed)
+    K = np.array([[focal, 0.0, (width - 1) / 2.0], [0.0, focal, (height - 1) / 2.0], [0.0, 0.0, 1.0]])
+    Ki = np.linalg.inv(K)
+    pix = rng.uniform([0.0, 0.0], [width - 1.0, height - 1.0], size=(num_points, 2))
+    X = (np.concatenate([pix, np.ones((num_points, 1))], 1) @ Ki.T) * rng.uniform(4.0, 10.0, (num_points, 1))
+    bank = np.empty((num_sets, num_points, 2))
+    Fs = np.empty((max(num_sets - 1, 0), 3, 3))
+    for s in range(num_sets):
+        if s:
+            axis = rng.normal(size=3)
+            R = _rotation(axis / np.linalg.norm(axis) * rng.uniform(0.02, 0.05))
+            t = rng.normal(size=3) if direction is None else np.asarray(direction, dtype=np.float64).copy()
+            t *= rng.uniform(*baseline) / np.linalg.norm(t)
+            X = X @ R.T + t
+            tx = np.array([[0, -t[2], t[1]], [t[2], 0, -t[0]], [-t[1], t[0], 0]])
+            Fm = Ki.T @ tx @ R @ Ki
+            Fm /= np.linalg.norm(Fm)
+            Fs[s - 1] = -Fm if Fm.reshape(9)[np.abs(Fm).argmax()] < 0 else Fm
+        p = X @ K.T
+        bank[s] = p[:, :2] / p[:, 2:3] + (rng.normal(0.0, noise, (num_points, 2)) if noise > 0 else 0.0)
+    return bank.astype(np.float32), Fs
+
+
+def two_view_lists(counts, list_stride, num_points, inlier_frac=0.7, seed=1):
+    """Padded match lists over two_view_bank sets: list p holds counts[p] rows (i, j) with ascending
+    distinct i; j = i (a true correspondence) with probability ``inlier_frac``, a uniform keypoint
+    otherwise.  -> pairs (P, L, 2) int32 (-1 padded), scores (P, L) fp32, counts (P,) int32, true (P, L)
+    bool (j = i)."""
+    rng = np.random.default_rng(seed)
+    P = len(counts)
+    pairs = np.full((P, list_stride, 2), -1, dtype=np.int32)
+    scores = np.zeros((P, list_stride), dtype=np.float32)
+    true = np.zeros((P, list_stride), dtype=bool)
+    for p, n in enumerate(counts):
+        i = np.sort(rng.choice(num_points, size=int(n), replace=False))
+        keep = rng.random(int(n)) < inlier_frac
+        j = np.where(keep, i, rng.integers(0, num_points, size=int(n)))
+        pairs[p, :n, 0], pairs[p, :n, 1] = i, j
+        scores[p, :n] = rng.random(int(n)).astype(np.float32)
+        true[p, :n] = j == i
+    return pairs, scores, np.asarray(counts, dtype=np.int32), true
