@@ -319,6 +319,53 @@ int sslam_ransac_fundamental(const float* kpts1, int F1, const float* kpts2, int
                              void* ws, size_t ws_bytes, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
+ * Relative pose from verified match lists: the camera motion (R, t) of each of P pairs and the
+ * triangulated points, in one launch (one CTA per pair), without workspace or host synchronisation
+ * (capturable in a CUDA graph), without atomics; a pair's result does not depend on its position in the
+ * batch.  The banks, pair_index and the padded lists are those of sslam_ransac_fundamental (typically its
+ * out_pairs / out_scores / out_counts); rows k < min(counts[p], L) are used.  E [P,9] double row-major is
+ * the essential matrix of each pair (K^T F K); one pinhole camera K = [[fx,0,cx],[0,fy,cy],[0,0,1]] is
+ * shared by both images of every pair.  A row is usable when its keypoint indices are in range and its
+ * coordinates finite; any other row is never good and stays out of the refinement.
+ *   Decomposition (double): E / |E|_F; the eigenvectors of E^T E by cyclic Jacobi, ordered by descending
+ *   eigenvalue (lowest index on ties), v3 negated when det V < 0; u1 = normalise(E v1), u2 =
+ *   normalise(E v2 - (u1.E v2) u1), u3 = u1 x u2; with W = [[0,1,0],[-1,0,0],[0,0,1]] (cv2's),
+ *   R_a = U W V^T, R_b = U W^T V^T, t = u3; the candidates are (R_a, t), (R_b, t), (R_a, -t), (R_b, -t).
+ *   Cheirality (double, correctly rounded operations): rays f1 = K^-1 x1, f2 = K^-1 x2, u = R f1;
+ *   a = u.u, b = u.f2, c = f2.f2, d = u.t, e = f2.t, den = a c - b^2, z1 = (b e - c d) / den, X1 = z1 f1
+ *   (camera-1 frame, |t| = 1).  A row is good iff den > 1e-12 a c, 0 < z1 < distance_thresh and
+ *   0 < (R X1 + t)_z < distance_thresh (cv2.recoverPose's cheirality and distanceThresh).  The candidate
+ *   with the most good rows is chosen, the lowest on ties.
+ *   Refinement (refine_iters Levenberg-Marquardt trials, 0 disables it; skipped with fewer than 5 usable
+ *   rows): R <- Exp(w) R (Rodrigues), t <- normalise(t + d1 b1 + d2 b2) with b1 = normalise(t x e_i),
+ *   i = argmin |t_i| (lowest on ties), b2 = t x b1; residual the signed Sampson distance in pixels of every
+ *   usable row, x2^T F x1 / sqrt((F x1)_0^2 + (F x1)_1^2 + (F^T x2)_0^2 + (F^T x2)_1^2), F = K^-T [t]x R K^-1
+ *   (0 when the denominator is 0); analytic Jacobian dE/dw_j = [t]x [e_j]x R, dE/dd_j = [b_j]x R.  J^T J,
+ *   J^T r and r^T r are reduced in fixed order once per relinearisation; lambda starts at 1e-3 times the
+ *   mean of diag(J^T J); each trial solves (J^T J + lambda diag(J^T J)) x = -J^T r by Cholesky and costs
+ *   the candidate; it is accepted iff the cost strictly decreases (lambda /= 10, relinearise), otherwise
+ *   lambda *= 10.  The candidate's sign and branch never change.
+ *   Outputs: R [P,9] and t [P,3] (unit; x2 ~ R x1 + t in camera coordinates); cand_good [P,4] the four
+ *   candidates' good rows before the refinement (may be NULL); rms [P,2] the RMS Sampson distance (px)
+ *   over the usable rows before and after the refinement (may be NULL); with the refined pose the
+ *   cheirality is run again: pose_mask [P,L] uint8 the good rows (may be NULL), points [P,L,3] fp32 X1 of
+ *   every good row and 0 elsewhere (may be NULL), and the good rows in input order as out_pairs [P,L,2]
+ *   (-1 padded), out_scores [P,L] (0 padded), out_counts [P] — the matcher's list format.
+ *   No pose is data: E all zeros (the fundamental RANSAC's "no model"), E not finite, sigma2 <= 1e-12
+ *   sigma1, or no good row for the best candidate give R, t, rms, mask and points all zeros and an empty
+ *   list, and SSLAM_OK.
+ * Limits: L <= 16384, 0 <= refine_iters <= 100, distance_thresh > 0 and finite, fx, fy > 0 and finite,
+ * cx, cy finite.
+ */
+int sslam_recover_pose(const float* kpts1, int F1, const float* kpts2, int F2, const int32_t* pair_index,
+                       int P, int N, int M, const double* E, const int32_t* pairs, const float* pair_scores,
+                       const int32_t* counts, int L, double fx, double fy, double cx, double cy,
+                       double distance_thresh, int refine_iters,
+                       double* R, double* t, int32_t* cand_good, double* rms,
+                       float* points, int32_t* out_pairs, float* out_scores,
+                       int32_t* out_counts, uint8_t* pose_mask, void* stream);
+
+/* ---------------------------------------------------------------------------------------------
  * Optional cell-softmax front stage of the decode (north_star "softmax/depth-to-space ... border
  * mask"; OFF by default — the reference code has no such mode, keypoint_selector.py:61-62 is a
  * sigmoid; the vocabulary is papers/pdfs/SuperPoint_DeTone.md:49-58):

@@ -1,0 +1,146 @@
+// Device helpers shared by the per-pair geometry kernels (ransac.cu, pose.cu): the padded match-list
+// accessors, correctly rounded double arithmetic, the fixed-order block reductions, cyclic Jacobi and the
+// order-preserving compaction into the matcher's list format.
+#pragma once
+
+#include "common.cuh"
+
+namespace sslam {
+namespace {
+
+constexpr int GEO_THREADS = 256;      // threads of the one-CTA-per-pair kernels (refit, pose)
+
+// Rows of pair p, clamped to the list stride; 0 when the pair's frame ids are out of range.  Pm has the
+// fields k1, k2, F1, F2, pair_index, N, M, pairs, counts, L of the C ABI's list arguments.
+template <class Pm>
+__device__ __forceinline__ int pair_rows(const Pm& r, int p, int& a, int& b) {
+  a = p; b = p;
+  if (r.pair_index) { a = r.pair_index[2 * p]; b = r.pair_index[2 * p + 1]; }
+  if (a < 0 || a >= r.F1 || b < 0 || b >= r.F2) return 0;
+  return min(max(r.counts[p], 0), r.L);
+}
+
+// Correspondence of row k as (x1, y1, x2, y2); NaN (never an inlier, degenerate sample) when the
+// row's keypoint indices are out of range.
+template <class Pm>
+__device__ __forceinline__ float4 corr(const Pm& r, int p, int a, int b, int k) {
+  const int2 ij = reinterpret_cast<const int2*>(r.pairs)[(size_t)p * r.L + k];
+  if (ij.x < 0 || ij.x >= r.N || ij.y < 0 || ij.y >= r.M) {
+    const float nan = __int_as_float(0x7fc00000);
+    return make_float4(nan, nan, nan, nan);
+  }
+  const float2 u = reinterpret_cast<const float2*>(r.k1)[(size_t)a * r.N + ij.x];
+  const float2 v = reinterpret_cast<const float2*>(r.k2)[(size_t)b * r.M + ij.y];
+  return make_float4(u.x, u.y, v.x, v.y);
+}
+
+__device__ __forceinline__ double dmul(double a, double b) { return __dmul_rn(a, b); }
+__device__ __forceinline__ double dadd(double a, double b) { return __dadd_rn(a, b); }
+__device__ __forceinline__ double dsub(double a, double b) { return __dadd_rn(a, -b); }
+
+// Fixed-order block sum of R doubles per thread over GEO_THREADS threads: warp butterflies, then warps
+// in order.
+template <int R>
+__device__ __forceinline__ void block_sum(double (&v)[R], double* red /* [GEO_THREADS/32][R] */,
+                                          double* out /* [R] */) {
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+#pragma unroll
+  for (int i = 0; i < R; ++i) {
+    double x = v[i];
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) x = dadd(x, __shfl_xor_sync(0xffffffffu, x, o));
+    if (lane == 0) red[warp * R + i] = x;
+  }
+  __syncthreads();
+  if (threadIdx.x < R) {
+    double s = red[threadIdx.x];
+    for (int w = 1; w < GEO_THREADS / 32; ++w) s = dadd(s, red[w * R + threadIdx.x]);
+    out[threadIdx.x] = s;
+  }
+  __syncthreads();
+}
+
+// Cyclic Jacobi on a symmetric NxN (one thread, shared or local memory): on return the diagonal of A
+// holds the eigenvalues and column i of V the eigenvector of A[i][i].
+template <int N>
+__device__ __forceinline__ void jacobi_eigen(double* A, double* V) {
+  for (int i = 0; i < N * N; ++i) V[i] = (i % (N + 1) == 0) ? 1.0 : 0.0;
+  for (int sweep = 0; sweep < 50; ++sweep) {
+    double off = 0.0, tot = 0.0;
+    for (int i = 0; i < N; ++i)
+      for (int j = 0; j < N; ++j) {
+        const double e = A[N * i + j] * A[N * i + j];
+        tot += e;
+        if (i != j) off += e;
+      }
+    if (!(off > 1e-30 * tot)) break;
+    for (int p = 0; p < N - 1; ++p)
+      for (int q = p + 1; q < N; ++q) {
+        const double apq = A[N * p + q];
+        if (apq == 0.0) continue;
+        const double theta = (A[N * q + q] - A[N * p + p]) / (2.0 * apq);
+        const double t = (theta >= 0.0 ? 1.0 : -1.0) / (fabs(theta) + sqrt(theta * theta + 1.0));
+        const double c = 1.0 / sqrt(t * t + 1.0), s = t * c;
+        for (int k = 0; k < N; ++k) {                    // A <- A J (columns p, q)
+          const double akp = A[N * k + p], akq = A[N * k + q];
+          A[N * k + p] = c * akp - s * akq;
+          A[N * k + q] = s * akp + c * akq;
+        }
+        for (int k = 0; k < N; ++k) {                    // A <- J^T A (rows p, q)
+          const double apk = A[N * p + k], aqk = A[N * q + k];
+          A[N * p + k] = c * apk - s * aqk;
+          A[N * q + k] = s * apk + c * aqk;
+        }
+        for (int k = 0; k < N; ++k) {                    // V <- V J
+          const double vkp = V[N * k + p], vkq = V[N * k + q];
+          V[N * k + p] = c * vkp - s * vkq;
+          V[N * k + q] = s * vkp + c * vkq;
+        }
+      }
+  }
+}
+
+// The eigenvector of the smallest eigenvalue of a symmetric NxN (lowest index on ties) in v_out.
+template <int N>
+__device__ void jacobi_smallest(double* A, double* V, double* v_out) {
+  jacobi_eigen<N>(A, V);
+  int m = 0;
+  for (int i = 1; i < N; ++i) if (A[(N + 1) * i] < A[(N + 1) * m]) m = i;
+  for (int k = 0; k < N; ++k) v_out[k] = V[N * k + m];
+}
+
+// Order-preserving compaction of the rows k < n with flag[k] set into list p of the matcher's format
+// (rows (i, j) -1 padded, scores 0 padded, stride L); every thread of the block calls it.  scan: int
+// [GEO_THREADS] shared scratch, s_total: shared.  Returns the number of rows kept.
+__device__ __forceinline__ int compact_rows(const uint8_t* flag, int n, int L, int p, const int32_t* pairs,
+                                            const float* pair_scores, int32_t* out_pairs, float* out_scores,
+                                            int* scan, int* s_total) {
+  const int tid = threadIdx.x;
+  const int seg = (n + GEO_THREADS - 1) / GEO_THREADS;
+  const int beg = min(n, tid * seg), end = min(n, beg + seg);
+  int cnt = 0;
+  for (int k = beg; k < end; ++k) cnt += flag[k];
+  scan[tid] = cnt;
+  __syncthreads();
+  for (int o = 1; o < GEO_THREADS; o <<= 1) {
+    const int v = (tid >= o) ? scan[tid - o] : 0;
+    __syncthreads();
+    scan[tid] += v;
+    __syncthreads();
+  }
+  int pos = scan[tid] - cnt;
+  if (tid == GEO_THREADS - 1) *s_total = scan[GEO_THREADS - 1];
+  __syncthreads();
+  const int total = *s_total;
+  const int2* in_pr = reinterpret_cast<const int2*>(pairs) + (size_t)p * L;
+  const float* in_sc = pair_scores + (size_t)p * L;
+  int2* pr = reinterpret_cast<int2*>(out_pairs) + (size_t)p * L;
+  float* ps = out_scores + (size_t)p * L;
+  for (int k = beg; k < end; ++k)
+    if (flag[k]) { pr[pos] = in_pr[k]; ps[pos] = in_sc[k]; ++pos; }
+  for (int k = total + tid; k < L; k += GEO_THREADS) { pr[k] = make_int2(-1, -1); ps[k] = 0.f; }
+  return total;
+}
+
+}  // namespace
+}  // namespace sslam

@@ -22,7 +22,7 @@
 // scoring operation by operation: the hypothesis path uses only correctly rounded operations
 // (__dmul_rn / __dadd_rn / __ddiv_rn / __dsqrt_rn, __fmul_rn / __fadd_rn / __frcp_rn) in fixed orders with
 // fixed iteration counts, so CUDA and NumPy agree bit for bit.
-#include "common.cuh"
+#include "geometry.cuh"
 
 namespace sslam {
 namespace {
@@ -34,7 +34,7 @@ constexpr int HYP_THREADS = 64;
 constexpr int SC_THREADS = 256;
 constexpr int SC_HYPS = 256;          // hypotheses per scoring CTA (32 per warp)
 constexpr int SC_TILE = 4096;         // correspondences staged per tile: 64 KB, three CTAs per SM
-constexpr int RF_THREADS = 256;
+constexpr int RF_THREADS = GEO_THREADS;
 constexpr double PIVOT_TOL = 1e-8;    // |pivot| of the normalised 8x8 / 7x9 solves, |h33| before scaling
 constexpr int BISECT = 64;            // bisection steps per sign-changing bracket of the 7-point cubic
 constexpr double SQRT2 = 1.4142135623730951;
@@ -57,27 +57,6 @@ struct RansacParams {
   uint8_t* hyp_mask;                         // [P,L]            inliers of the best slot
   float* hyp;                                // [P,SLOTS*iters,9]
 };
-
-// Rows of pair p, clamped to the list stride; 0 when the pair's frame ids are out of range.
-__device__ __forceinline__ int pair_rows(const RansacParams& r, int p, int& a, int& b) {
-  a = p; b = p;
-  if (r.pair_index) { a = r.pair_index[2 * p]; b = r.pair_index[2 * p + 1]; }
-  if (a < 0 || a >= r.F1 || b < 0 || b >= r.F2) return 0;
-  return min(max(r.counts[p], 0), r.L);
-}
-
-// Correspondence of row k as (x1, y1, x2, y2); NaN (never an inlier, degenerate sample) when the
-// row's keypoint indices are out of range.
-__device__ __forceinline__ float4 corr(const RansacParams& r, int p, int a, int b, int k) {
-  const int2 ij = reinterpret_cast<const int2*>(r.pairs)[(size_t)p * r.L + k];
-  if (ij.x < 0 || ij.x >= r.N || ij.y < 0 || ij.y >= r.M) {
-    const float nan = __int_as_float(0x7fc00000);
-    return make_float4(nan, nan, nan, nan);
-  }
-  const float2 u = reinterpret_cast<const float2*>(r.k1)[(size_t)a * r.N + ij.x];
-  const float2 v = reinterpret_cast<const float2*>(r.k2)[(size_t)b * r.M + ij.y];
-  return make_float4(u.x, u.y, v.x, v.y);
-}
 
 // Output k (0-based) of the splitmix64 stream seeded with `seed`.
 __device__ __forceinline__ u64 splitmix64(u64 seed, u64 k) {
@@ -105,10 +84,6 @@ __device__ __forceinline__ bool sample_rows(u64 seed, int h, int n, int idx[R]) 
   }
   return got == R;
 }
-
-__device__ __forceinline__ double dmul(double a, double b) { return __dmul_rn(a, b); }
-__device__ __forceinline__ double dadd(double a, double b) { return __dadd_rn(a, b); }
-__device__ __forceinline__ double dsub(double a, double b) { return __dadd_rn(a, -b); }
 
 // H = T2^-1 . Hn . T1 with T = [[s,0,-s*cx],[0,s,-s*cy],[0,0,1]], then scaled to h33 = 1.
 // false when |h33| < PIVOT_TOL or a coefficient is not finite.
@@ -219,49 +194,6 @@ __device__ __forceinline__ bool is_inlier(const float h[9], float4 q, float t2) 
   const float dx = __fsub_rn(__fmul_rn(u, iw), q.z);
   const float dy = __fsub_rn(__fmul_rn(v, iw), q.w);
   return __fadd_rn(__fmul_rn(dx, dx), __fmul_rn(dy, dy)) < t2;
-}
-
-// Cyclic Jacobi on a symmetric NxN (one thread, shared memory); returns the eigenvector of the
-// smallest eigenvalue in v_out.
-template <int N>
-__device__ void jacobi_smallest(double* A, double* V, double* v_out) {
-  for (int i = 0; i < N * N; ++i) V[i] = (i % (N + 1) == 0) ? 1.0 : 0.0;
-  for (int sweep = 0; sweep < 50; ++sweep) {
-    double off = 0.0, tot = 0.0;
-    for (int i = 0; i < N; ++i)
-      for (int j = 0; j < N; ++j) {
-        const double e = A[N * i + j] * A[N * i + j];
-        tot += e;
-        if (i != j) off += e;
-      }
-    if (!(off > 1e-30 * tot)) break;
-    for (int p = 0; p < N - 1; ++p)
-      for (int q = p + 1; q < N; ++q) {
-        const double apq = A[N * p + q];
-        if (apq == 0.0) continue;
-        const double theta = (A[N * q + q] - A[N * p + p]) / (2.0 * apq);
-        const double t = (theta >= 0.0 ? 1.0 : -1.0) / (fabs(theta) + sqrt(theta * theta + 1.0));
-        const double c = 1.0 / sqrt(t * t + 1.0), s = t * c;
-        for (int k = 0; k < N; ++k) {                    // A <- A J (columns p, q)
-          const double akp = A[N * k + p], akq = A[N * k + q];
-          A[N * k + p] = c * akp - s * akq;
-          A[N * k + q] = s * akp + c * akq;
-        }
-        for (int k = 0; k < N; ++k) {                    // A <- J^T A (rows p, q)
-          const double apk = A[N * p + k], aqk = A[N * q + k];
-          A[N * p + k] = c * apk - s * aqk;
-          A[N * q + k] = s * apk + c * aqk;
-        }
-        for (int k = 0; k < N; ++k) {                    // V <- V J
-          const double vkp = V[N * k + p], vkq = V[N * k + q];
-          V[N * k + p] = c * vkp - s * vkq;
-          V[N * k + q] = s * vkp + c * vkq;
-        }
-      }
-  }
-  int m = 0;
-  for (int i = 1; i < N; ++i) if (A[(N + 1) * i] < A[(N + 1) * m]) m = i;
-  for (int k = 0; k < N; ++k) v_out[k] = V[N * k + m];
 }
 
 // ---------------------------------------------------------------------------- homography model
@@ -626,27 +558,6 @@ __global__ void __launch_bounds__(SC_THREADS) ransac_score_kernel(RansacParams r
   for (int t = tid; t < nh; t += SC_THREADS) r.hyp_count[base + t] = cnt[t];
 }
 
-// Fixed-order block sum of R doubles per thread: warp butterflies, then warps in order.
-template <int R>
-__device__ __forceinline__ void block_sum(double (&v)[R], double* red /* [RF_THREADS/32][R] */,
-                                          double* out /* [R] */) {
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-#pragma unroll
-  for (int i = 0; i < R; ++i) {
-    double x = v[i];
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) x = dadd(x, __shfl_xor_sync(0xffffffffu, x, o));
-    if (lane == 0) red[warp * R + i] = x;
-  }
-  __syncthreads();
-  if (threadIdx.x < R) {
-    double s = red[threadIdx.x];
-    for (int w = 1; w < RF_THREADS / 32; ++w) s = dadd(s, red[w * R + threadIdx.x]);
-    out[threadIdx.x] = s;
-  }
-  __syncthreads();
-}
-
 template <class M>
 __global__ void __launch_bounds__(RF_THREADS) ransac_refit_kernel(RansacParams r) {
   __shared__ uint8_t flag[MAX_L];
@@ -759,29 +670,7 @@ __global__ void __launch_bounds__(RF_THREADS) ransac_refit_kernel(RansacParams r
 
   // ---- order-preserving compaction of the kept rows (matcher list format)
   __syncthreads();
-  const int seg = (n + RF_THREADS - 1) / RF_THREADS;
-  const int beg = min(n, tid * seg), end = min(n, beg + seg);
-  int cnt = 0;
-  for (int k = beg; k < end; ++k) cnt += flag[k];
-  scan[tid] = cnt;
-  __syncthreads();
-  for (int o = 1; o < RF_THREADS; o <<= 1) {
-    const int v = (tid >= o) ? scan[tid - o] : 0;
-    __syncthreads();
-    scan[tid] += v;
-    __syncthreads();
-  }
-  int pos = scan[tid] - cnt;
-  if (tid == RF_THREADS - 1) s_total = scan[RF_THREADS - 1];
-  __syncthreads();
-  const int total = s_total;
-  const int2* in_pr = reinterpret_cast<const int2*>(r.pairs) + (size_t)p * r.L;
-  const float* in_sc = r.pair_scores + (size_t)p * r.L;
-  int2* pr = reinterpret_cast<int2*>(r.out_pairs) + (size_t)p * r.L;
-  float* ps = r.out_scores + (size_t)p * r.L;
-  for (int k = beg; k < end; ++k)
-    if (flag[k]) { pr[pos] = in_pr[k]; ps[pos] = in_sc[k]; ++pos; }
-  for (int k = total + tid; k < r.L; k += RF_THREADS) { pr[k] = make_int2(-1, -1); ps[k] = 0.f; }
+  const int total = compact_rows(flag, n, r.L, p, r.pairs, r.pair_scores, r.out_pairs, r.out_scores, scan, &s_total);
   if (r.mask)
     for (int k = tid; k < r.L; k += RF_THREADS) r.mask[(size_t)p * r.L + k] = k < n ? flag[k] : 0;
   if (tid == 0) r.out_counts[p] = total;

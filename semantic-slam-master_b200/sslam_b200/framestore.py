@@ -12,6 +12,8 @@ slots through ``pair_index`` (slot ids), so nothing leaves the device until the 
 ``match_spacings``      frame t against frame t - s for several spacings s at once (one matcher call).
 ``verify_pairs``        RANSAC homography or fundamental matrix over lists those calls returned, from the
                         resident keypoints.
+``relative_poses``      RANSAC fundamental matrix, then the relative pose and the points of a calibrated
+                        camera, from the resident keypoints.
 ``TrackingCounters``    the counters of track_frame_sequence (:166-199) accumulated on the device.
 """
 
@@ -125,6 +127,25 @@ class FrameStore:
         if self.fe.grid != "pixel":
             kp = kp * self.fe.patch + self.fe.patch / 2
         return verify(kp, kp, pairs, scores, counts, pair_index=self.pair_index(frame_pairs), **ransac)
+
+    @torch.no_grad()
+    def relative_poses(self, frame_pairs, pairs, scores, counts, camera, distance_thresh=50.0, refine_iters=10,
+                       want_mask=False, want_points=False, **ransac):
+        """Two-view initialisation for the lists match_pairs / match_spacings returned: verify_pairs with
+        model="fundamental" (``ransac``: threshold, iters, seed), E = K^T F K, then the relative pose of
+        every pair on the resident keypoints.  camera: (fx, fy, cx, cy) or a 3x3 matrix of the frames.
+        Returns (R (P,3,3), t (P,3) unit, F (P,3,3), pose pairs, pose scores, pose counts[, mask (P,L)][,
+        points (P,L,3)]); the pose lists hold the rows of the F inlier lists that lie in front of both
+        cameras.  A pair without an F or without a pose has R, t all zeros and an empty list."""
+        F, vp, vs, vc = self.verify_pairs(frame_pairs, pairs, scores, counts, model="fundamental", **ransac)
+        kp = self.bank["keypoints"]
+        if self.fe.grid != "pixel":
+            kp = kp * self.fe.patch + self.fe.patch / 2
+        out = geometry.recover_pose_device(kp, kp, geometry.essential_from_fundamental(F, camera), vp, vs, vc,
+                                           camera, pair_index=self.pair_index(frame_pairs),
+                                           distance_thresh=distance_thresh, refine_iters=refine_iters,
+                                           want_mask=want_mask, want_points=want_points)
+        return (out[0], out[1], F) + tuple(out[2:5]) + tuple(out[7:])
 
 
 class TrackingCounters:

@@ -1,6 +1,8 @@
 """Geometric verification of match lists on the device (csrc/ransac.cu): RANSAC homography, for planar
 scenes and rotating cameras, and RANSAC fundamental matrix (the epipolar constraint), for a camera that
-translates through a 3-D scene.
+translates through a 3-D scene; and the relative pose (csrc/pose.cu) of a calibrated camera from the
+verified lists: decomposition of E = K^T F K, cheirality, Levenberg-Marquardt refinement of (R, t) and the
+triangulated points.
 
 Device API — ``verify_homography_device`` / ``verify_fundamental_device`` take banks of keypoint sets and
 the padded lists the matcher produced (``pairs [P,N,2]``, ``pair_scores [P,N]``, ``counts [P]``) and
@@ -11,7 +13,8 @@ estimated ``H`` feeds ``evaluation.ground_truth_matches_device`` directly.
 
 Host API — ``find_homography`` has the arguments and the return shape of ``cv2.findHomography(src,
 dst, cv2.RANSAC, thresh)``: ``(H (3,3) float64 or None, mask (n,1) uint8)``; ``find_fundamental`` those
-of ``cv2.findFundamentalMat(pts1, pts2, cv2.FM_RANSAC, thresh)``.
+of ``cv2.findFundamentalMat(pts1, pts2, cv2.FM_RANSAC, thresh)``; ``recover_pose`` those of
+``cv2.recoverPose(E, pts1, pts2, K, distanceThresh)``.
 """
 
 import numpy as np
@@ -84,3 +87,79 @@ def find_fundamental(pts1, pts2, ransac_thresh=3.0, max_iters=1024, seed=0):
     if F is not None and abs(F[2, 2]) > np.finfo(np.float32).eps:
         F = F / F[2, 2]
     return F, mask
+
+
+def _intrinsics(camera):
+    """(fx, fy, cx, cy) or a 3x3 pinhole matrix without skew -> (fx, fy, cx, cy) floats."""
+    K = np.asarray(camera, dtype=np.float64)
+    if K.shape == (4,):
+        return tuple(float(v) for v in K)
+    if K.shape != (3, 3):
+        raise ValueError("camera must be (fx, fy, cx, cy) or a 3x3 camera matrix")
+    if K[0, 1] != 0.0 or K[1, 0] != 0.0 or (K[2] != [0.0, 0.0, 1.0]).any():
+        raise ValueError("camera matrix must be [[fx, 0, cx], [0, fy, cy], [0, 0, 1]] (no skew)")
+    return float(K[0, 0]), float(K[1, 1]), float(K[0, 2]), float(K[1, 2])
+
+
+def essential_from_fundamental(F, camera):
+    """F (P,3,3) on the device, one camera for both images -> E = K^T F K (P,3,3) float64 on the device.
+    Element-wise from the intrinsics (no host copy), so it can be captured in a CUDA graph, and a zero F
+    (no model) stays zero."""
+    fx, fy, cx, cy = _intrinsics(camera)
+    F = F.to(torch.float64)
+    FK = torch.stack([fx * F[..., 0], fy * F[..., 1], cx * F[..., 0] + cy * F[..., 1] + F[..., 2]], -1)
+    return torch.stack([fx * FK[..., 0, :], fy * FK[..., 1, :], cx * FK[..., 0, :] + cy * FK[..., 1, :] + FK[..., 2, :]],
+                       -2)
+
+
+def recover_pose_device(kpts1, kpts2, E, pairs, scores, counts, camera, pair_index=None, distance_thresh=50.0,
+                        refine_iters=10, want_mask=False, want_points=False):
+    """Banks, E (P,3,3) float64 and the verified lists on device (usually verify_fundamental_device's) ->
+    ops.recover_pose's (R (P,3,3), t (P,3), pairs, scores, counts, cand_good (P,4), rms (P,2)[, mask][,
+    points (P,L,3)]) on device.  camera: (fx, fy, cx, cy) or a 3x3 matrix, shared by both images.  A pair
+    without a pose (E zero or of rank < 2, or no row in front of both cameras) has R, t all zeros and an
+    empty list."""
+    fx, fy, cx, cy = _intrinsics(camera)
+    return ops.recover_pose(kpts1, kpts2, E, pairs, scores, counts, fx, fy, cx, cy, pair_index=pair_index,
+                            distance_thresh=distance_thresh, refine_iters=refine_iters, want_mask=want_mask,
+                            want_points=want_points)
+
+
+def recover_pose(E, pts1, pts2, camera_matrix, distance_thresh=50.0, mask=None, refine_iters=10):
+    """cv2.recoverPose(E, pts1, pts2, K, distanceThresh[, mask]) on the device: -> (retval = good rows,
+    R (3,3), t (3,1) unit, mask (n,1) uint8, points (4,n) float64 with w = 1: X in the camera-1 frame for
+    good rows, (0, 0, 0, 1) elsewhere).  Rows whose input ``mask`` is 0 are left out.  refine_iters = 0
+    returns the chosen decomposition candidate, as cv2 does; the default refines it on the Sampson error.
+    Without a pose R and t are zeros and retval is 0.  A camera matrix with skew raises ValueError."""
+    if not torch.cuda.is_available():
+        raise RuntimeError("sslam_b200 needs a CUDA device (no CPU fallback)")
+    cam = _intrinsics(camera_matrix)
+    p1 = np.ascontiguousarray(np.asarray(pts1, dtype=np.float32).reshape(-1, 2))
+    p2 = np.ascontiguousarray(np.asarray(pts2, dtype=np.float32).reshape(-1, 2))
+    if p1.shape != p2.shape:
+        raise ValueError("recover_pose: pts1 and pts2 must hold the same number of points")
+    n = p1.shape[0]
+    use = np.ones(n, bool) if mask is None else np.asarray(mask).reshape(-1) != 0
+    if use.shape[0] != n:
+        raise ValueError("recover_pose: mask must hold one entry per point")
+    dev = torch.device("cuda", torch.cuda.current_device())
+    L = max(n, 1)
+    rows = torch.full((1, L, 2), -1, dtype=torch.int32)
+    idx = torch.as_tensor(np.flatnonzero(use).astype(np.int32))
+    rows[0, :idx.numel(), 0] = idx
+    rows[0, :idx.numel(), 1] = idx
+    k1 = torch.zeros(1, L, 2)                         # at least one row: the C ABI takes no null banks
+    k2 = torch.zeros(1, L, 2)
+    k1[0, :n], k2[0, :n] = torch.as_tensor(p1), torch.as_tensor(p2)
+    Ed = torch.as_tensor(np.asarray(E, dtype=np.float64).reshape(1, 3, 3)).to(dev)
+    R, t, _, _, cnt, _, _, m, X = recover_pose_device(
+        k1.to(dev), k2.to(dev), Ed, rows.to(dev), torch.zeros(1, L, device=dev),
+        torch.tensor([int(idx.numel())], dtype=torch.int32, device=dev), cam, distance_thresh=distance_thresh,
+        refine_iters=refine_iters, want_mask=True, want_points=True)
+    k = idx.numpy()
+    out_mask = np.zeros((n, 1), dtype=np.uint8)
+    out_mask[k, 0] = m[0, :k.size].cpu().numpy()
+    pts = np.zeros((4, n))
+    pts[3] = 1.0
+    pts[:3, k] = X[0, :k.size].cpu().numpy().astype(np.float64).T
+    return int(cnt[0]), R[0].cpu().numpy(), t[0].cpu().numpy().reshape(3, 1), out_mask, pts

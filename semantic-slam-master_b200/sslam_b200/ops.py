@@ -450,6 +450,57 @@ def ransac_workspace_views(workspace, P, L, iters, model="homography"):
             w[o_mask:o_mask + P * L].reshape(P, L))
 
 
+def recover_pose(kpts1, kpts2, E, pairs, pair_scores, counts, fx, fy, cx, cy, pair_index=None, num_pairs=None,
+                 distance_thresh=50.0, refine_iters=10, want_mask=False, want_points=False):
+    """Relative pose per verified match list (sslam_recover_pose).
+
+    kpts1 (F1,N,2), kpts2 (F2,M,2) fp32, pairs (P,L,2) int32, pair_scores (P,L), counts (P,) and pair_index
+    as for ransac_fundamental (usually its output lists); E (P,3,3) or (P,9) float64, one pinhole camera
+    (fx, fy, cx, cy) for both images of every pair.
+    Returns (R (P,3,3) float64, t (P,3) float64 unit with x2 ~ R x1 + t, good pairs (P,L,2) int32 in input
+    order -1 padded, their scores (P,L), counts (P,) int32, cand_good (P,4) int32 — the four candidates'
+    good rows —, rms (P,2) float64 — RMS Sampson distance in px before / after the refinement —[, pose
+    mask (P,L) uint8][, points (P,L,3) fp32 in the camera-1 frame, |t| = 1, zero where a row is not
+    good]).  A pair without a pose has R, t, rms all zeros and an empty list."""
+    lib = _lib.load()
+    _need_cuda(kpts1, kpts2, E, pairs, pair_scores, counts, pair_index)
+    k1, k2 = kpts1.contiguous(), kpts2.contiguous()
+    if k1.dtype != torch.float32 or k2.dtype != torch.float32:
+        raise RuntimeError("recover_pose expects fp32 keypoints")
+    pr = pairs.to(torch.int32).contiguous()
+    ps = pair_scores.to(torch.float32).contiguous()
+    cn = counts.to(torch.int32).contiguous()
+    F1, N = k1.shape[0], k1.shape[1]
+    F2, M = k2.shape[0], k2.shape[1]
+    P, L = pr.shape[0], pr.shape[1]
+    Ed = E.to(torch.float64).reshape(-1, 9).contiguous()
+    if Ed.shape[0] != P:
+        raise RuntimeError("recover_pose: E must hold one matrix per match list")
+    if pair_index is not None:
+        pair_index = pair_index.to(torch.int32).contiguous()
+        if pair_index.shape[0] != P:
+            raise RuntimeError("recover_pose: pair_index must hold one (a, b) row per match list")
+    elif num_pairs is not None and int(num_pairs) != P:
+        raise RuntimeError("recover_pose: num_pairs differs from the number of match lists")
+    dev = pr.device
+    R = torch.empty(P, 3, 3, dtype=torch.float64, device=dev)
+    t = torch.empty(P, 3, dtype=torch.float64, device=dev)
+    cand = torch.empty(P, 4, dtype=torch.int32, device=dev)
+    rms = torch.empty(P, 2, dtype=torch.float64, device=dev)
+    out_pairs = torch.empty(P, L, 2, dtype=torch.int32, device=dev)
+    out_scores = torch.empty(P, L, dtype=torch.float32, device=dev)
+    out_counts = torch.empty(P, dtype=torch.int32, device=dev)
+    mask = torch.empty(P, L, dtype=torch.uint8, device=dev) if want_mask else None
+    points = torch.empty(P, L, 3, dtype=torch.float32, device=dev) if want_points else None
+    _lib.check(lib.sslam_recover_pose(_ptr(k1), F1, _ptr(k2), F2, _ptr(pair_index), P, N, M, _ptr(Ed), _ptr(pr),
+                                      _ptr(ps), _ptr(cn), L, float(fx), float(fy), float(cx), float(cy),
+                                      float(distance_thresh), int(refine_iters), _ptr(R), _ptr(t), _ptr(cand),
+                                      _ptr(rms), _ptr(points), _ptr(out_pairs), _ptr(out_scores), _ptr(out_counts),
+                                      _ptr(mask), _stream()))
+    return (R, t, out_pairs, out_scores, out_counts, cand, rms) + ((mask,) if want_mask else ()) + \
+        ((points,) if want_points else ())
+
+
 # ---------------------------------------------------------------------------------- optional decode front stage (J1)
 def heatmap_from_cells(logits, cell=8, border=0):
     """(B, cell*cell+1, Hc, Wc) fp32 cell logits -> (B, Hc*cell, Wc*cell) heatmap: channel softmax,

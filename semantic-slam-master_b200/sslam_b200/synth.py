@@ -114,7 +114,7 @@ def _rotation(w):
 
 
 def two_view_bank(num_sets=2, num_points=2048, seed=0, noise=0.0, baseline=(0.2, 0.4), direction=None,
-                  focal=525.0, height=480, width=640):
+                  focal=525.0, height=480, width=640, poses=False):
     """Keypoint banks of one static 3-D scene seen by a moving pinhole camera (general motion, so the
     epipolar geometry is identifiable — unlike make_sequence, whose frames are translated crops of a flat
     canvas).  Point k is drawn at a uniform pixel of set 0 and a depth of 4-10 m; each later camera pose
@@ -125,7 +125,10 @@ def two_view_bank(num_sets=2, num_points=2048, seed=0, noise=0.0, baseline=(0.2,
 
     Returns (bank (num_sets, num_points, 2) float32 ndarray in the [F,K,2] layout, F (num_sets-1, 3, 3)
     float64): F[s] is the true fundamental matrix of sets (s, s+1), x_{s+1}^T F x_s = 0, at unit Frobenius
-    norm with its largest-|entry| element positive."""
+    norm with its largest-|entry| element positive.  With ``poses=True`` also the true relative motions
+    R (num_sets-1, 3, 3) and t (num_sets-1, 3) (metres; X_{s+1} = R[s] X_s + t[s] in camera coordinates) and
+    the camera matrix K (3, 3); the bank and F are the same as without (the motions are drawn from the
+    same stream, after set 0's noise, so they cannot be re-derived outside)."""
     rng = np.random.default_rng(seed)
     K = np.array([[focal, 0.0, (width - 1) / 2.0], [0.0, focal, (height - 1) / 2.0], [0.0, 0.0, 1.0]])
     Ki = np.linalg.inv(K)
@@ -133,6 +136,7 @@ def two_view_bank(num_sets=2, num_points=2048, seed=0, noise=0.0, baseline=(0.2,
     X = (np.concatenate([pix, np.ones((num_points, 1))], 1) @ Ki.T) * rng.uniform(4.0, 10.0, (num_points, 1))
     bank = np.empty((num_sets, num_points, 2))
     Fs = np.empty((max(num_sets - 1, 0), 3, 3))
+    Rs, ts = np.empty_like(Fs), np.empty((max(num_sets - 1, 0), 3))
     for s in range(num_sets):
         if s:
             axis = rng.normal(size=3)
@@ -140,12 +144,15 @@ def two_view_bank(num_sets=2, num_points=2048, seed=0, noise=0.0, baseline=(0.2,
             t = rng.normal(size=3) if direction is None else np.asarray(direction, dtype=np.float64).copy()
             t *= rng.uniform(*baseline) / np.linalg.norm(t)
             X = X @ R.T + t
+            Rs[s - 1], ts[s - 1] = R, t
             tx = np.array([[0, -t[2], t[1]], [t[2], 0, -t[0]], [-t[1], t[0], 0]])
             Fm = Ki.T @ tx @ R @ Ki
             Fm /= np.linalg.norm(Fm)
             Fs[s - 1] = -Fm if Fm.reshape(9)[np.abs(Fm).argmax()] < 0 else Fm
         p = X @ K.T
         bank[s] = p[:, :2] / p[:, 2:3] + (rng.normal(0.0, noise, (num_points, 2)) if noise > 0 else 0.0)
+    if poses:
+        return bank.astype(np.float32), Fs, Rs, ts, K
     return bank.astype(np.float32), Fs
 
 
