@@ -366,6 +366,57 @@ int sslam_recover_pose(const float* kpts1, int F1, const float* kpts2, int F2, c
                        int32_t* out_counts, uint8_t* pose_mask, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
+ * Camera tracking: RANSAC P3P over padded 2D-3D match lists, the pose of camera 2 with respect to the
+ * 3-D points of each of P lists.  Three launches for all lists, no host synchronisation (capturable in
+ * a CUDA graph), no atomics; a list's result depends only on its own inputs and (iters, threshold, seed,
+ * refine_iters), never on its position in the batch.
+ *   points [F1,N,3] fp32 are 3-D points in some camera frame (NaN where there is no point), kpts2
+ *   [F2,M,2] fp32 pixels; pair_index [P,2] selects (a, b) per list (NULL: (p, p)); pairs [P,L,2] int32,
+ *   pair_scores [P,L], counts [P] as sslam_match_finalize writes them, row (i, j) pairing points[a][i]
+ *   with kpts2[b][j].  Rows k < n = min(counts[p], L) are used; a row with an index out of range or a
+ *   coordinate that is not finite is never an inlier and makes a sample that holds it degenerate.  One
+ *   pinhole camera K = [[fx,0,cx],[0,fy,cy],[0,0,1]] for camera 2.
+ *   Sample s (0 <= s < iters) draws 4 distinct rows with the sampler of sslam_ransac_homography (draw
+ *   c < 32 is output s*32 + c, repeats redrawn).  Rows 0-2 go to the Lambda Twist P3P solver (Persson
+ *   & Nordberg, ECCV 2018) in double with correctly rounded operations only: bearings y = normalise(
+ *   (u - cx) / fx, (v - cy) / fy, 1); the cubic's root by bisection of [-B, B], B = 1 + max |k_i| (the
+ *   Cauchy bound of the monic cubic), 100 steps; the rank-2 conic's eigenvectors in closed form; up to 5
+ *   Gauss-Newton steps on the depths.  Among the solutions that are finite and put all four points at
+ *   z > 0, row 3 picks the one with the least squared reprojection error (lowest on ties).  A sample is
+ *   degenerate when n < 4, the sampler finds no 4 distinct rows, a row is not usable, the three solver
+ *   points are collinear or coincident (|d12 x d13|^2 <= 1e-12 |d12|^2 |d13|^2, d1j = X1 - Xj), or no
+ *   solution is real and in front of the camera.
+ *   Row k is an inlier of the fp32 hypothesis (R, t) iff Zc > 0 and du^2 + dv^2 < threshold^2, in fp32
+ *   without contraction: Xc = ((R0 X + R1 Y) + R2 Z) + t0 (Yc, Zc likewise), iz = 1 / Zc (correctly
+ *   rounded), du = ((fx Xc) iz + cx) - u, dv = ((fy Yc) iz + cy) - v, (du du + dv dv) < t^2; a NaN is an
+ *   outlier.  cv2.solvePnPRansac uses <= and no depth test.
+ *   The best sample has the most inliers (lowest sample on ties).  With at least 4 inliers and
+ *   refine_iters > 0 its pose is refined by Levenberg-Marquardt in 6 DOF (R <- Exp(w) R, t <- t + d) on
+ *   the reprojection error in pixels of its inliers (2 residuals per row, analytic Jacobian); lambda
+ *   starts at 1e-3 times the mean of diag(J^T J); each trial solves (J^T J + lambda diag(J^T J)) x =
+ *   -J^T r by Cholesky and is accepted iff the cost strictly decreases (lambda /= 10), otherwise
+ *   lambda *= 10.  The refined pose is kept iff it has at least as many inliers over all rows.
+ *   Outputs: R [P,9] and t [P,3] double, x_cam2 ~ R X + t in the points' units; rms [P,2] the RMS
+ *   reprojection error (px) over the best sample's inliers before and after the refinement (the second
+ *   equals the first when the refinement is skipped or not kept; may be NULL); out_pairs, out_scores,
+ *   out_counts and inlier_mask as for sslam_ransac_homography.  No model is data: R, t and rms all
+ *   zeros, an empty list, SSLAM_OK; so is a best sample without any inlier.  On return the workspace starts
+ *   with the inlier count of every sample, int32 [P,iters] (-1: degenerate), then at the next 256-byte
+ *   boundary the best sample per list, int32 [P] (-1: none), then the best sample's inlier mask before the
+ *   refinement, uint8 [P,L], then the fp32 hypotheses.
+ * Limits: L <= 16384, 1 <= iters <= 65536, 0 <= refine_iters <= 100, threshold > 0 and finite, fx, fy > 0
+ * and finite, cx, cy finite.  The workspace holds 52 bytes per sample, so 32 640 lists at 1024 samples
+ * need about 1.7 GB.
+ */
+size_t sslam_ransac_pnp_workspace_bytes(int P, int L, int iters);
+int sslam_ransac_pnp(const float* points, int F1, const float* kpts2, int F2, const int32_t* pair_index,
+                     int P, int N, int M, const int32_t* pairs, const float* pair_scores,
+                     const int32_t* counts, int L, double fx, double fy, double cx, double cy, int iters,
+                     double threshold, uint64_t seed, int refine_iters,
+                     double* R, double* t, double* rms, int32_t* out_pairs, float* out_scores,
+                     int32_t* out_counts, uint8_t* inlier_mask, void* ws, size_t ws_bytes, void* stream);
+
+/* ---------------------------------------------------------------------------------------------
  * Optional cell-softmax front stage of the decode (north_star "softmax/depth-to-space ... border
  * mask"; OFF by default — the reference code has no such mode, keypoint_selector.py:61-62 is a
  * sigmoid; the vocabulary is papers/pdfs/SuperPoint_DeTone.md:49-58):

@@ -129,7 +129,8 @@ extern "C" uint64_t sslam_launch_count(void) { return sslam::g_launches.load(); 
 static const char* const kKindNames[sslam::KK_COUNT] = {
     "decode_scan", "decode_topk", "decode_count", "decode_resolve", "nms", "gather", "l2norm",
     "match_f32", "match_tc", "split_pair", "unpack_cols", "match_finalize", "gemm_f16x3", "layernorm",
-    "eval_points", "cell_softmax", "conv_head", "ransac_hyp", "ransac_score", "ransac_refit", "pose"};
+    "eval_points", "cell_softmax", "conv_head", "ransac_hyp", "ransac_score", "ransac_refit", "pose",
+    "pnp_hyp", "pnp_score", "pnp_refit"};
 
 extern "C" int sslam_profile_enable(int on) {
   std::lock_guard<std::mutex> lk(sslam::g_prof_mu);

@@ -1,6 +1,7 @@
-// Device helpers shared by the per-pair geometry kernels (ransac.cu, pose.cu): the padded match-list
-// accessors, correctly rounded double arithmetic, the fixed-order block reductions, cyclic Jacobi and the
-// order-preserving compaction into the matcher's list format.
+// Device helpers shared by the per-pair geometry kernels (ransac.cu, pose.cu, pnp.cu): the padded
+// match-list accessors, the splitmix64 row sampler, correctly rounded double arithmetic, 3x3 helpers and
+// Rodrigues, the fixed-order block reductions, cyclic Jacobi, the order-preserving compaction into the
+// matcher's list format and the RANSAC workspace layout.
 #pragma once
 
 #include "common.cuh"
@@ -9,6 +10,7 @@ namespace sslam {
 namespace {
 
 constexpr int GEO_THREADS = 256;      // threads of the one-CTA-per-pair kernels (refit, pose)
+constexpr int MAX_DRAWS = 32;         // sampler draws per sample (redraws included)
 
 // Rows of pair p, clamped to the list stride; 0 when the pair's frame ids are out of range.  Pm has the
 // fields k1, k2, F1, F2, pair_index, N, M, pairs, counts, L of the C ABI's list arguments.
@@ -37,6 +39,70 @@ __device__ __forceinline__ float4 corr(const Pm& r, int p, int a, int b, int k) 
 __device__ __forceinline__ double dmul(double a, double b) { return __dmul_rn(a, b); }
 __device__ __forceinline__ double dadd(double a, double b) { return __dadd_rn(a, b); }
 __device__ __forceinline__ double dsub(double a, double b) { return __dadd_rn(a, -b); }
+
+// Output k (0-based) of the splitmix64 stream seeded with `seed`.
+__device__ __forceinline__ u64 splitmix64(u64 seed, u64 k) {
+  u64 z = seed + (k + 1) * 0x9e3779b97f4a7c15ull;
+  z = (z ^ (z >> 30)) * 0xbf58476d1ce4e5b9ull;
+  z = (z ^ (z >> 27)) * 0x94d049bb133111ebull;
+  return z ^ (z >> 31);
+}
+
+// R distinct rows of [0, n) for sample h: draw c uses output h*MAX_DRAWS + c, a repeat is redrawn.
+template <int R>
+__device__ __forceinline__ bool sample_rows(u64 seed, int h, int n, int idx[R]) {
+  int got = 0;
+  for (int c = 0; c < MAX_DRAWS && got < R; ++c) {
+    const u64 u = splitmix64(seed, (u64)h * MAX_DRAWS + c);
+    const int i = (int)(((u >> 32) * (u64)n) >> 32);
+    bool dup = false;
+#pragma unroll
+    for (int q = 0; q < R; ++q) dup |= (q < got && idx[q] == i);
+    if (!dup) {
+#pragma unroll
+      for (int q = 0; q < R; ++q) if (q == got) idx[q] = i;
+      ++got;
+    }
+  }
+  return got == R;
+}
+
+__device__ __forceinline__ double dot3(const double* a, const double* b) {
+  return dadd(dadd(dmul(a[0], b[0]), dmul(a[1], b[1])), dmul(a[2], b[2]));
+}
+
+// C = A B (3x3, row-major).
+__device__ __forceinline__ void mat3(const double* A, const double* B, double* C) {
+  for (int i = 0; i < 3; ++i)
+    for (int j = 0; j < 3; ++j)
+      C[3 * i + j] = dadd(dadd(dmul(A[3 * i], B[j]), dmul(A[3 * i + 1], B[3 + j])), dmul(A[3 * i + 2], B[6 + j]));
+}
+
+__device__ __forceinline__ void skew(const double* v, double* S) {
+  S[0] = 0.0; S[1] = -v[2]; S[2] = v[1];
+  S[3] = v[2]; S[4] = 0.0; S[5] = -v[0];
+  S[6] = -v[1]; S[7] = v[0]; S[8] = 0.0;
+}
+
+__device__ __forceinline__ void cross3(const double* a, const double* b, double* c) {
+  c[0] = dsub(dmul(a[1], b[2]), dmul(a[2], b[1]));
+  c[1] = dsub(dmul(a[2], b[0]), dmul(a[0], b[2]));
+  c[2] = dsub(dmul(a[0], b[1]), dmul(a[1], b[0]));
+}
+
+// Exp(w) by Rodrigues: I + sin(th) K + (1 - cos(th)) K^2, K = [w / th]x, th = |w|; I when th = 0.
+__device__ __forceinline__ void rodrigues(const double* w, double* X) {
+  for (int i = 0; i < 9; ++i) X[i] = (i % 4 == 0) ? 1.0 : 0.0;
+  const double th = __dsqrt_rn(dot3(w, w));
+  if (th > 0.0) {
+    const double k[3] = {__ddiv_rn(w[0], th), __ddiv_rn(w[1], th), __ddiv_rn(w[2], th)};
+    double K[9], K2[9];
+    skew(k, K);
+    mat3(K, K, K2);
+    const double sn = sin(th), cs = dsub(1.0, cos(th));
+    for (int i = 0; i < 9; ++i) X[i] = dadd(dadd(X[i], dmul(sn, K[i])), dmul(cs, K2[i]));
+  }
+}
 
 // Fixed-order block sum of R doubles per thread over GEO_THREADS threads: warp butterflies, then warps
 // in order.
@@ -140,6 +206,22 @@ __device__ __forceinline__ int compact_rows(const uint8_t* flag, int n, int L, i
     if (flag[k]) { pr[pos] = in_pr[k]; ps[pos] = in_sc[k]; ++pos; }
   for (int k = total + tid; k < L; k += GEO_THREADS) { pr[k] = make_int2(-1, -1); ps[k] = 0.f; }
   return total;
+}
+
+// Workspace of the three-launch RANSAC kernels (ransac.cu, pnp.cu): per-slot inlier counts int32
+// [P, slots], the best slot [P], the best slot's pre-refit mask [P, L], the fp32 hypotheses
+// [P, slots, floats]; each part starts at a 256-byte boundary.
+struct WsLayout { size_t count, best, mask, hyp, total; };
+
+inline WsLayout ws_layout(int P, int L, int iters, int slots_per_sample, int floats) {
+  const size_t slots = (size_t)iters * slots_per_sample;
+  WsLayout w;
+  w.count = 0;
+  w.best = align_up((size_t)P * slots * 4, 256);
+  w.mask = w.best + align_up((size_t)P * 4, 256);
+  w.hyp = w.mask + align_up((size_t)P * L, 256);
+  w.total = w.hyp + align_up((size_t)P * slots * floats * 4, 256);
+  return w;
 }
 
 }  // namespace

@@ -44,10 +44,6 @@ struct PoseParams {
   int32_t* out_pairs; float* out_scores; int32_t* out_counts; uint8_t* mask;
 };
 
-__device__ __forceinline__ double dot3(const double* a, const double* b) {
-  return dadd(dadd(dmul(a[0], b[0]), dmul(a[1], b[1])), dmul(a[2], b[2]));
-}
-
 // Normalised rays (K^-1 x) of row k; false when the row is not usable (a keypoint index out of range, or
 // a coordinate that is not finite).
 __device__ __forceinline__ bool rays(const PoseParams& r, int p, int a, int b, int k, double f1[3], double f2[3]) {
@@ -95,25 +91,6 @@ __device__ __forceinline__ double sampson(const double* E, const double f1[3], c
   const double s2 = dot4(l, l);
   s = __dsqrt_rn(s2);
   return s2 > 0.0 ? __ddiv_rn(num, s) : 0.0;
-}
-
-// C = A B (3x3, row-major).
-__device__ __forceinline__ void mat3(const double* A, const double* B, double* C) {
-  for (int i = 0; i < 3; ++i)
-    for (int j = 0; j < 3; ++j)
-      C[3 * i + j] = dadd(dadd(dmul(A[3 * i], B[j]), dmul(A[3 * i + 1], B[3 + j])), dmul(A[3 * i + 2], B[6 + j]));
-}
-
-__device__ __forceinline__ void skew(const double* v, double* S) {
-  S[0] = 0.0; S[1] = -v[2]; S[2] = v[1];
-  S[3] = v[2]; S[4] = 0.0; S[5] = -v[0];
-  S[6] = -v[1]; S[7] = v[0]; S[8] = 0.0;
-}
-
-__device__ __forceinline__ void cross3(const double* a, const double* b, double* c) {
-  c[0] = dsub(dmul(a[1], b[2]), dmul(a[2], b[1]));
-  c[1] = dsub(dmul(a[2], b[0]), dmul(a[0], b[2]));
-  c[2] = dsub(dmul(a[0], b[1]), dmul(a[1], b[0]));
 }
 
 // v / |v|; false when |v| is 0 or not finite.
@@ -230,16 +207,8 @@ __device__ __noinline__ bool lm_candidate(const double* J, double lam, const dou
   bool ok = true;
   for (int i = 0; i < NP; ++i) ok &= isfinite(x[i]);
   if (!ok) return false;
-  double X[9] = {1.0, 0.0, 0.0, 0.0, 1.0, 0.0, 0.0, 0.0, 1.0};
-  const double th = __dsqrt_rn(dot3(x, x));
-  if (th > 0.0) {                                       // Rodrigues
-    const double k[3] = {__ddiv_rn(x[0], th), __ddiv_rn(x[1], th), __ddiv_rn(x[2], th)};
-    double K[9], K2[9];
-    skew(k, K);
-    mat3(K, K, K2);
-    const double sn = sin(th), cs = dsub(1.0, cos(th));
-    for (int i = 0; i < 9; ++i) X[i] = dadd(dadd(X[i], dmul(sn, K[i])), dmul(cs, K2[i]));
-  }
+  double X[9];
+  rodrigues(x, X);
   mat3(X, R, Rn);
   for (int i = 0; i < 3; ++i) tn[i] = dadd(dadd(t[i], dmul(x[3], B[i])), dmul(x[4], B[3 + i]));
   if (!normalise3(tn)) return false;

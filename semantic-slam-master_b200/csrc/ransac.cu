@@ -29,7 +29,6 @@ namespace {
 
 constexpr int MAX_L = 16384;          // list stride limit (refit flags live in shared memory)
 constexpr int MAX_ITERS = 65536;
-constexpr int MAX_DRAWS = 32;         // sampler draws per sample (redraws included)
 constexpr int HYP_THREADS = 64;
 constexpr int SC_THREADS = 256;
 constexpr int SC_HYPS = 256;          // hypotheses per scoring CTA (32 per warp)
@@ -57,33 +56,6 @@ struct RansacParams {
   uint8_t* hyp_mask;                         // [P,L]            inliers of the best slot
   float* hyp;                                // [P,SLOTS*iters,9]
 };
-
-// Output k (0-based) of the splitmix64 stream seeded with `seed`.
-__device__ __forceinline__ u64 splitmix64(u64 seed, u64 k) {
-  u64 z = seed + (k + 1) * 0x9e3779b97f4a7c15ull;
-  z = (z ^ (z >> 30)) * 0xbf58476d1ce4e5b9ull;
-  z = (z ^ (z >> 27)) * 0x94d049bb133111ebull;
-  return z ^ (z >> 31);
-}
-
-// R distinct rows of [0, n) for sample h: draw c uses output h*MAX_DRAWS + c, a repeat is redrawn.
-template <int R>
-__device__ __forceinline__ bool sample_rows(u64 seed, int h, int n, int idx[R]) {
-  int got = 0;
-  for (int c = 0; c < MAX_DRAWS && got < R; ++c) {
-    const u64 u = splitmix64(seed, (u64)h * MAX_DRAWS + c);
-    const int i = (int)(((u >> 32) * (u64)n) >> 32);
-    bool dup = false;
-#pragma unroll
-    for (int q = 0; q < R; ++q) dup |= (q < got && idx[q] == i);
-    if (!dup) {
-#pragma unroll
-      for (int q = 0; q < R; ++q) if (q == got) idx[q] = i;
-      ++got;
-    }
-  }
-  return got == R;
-}
 
 // H = T2^-1 . Hn . T1 with T = [[s,0,-s*cx],[0,s,-s*cy],[0,0,1]], then scaled to h33 = 1.
 // false when |h33| < PIVOT_TOL or a coefficient is not finite.
@@ -676,23 +648,10 @@ __global__ void __launch_bounds__(RF_THREADS) ransac_refit_kernel(RansacParams r
   if (tid == 0) r.out_counts[p] = total;
 }
 
-struct WsLayout { size_t count, best, mask, hyp, total; };
-
-WsLayout ws_layout(int P, int L, int iters, int slots_per_sample) {
-  const size_t slots = (size_t)iters * slots_per_sample;
-  WsLayout w;
-  w.count = 0;
-  w.best = align_up((size_t)P * slots * 4, 256);
-  w.mask = w.best + align_up((size_t)P * 4, 256);
-  w.hyp = w.mask + align_up((size_t)P * L, 256);
-  w.total = w.hyp + align_up((size_t)P * slots * 9 * 4, 256);
-  return w;
-}
-
 template <class M>
 size_t workspace_bytes(int P, int L, int iters) {
   if (P <= 0 || L < 0 || iters <= 0) return 0;
-  return ws_layout(P, L, iters, M::SLOTS).total;
+  return ws_layout(P, L, iters, M::SLOTS, 9).total;
 }
 
 template <class Model>
@@ -712,7 +671,7 @@ int ransac(const float* kpts1, int F1, const float* kpts2, int F2, const int32_t
                 SSLAM_EINVAL, "ransac: null pointer");
   SSLAM_REQUIRE(F1 > 0 && F2 > 0 && (pair_index || (F1 >= P && F2 >= P)), SSLAM_EINVAL,
                 "ransac: banks hold %d / %d sets but %d implicit pairs were requested", F1, F2, P);
-  const WsLayout w = ws_layout(P, L, iters, Model::SLOTS);
+  const WsLayout w = ws_layout(P, L, iters, Model::SLOTS, 9);
   SSLAM_REQUIRE(ws_bytes >= w.total, SSLAM_EWORKSPACE, "ransac: workspace %zu < %zu", ws_bytes, w.total);
   char* base = static_cast<char*>(ws);
   RansacParams r{kpts1, kpts2, F1, F2, pair_index, P, N, M, pairs, pair_scores, counts, L, iters,

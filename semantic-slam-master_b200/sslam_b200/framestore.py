@@ -14,6 +14,8 @@ slots through ``pair_index`` (slot ids), so nothing leaves the device until the 
                         resident keypoints.
 ``relative_poses``      RANSAC fundamental matrix, then the relative pose and the points of a calibrated
                         camera, from the resident keypoints.
+``track_poses``         the pose of each list's second frame against 3-D points attached to its first
+                        frame's keypoints (geometry.point_map), by RANSAC P3P on the resident keypoints.
 ``TrackingCounters``    the counters of track_frame_sequence (:166-199) accumulated on the device.
 """
 
@@ -146,6 +148,32 @@ class FrameStore:
                                            distance_thresh=distance_thresh, refine_iters=refine_iters,
                                            want_mask=want_mask, want_points=want_points)
         return (out[0], out[1], F) + tuple(out[2:5]) + tuple(out[7:])
+
+    @torch.no_grad()
+    def track_poses(self, frame_pairs, pairs, scores, counts, point_maps, camera, threshold=3.0, iters=1024, seed=0,
+                    refine_iters=10):
+        """Camera tracking for the lists match_pairs / match_spacings returned for ``frame_pairs`` (a, b):
+        point_maps (P, Ka, 3) holds, for list p, the 3-D point of each keypoint of frame a (NaN where there is
+        none; geometry.point_map builds it).  Each list is first restricted, in order, to the rows whose point
+        is finite (geometry.rows_with_points: no sample is spent on a row without a point), then the pose of
+        frame b against those
+        points is estimated by RANSAC P3P on the resident keypoints of b.  camera: (fx, fy, cx, cy) or a 3x3
+        matrix of the frames.  Returns (R (P,3,3), t (P,3) in the points' units, pairs, scores, counts): the
+        inlier rows, a subset of the input lists in input order.  A list without a model has R, t all zeros
+        and an empty list."""
+        kp = self.bank["keypoints"]
+        if self.fe.grid != "pixel":
+            kp = kp * self.fe.patch + self.fe.patch / 2
+        maps = point_maps.to(torch.float32).contiguous()
+        rows, sc, n = geometry.rows_with_points(pairs, scores, counts, maps)
+        P = rows.shape[0]
+        dev = rows.device
+        idx = self.pair_index(frame_pairs)
+        idx = torch.stack([torch.arange(P, dtype=torch.int32, device=dev), idx[:, 1]], 1)
+        out = geometry.solve_pnp_device(maps, kp, rows, sc, n, camera,
+                                        pair_index=idx, threshold=threshold, iters=iters, seed=seed,
+                                        refine_iters=refine_iters)
+        return out[:5]
 
 
 class TrackingCounters:

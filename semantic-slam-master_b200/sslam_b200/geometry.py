@@ -1,8 +1,15 @@
 """Geometric verification of match lists on the device (csrc/ransac.cu): RANSAC homography, for planar
 scenes and rotating cameras, and RANSAC fundamental matrix (the epipolar constraint), for a camera that
-translates through a 3-D scene; and the relative pose (csrc/pose.cu) of a calibrated camera from the
+translates through a 3-D scene; the relative pose (csrc/pose.cu) of a calibrated camera from the
 verified lists: decomposition of E = K^T F K, cheirality, Levenberg-Marquardt refinement of (R, t) and the
-triangulated points.
+triangulated points; and camera tracking (csrc/pnp.cu): the pose of a frame against 3-D points already
+triangulated, by RANSAC P3P on 2D-3D match lists with a Levenberg-Marquardt refinement, in the points' units.
+
+Tracking chain — ``recover_pose_device(..., want_mask=True, want_points=True)`` initialises two views (unit
+|t|); ``point_map`` moves its points onto the keypoints of the second frame; the next frame's lists from that
+frame then pair points with keypoints, and ``solve_pnp_device`` gives that frame's pose in the same units,
+so chained poses share one scale (``rows_with_points`` first drops the rows without a point).  ``point_map``
+with the PnP's mask and (R, t) carries the points on.
 
 Device API — ``verify_homography_device`` / ``verify_fundamental_device`` take banks of keypoint sets and
 the padded lists the matcher produced (``pairs [P,N,2]``, ``pair_scores [P,N]``, ``counts [P]``) and
@@ -14,7 +21,8 @@ estimated ``H`` feeds ``evaluation.ground_truth_matches_device`` directly.
 Host API — ``find_homography`` has the arguments and the return shape of ``cv2.findHomography(src,
 dst, cv2.RANSAC, thresh)``: ``(H (3,3) float64 or None, mask (n,1) uint8)``; ``find_fundamental`` those
 of ``cv2.findFundamentalMat(pts1, pts2, cv2.FM_RANSAC, thresh)``; ``recover_pose`` those of
-``cv2.recoverPose(E, pts1, pts2, K, distanceThresh)``.
+``cv2.recoverPose(E, pts1, pts2, K, distanceThresh)``; ``solve_pnp_ransac`` those of
+``cv2.solvePnPRansac(X, uv, K, None, flags=cv2.SOLVEPNP_P3P)``.
 """
 
 import numpy as np
@@ -163,3 +171,117 @@ def recover_pose(E, pts1, pts2, camera_matrix, distance_thresh=50.0, mask=None, 
     pts[3] = 1.0
     pts[:3, k] = X[0, :k.size].cpu().numpy().astype(np.float64).T
     return int(cnt[0]), R[0].cpu().numpy(), t[0].cpu().numpy().reshape(3, 1), out_mask, pts
+
+
+def solve_pnp_device(points, kpts, pairs, scores, counts, camera, pair_index=None, threshold=3.0, iters=1024,
+                     seed=0, refine_iters=10, want_mask=False, workspace=None):
+    """Camera pose per 2D-3D match list on device: points (F1,N,3) fp32 (NaN where a keypoint has no
+    point), keypoints (F2,M,2) fp32 pixels of the camera ``camera`` ((fx, fy, cx, cy) or a 3x3 matrix),
+    padded lists pairing point i with keypoint j -> ops.ransac_pnp's (R (P,3,3), t (P,3), pairs, scores,
+    counts, rms (P,2)[, mask]) on device, x_cam ~ R X + t in the points' units.  A list without a model
+    (fewer than 4 usable rows, or only degenerate samples) has R, t all zeros and an empty list."""
+    fx, fy, cx, cy = _intrinsics(camera)
+    return ops.ransac_pnp(points, kpts, pairs, scores, counts, fx, fy, cx, cy, pair_index=pair_index,
+                          threshold=threshold, iters=iters, seed=seed, refine_iters=refine_iters,
+                          want_mask=want_mask, workspace=workspace)
+
+
+def _log_so3(R):
+    """Rotation matrix -> axis-angle vector (3,) (NumPy; the angle in [0, pi])."""
+    c = np.clip((np.trace(R) - 1.0) / 2.0, -1.0, 1.0)
+    th = float(np.arccos(c))
+    w = np.array([R[2, 1] - R[1, 2], R[0, 2] - R[2, 0], R[1, 0] - R[0, 1]])
+    if th < 1e-7:
+        return 0.5 * w
+    if np.pi - th < 1e-5:                             # near pi: the axis from the symmetric part
+        k = int(np.argmax(np.diag(R)))
+        a = R[:, k] + np.eye(3)[k]
+        a = a / np.linalg.norm(a)
+        if w @ a < 0.0:
+            a = -a
+        return th * a
+    return th / (2.0 * np.sin(th)) * w
+
+
+def solve_pnp_ransac(object_points, image_points, camera_matrix, dist_coeffs=None, iterations_count=1024,
+                     reprojection_error=3.0, seed=0, refine_iters=10):
+    """cv2.solvePnPRansac(objectPoints, imagePoints, K, distCoeffs, iterationsCount=, reprojectionError=,
+    flags=SOLVEPNP_P3P) on the device: (n,3) points, (n,2) pixels -> (retval, rvec (3,1), tvec (3,1),
+    inliers (k,1) int32 or None), x_cam ~ R(rvec) X + tvec.  A row is an inlier when its squared
+    reprojection error is < reprojection_error^2 (cv2: <=) and it lies in front of the camera (cv2 does not
+    test depth).  There is no distortion model: non-zero dist_coeffs raise ValueError.  n < 4 or no model
+    gives (False, zeros, zeros, None).  n <= 16384."""
+    if not torch.cuda.is_available():
+        raise RuntimeError("sslam_b200 needs a CUDA device (no CPU fallback)")
+    if dist_coeffs is not None and np.any(np.asarray(dist_coeffs, dtype=np.float64) != 0.0):
+        raise ValueError("solve_pnp_ransac: lens distortion is not modelled; undistort the points first")
+    cam = _intrinsics(camera_matrix)
+    X = np.ascontiguousarray(np.asarray(object_points, dtype=np.float32).reshape(-1, 3))
+    uv = np.ascontiguousarray(np.asarray(image_points, dtype=np.float32).reshape(-1, 2))
+    if X.shape[0] != uv.shape[0]:
+        raise ValueError("solve_pnp_ransac: object_points and image_points must hold the same number of points")
+    n = X.shape[0]
+    zeros = np.zeros((3, 1))
+    if n < 4:
+        return False, zeros, zeros.copy(), None
+    dev = torch.device("cuda", torch.cuda.current_device())
+    rows = torch.arange(n, dtype=torch.int32).reshape(1, n, 1).expand(1, n, 2).contiguous()
+    R, t, _, _, cnt, _, mask = solve_pnp_device(
+        torch.as_tensor(X).reshape(1, n, 3).to(dev), torch.as_tensor(uv).reshape(1, n, 2).to(dev), rows.to(dev),
+        torch.zeros(1, n, device=dev), torch.tensor([n], dtype=torch.int32, device=dev), cam,
+        threshold=reprojection_error, iters=iterations_count, seed=seed, refine_iters=refine_iters, want_mask=True)
+    R, t = R[0].cpu().numpy(), t[0].cpu().numpy()
+    if not R.any():
+        return False, zeros, zeros.copy(), None
+    inl = np.flatnonzero(mask[0].cpu().numpy()).astype(np.int32).reshape(-1, 1)
+    return True, _log_so3(R).reshape(3, 1), t.reshape(3, 1), inl
+
+
+def point_map(pairs, counts, points, mask, num_keypoints, R=None, t=None):
+    """Carry one step's 3-D points to the keypoints of the next: for list p, every row k < counts[p] with
+    mask[p, k] set and 0 <= j = pairs[p, k, 1] < num_keypoints gives map[p, j] = R[p] points[p, k] + t[p]
+    (points[p, k] without R, t).  A keypoint in several such rows takes the lowest row (a scatter-min of row
+    indices: deterministic).  -> (P, num_keypoints, 3) fp32 on device, NaN where a keypoint has no point.
+    pairs (P,L,2), counts (P,), points (P,L,3) and mask (P,L) index the same rows — for recover_pose_device,
+    its input lists with want_mask / want_points; for solve_pnp_device, its input lists with its mask and
+    its (R, t).  Device-only, no synchronisation, capturable in a CUDA graph."""
+    P, L = pairs.shape[0], pairs.shape[1]
+    K = int(num_keypoints)
+    dev = pairs.device
+    k = torch.arange(L, device=dev)
+    j = pairs[..., 1].to(torch.int64)
+    keep = (k[None] < counts.to(torch.int64)[:, None]) & mask.to(torch.bool) & (j >= 0) & (j < K)
+    col = torch.where(keep, j, torch.full_like(j, K))             # dropped rows go to a spare column
+    first = torch.full((P, K + 1), L, dtype=torch.int64, device=dev)
+    first.scatter_reduce_(1, col, k[None].expand(P, L), reduce="amin", include_self=True)
+    first = first[:, :K]
+    has = first < L
+    if L == 0:
+        return torch.full((P, K, 3), float("nan"), dtype=torch.float32, device=dev)
+    X = points.to(torch.float64).gather(1, first.clamp(max=L - 1)[..., None].expand(P, K, 3))
+    if R is not None:
+        X = torch.einsum("pij,pkj->pki", R.to(torch.float64).reshape(P, 3, 3), X) + \
+            t.to(torch.float64).reshape(P, 1, 3)
+    return torch.where(has[..., None], X, torch.full_like(X, float("nan"))).to(torch.float32)
+
+
+def rows_with_points(pairs, scores, counts, point_maps):
+    """Restrict each list to its rows (i, j) whose point point_maps[p, i] is finite, in input order, so that
+    solve_pnp_device spends no sample on a row without a point.  pairs (P,L,2), scores (P,L), counts (P,),
+    point_maps (P,N,3) -> (pairs (P,L,2) int32 -1 padded, scores (P,L) fp32 0 padded, counts (P,) int32) on
+    device.  No synchronisation, capturable."""
+    P, L = pairs.shape[0], pairs.shape[1]
+    N = point_maps.shape[1]
+    dev = pairs.device
+    k = torch.arange(L, device=dev)
+    i = pairs[..., 0].to(torch.int64)
+    keep = (k[None] < counts.to(torch.int64)[:, None]) & (i >= 0) & (i < N)
+    if N:
+        X = point_maps.gather(1, i.clamp(0, N - 1)[..., None].expand(P, L, 3))
+        keep &= torch.isfinite(X).all(-1)
+    pos = torch.where(keep, keep.to(torch.int64).cumsum(1) - 1, torch.full_like(i, L))   # dropped: spare column
+    rows = torch.full((P, L + 1, 2), -1, dtype=torch.int32, device=dev)
+    rows.scatter_(1, pos[..., None].expand(P, L, 2), pairs.to(torch.int32))
+    sc = torch.zeros(P, L + 1, dtype=torch.float32, device=dev)
+    sc.scatter_(1, pos, scores.to(torch.float32))
+    return rows[:, :L].contiguous(), sc[:, :L].contiguous(), keep.sum(1).to(torch.int32)

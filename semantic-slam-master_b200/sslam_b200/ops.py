@@ -388,11 +388,13 @@ def ransac_fundamental(kpts1, kpts2, pairs, pair_scores, counts, pair_index=None
 
 
 _RANSAC_SYMBOLS = {"homography": ("sslam_ransac_homography", "sslam_ransac_workspace_bytes", 1),
-                   "fundamental": ("sslam_ransac_fundamental", "sslam_ransac_fundamental_workspace_bytes", 3)}
+                   "fundamental": ("sslam_ransac_fundamental", "sslam_ransac_fundamental_workspace_bytes", 3),
+                   "pnp": ("sslam_ransac_pnp", "sslam_ransac_pnp_workspace_bytes", 1)}
 
 
 def ransac_workspace_bytes(P, L, iters, model="homography"):
-    """Workspace bytes ransac_homography / ransac_fundamental need for P lists of stride L."""
+    """Workspace bytes ransac_homography / ransac_fundamental / ransac_pnp (model="pnp") need for P lists of
+    stride L."""
     return getattr(_lib.load(), _RANSAC_SYMBOLS[model][1])(int(P), int(L), int(iters))
 
 
@@ -434,11 +436,11 @@ def _ransac(model, kpts1, kpts2, pairs, pair_scores, counts, pair_index, num_pai
 
 
 def ransac_workspace_views(workspace, P, L, iters, model="homography"):
-    """Views of what sslam_ransac_homography (model="homography") or sslam_ransac_fundamental
-    (model="fundamental") leaves at the start of its workspace: per-slot inlier counts (P,S) int32 (-1
-    degenerate), S = iters for the homography and 3*iters for the fundamental matrix (slots 3s..3s+2
-    belong to sample s); the best slot (P,) int32 (-1 none); and the best slot's inlier mask before the
-    refit (P,L) uint8."""
+    """Views of what sslam_ransac_homography (model="homography"), sslam_ransac_fundamental
+    (model="fundamental") or sslam_ransac_pnp (model="pnp") leaves at the start of its workspace: per-slot
+    inlier counts (P,S) int32 (-1 degenerate), S = iters for the homography and the PnP and 3*iters for the
+    fundamental matrix (slots 3s..3s+2 belong to sample s); the best slot (P,) int32 (-1 none); and the best
+    slot's inlier mask before the refit (P,L) uint8."""
     def up(x):
         return (x + 255) // 256 * 256
     S = iters * _RANSAC_SYMBOLS[model][2]
@@ -499,6 +501,54 @@ def recover_pose(kpts1, kpts2, E, pairs, pair_scores, counts, fx, fy, cx, cy, pa
                                       _ptr(mask), _stream()))
     return (R, t, out_pairs, out_scores, out_counts, cand, rms) + ((mask,) if want_mask else ()) + \
         ((points,) if want_points else ())
+
+
+def ransac_pnp(points, kpts2, pairs, pair_scores, counts, fx, fy, cx, cy, pair_index=None, num_pairs=None,
+               threshold=3.0, iters=1024, seed=0, refine_iters=10, want_mask=False, workspace=None):
+    """Camera pose per padded 2D-3D match list (sslam_ransac_pnp): P3P samples, reprojection inlier test,
+    Levenberg-Marquardt refinement.
+
+    points (F1,N,3) fp32 3-D points (NaN where there is none), kpts2 (F2,M,2) fp32 pixels; pairs (P,L,2)
+    int32 rows (i, j) pairing points[a][i] with kpts2[b][j], pair_scores (P,L), counts (P,), pair_index
+    (P,2) as for ransac_homography; one pinhole camera (fx, fy, cx, cy) for kpts2.  ``iters`` counts
+    4-row samples.
+    Returns (R (P,3,3) float64, t (P,3) float64 with x_cam2 ~ R X + t in the points' units, inlier pairs
+    (P,L,2) int32 in input order -1 padded, their scores (P,L), counts (P,) int32, rms (P,2) float64 — RMS
+    reprojection error in px over the best sample's inliers before / after the refinement —[, inlier mask
+    (P,L) uint8]).  A list without a model has R, t, rms all zeros and an empty list."""
+    lib = _lib.load()
+    _need_cuda(points, kpts2, pairs, pair_scores, counts, pair_index)
+    X, k2 = points.contiguous(), kpts2.contiguous()
+    if X.dtype != torch.float32 or k2.dtype != torch.float32 or X.dim() != 3 or X.shape[-1] != 3:
+        raise RuntimeError("ransac_pnp expects fp32 points (F1,N,3) and fp32 keypoints (F2,M,2)")
+    pr = pairs.to(torch.int32).contiguous()
+    ps = pair_scores.to(torch.float32).contiguous()
+    cn = counts.to(torch.int32).contiguous()
+    F1, N = X.shape[0], X.shape[1]
+    F2, M = k2.shape[0], k2.shape[1]
+    P, L = pr.shape[0], pr.shape[1]
+    if pair_index is not None:
+        pair_index = pair_index.to(torch.int32).contiguous()
+        if pair_index.shape[0] != P:
+            raise RuntimeError("ransac_pnp: pair_index must hold one (a, b) row per match list")
+    elif num_pairs is not None and int(num_pairs) != P:
+        raise RuntimeError("ransac_pnp: num_pairs differs from the number of match lists")
+    dev = pr.device
+    R = torch.empty(P, 3, 3, dtype=torch.float64, device=dev)
+    t = torch.empty(P, 3, dtype=torch.float64, device=dev)
+    rms = torch.empty(P, 2, dtype=torch.float64, device=dev)
+    out_pairs = torch.empty(P, L, 2, dtype=torch.int32, device=dev)
+    out_scores = torch.empty(P, L, dtype=torch.float32, device=dev)
+    out_counts = torch.empty(P, dtype=torch.int32, device=dev)
+    mask = torch.empty(P, L, dtype=torch.uint8, device=dev) if want_mask else None
+    need = lib.sslam_ransac_pnp_workspace_bytes(P, L, int(iters))
+    ws = workspace if workspace is not None else _ws("ransac", need, dev)
+    _lib.check(lib.sslam_ransac_pnp(_ptr(X), F1, _ptr(k2), F2, _ptr(pair_index), P, N, M, _ptr(pr), _ptr(ps),
+                                    _ptr(cn), L, float(fx), float(fy), float(cx), float(cy), int(iters),
+                                    float(threshold), int(seed) & 0xFFFFFFFFFFFFFFFF, int(refine_iters), _ptr(R),
+                                    _ptr(t), _ptr(rms), _ptr(out_pairs), _ptr(out_scores), _ptr(out_counts),
+                                    _ptr(mask), _ptr(ws), ws.numel(), _stream()))
+    return (R, t, out_pairs, out_scores, out_counts, rms) + ((mask,) if want_mask else ())
 
 
 # ---------------------------------------------------------------------------------- optional decode front stage (J1)

@@ -114,7 +114,7 @@ def _rotation(w):
 
 
 def two_view_bank(num_sets=2, num_points=2048, seed=0, noise=0.0, baseline=(0.2, 0.4), direction=None,
-                  focal=525.0, height=480, width=640, poses=False):
+                  focal=525.0, height=480, width=640, poses=False, points=False):
     """Keypoint banks of one static 3-D scene seen by a moving pinhole camera (general motion, so the
     epipolar geometry is identifiable — unlike make_sequence, whose frames are translated crops of a flat
     canvas).  Point k is drawn at a uniform pixel of set 0 and a depth of 4-10 m; each later camera pose
@@ -128,7 +128,10 @@ def two_view_bank(num_sets=2, num_points=2048, seed=0, noise=0.0, baseline=(0.2,
     norm with its largest-|entry| element positive.  With ``poses=True`` also the true relative motions
     R (num_sets-1, 3, 3) and t (num_sets-1, 3) (metres; X_{s+1} = R[s] X_s + t[s] in camera coordinates) and
     the camera matrix K (3, 3); the bank and F are the same as without (the motions are drawn from the
-    same stream, after set 0's noise, so they cannot be re-derived outside)."""
+    same stream, after set 0's noise, so they cannot be re-derived outside).  With ``points=True`` also the
+    true points of every set in that set's camera frame, (num_sets, num_points, 3) float64 (metres; keypoint
+    k of set s is the projection of points[s, k] plus the noise), appended last; this draws no random numbers, so the other
+    arrays are unchanged."""
     rng = np.random.default_rng(seed)
     K = np.array([[focal, 0.0, (width - 1) / 2.0], [0.0, focal, (height - 1) / 2.0], [0.0, 0.0, 1.0]])
     Ki = np.linalg.inv(K)
@@ -137,6 +140,7 @@ def two_view_bank(num_sets=2, num_points=2048, seed=0, noise=0.0, baseline=(0.2,
     bank = np.empty((num_sets, num_points, 2))
     Fs = np.empty((max(num_sets - 1, 0), 3, 3))
     Rs, ts = np.empty_like(Fs), np.empty((max(num_sets - 1, 0), 3))
+    Xs = np.empty((num_sets, num_points, 3))
     for s in range(num_sets):
         if s:
             axis = rng.normal(size=3)
@@ -149,11 +153,10 @@ def two_view_bank(num_sets=2, num_points=2048, seed=0, noise=0.0, baseline=(0.2,
             Fm = Ki.T @ tx @ R @ Ki
             Fm /= np.linalg.norm(Fm)
             Fs[s - 1] = -Fm if Fm.reshape(9)[np.abs(Fm).argmax()] < 0 else Fm
+        Xs[s] = X
         p = X @ K.T
         bank[s] = p[:, :2] / p[:, 2:3] + (rng.normal(0.0, noise, (num_points, 2)) if noise > 0 else 0.0)
-    if poses:
-        return bank.astype(np.float32), Fs, Rs, ts, K
-    return bank.astype(np.float32), Fs
+    return (bank.astype(np.float32), Fs) + ((Rs, ts, K) if poses else ()) + ((Xs,) if points else ())
 
 
 def two_view_lists(counts, list_stride, num_points, inlier_frac=0.7, seed=1):
