@@ -1,7 +1,8 @@
-// Device helpers shared by the per-pair geometry kernels (ransac.cu, pose.cu, pnp.cu): the padded
-// match-list accessors, the splitmix64 row sampler, correctly rounded double arithmetic, 3x3 helpers and
-// Rodrigues, the fixed-order block reductions, cyclic Jacobi, the order-preserving compaction into the
-// matcher's list format and the RANSAC workspace layout.
+// Helpers shared by the per-pair geometry kernels (ransac.cu, pose.cu, pnp.cu): the argument checks of
+// the list entries, the padded match-list accessors, the splitmix64 row sampler, correctly rounded double
+// arithmetic, 3x3 helpers and Rodrigues, the fixed-order block reductions, cyclic Jacobi, the
+// Levenberg-Marquardt loop, the order-preserving compaction into the matcher's list format and the RANSAC
+// workspace layout.
 #pragma once
 
 #include "common.cuh"
@@ -10,7 +11,33 @@ namespace sslam {
 namespace {
 
 constexpr int GEO_THREADS = 256;      // threads of the one-CTA-per-pair kernels (refit, pose)
+constexpr int MAX_L = 16384;          // list stride limit (row flags live in shared memory)
+constexpr int MAX_ITERS = 65536;      // RANSAC samples per list
+constexpr int MAX_REFINE = 100;       // Levenberg-Marquardt trials
 constexpr int MAX_DRAWS = 32;         // sampler draws per sample (redraws included)
+
+// Checks shared by the match-list entries; SSLAM_OK or the code to return, the message prefixed by fn.
+// iters, refine_iters and the intrinsics K = {fx, fy, cx, cy} are checked where the entry takes them (not
+// null); thresh (named thresh_name) must be finite and > 0.  With P == 0 nothing else is needed, so
+// pointers (every required pointer set) and the banks are checked only for P > 0.
+inline int check_list_args(const char* fn, int P, int N, int M, int L, int F1, int F2, const void* pair_index,
+                           bool pointers, const int* iters, const int* refine_iters, const char* thresh_name,
+                           double thresh, const double* K) {
+  SSLAM_REQUIRE(P >= 0 && N >= 0 && M >= 0 && L >= 0, SSLAM_EINVAL, "%s: bad size", fn);
+  SSLAM_REQUIRE(L <= MAX_L, SSLAM_EINVAL, "%s: list stride %d > %d", fn, L, MAX_L);
+  SSLAM_REQUIRE(!iters || (*iters >= 1 && *iters <= MAX_ITERS), SSLAM_EINVAL, "%s: iters=%d (need 1..%d)", fn,
+                *iters, MAX_ITERS);
+  SSLAM_REQUIRE(!refine_iters || (*refine_iters >= 0 && *refine_iters <= MAX_REFINE), SSLAM_EINVAL,
+                "%s: refine_iters=%d (need 0..%d)", fn, *refine_iters, MAX_REFINE);
+  SSLAM_REQUIRE(thresh > 0.0 && isfinite(thresh), SSLAM_EINVAL, "%s: %s must be finite and > 0", fn, thresh_name);
+  SSLAM_REQUIRE(!K || (K[0] > 0.0 && K[1] > 0.0 && isfinite(K[0]) && isfinite(K[1]) && isfinite(K[2]) &&
+                       isfinite(K[3])), SSLAM_EINVAL, "%s: need fx, fy > 0 and finite intrinsics", fn);
+  if (P == 0) return SSLAM_OK;
+  SSLAM_REQUIRE(pointers, SSLAM_EINVAL, "%s: null pointer", fn);
+  SSLAM_REQUIRE(F1 > 0 && F2 > 0 && (pair_index || (F1 >= P && F2 >= P)), SSLAM_EINVAL,
+                "%s: banks hold %d / %d sets but %d implicit lists were requested", fn, F1, F2, P);
+  return SSLAM_OK;
+}
 
 // Rows of pair p, clamped to the list stride; 0 when the pair's frame ids are out of range.  Pm has the
 // fields k1, k2, F1, F2, pair_index, N, M, pairs, counts, L of the C ABI's list arguments.
@@ -124,6 +151,121 @@ __device__ __forceinline__ void block_sum(double (&v)[R], double* red /* [GEO_TH
     out[threadIdx.x] = s;
   }
   __syncthreads();
+}
+
+// ---------------------------------------------------------------------------- Levenberg-Marquardt
+// Accumulators of an NP-parameter refinement: J^T J upper triangle, J^T r, r^T r.
+constexpr int lm_nj(int np) { return np * (np + 1) / 2 + np + 1; }
+
+// Adds one residual r with Jacobian row j to the accumulators.
+template <int NP>
+__device__ __forceinline__ void lm_add(double (&acc)[lm_nj(NP)], const double* j, double r) {
+  int q = 0;
+#pragma unroll
+  for (int i = 0; i < NP; ++i)
+#pragma unroll
+    for (int k = i; k < NP; ++k, ++q) acc[q] = dadd(acc[q], dmul(j[i], j[k]));
+#pragma unroll
+  for (int i = 0; i < NP; ++i) acc[q + i] = dadd(acc[q + i], dmul(j[i], r));
+  acc[lm_nj(NP) - 1] = dadd(acc[lm_nj(NP) - 1], dmul(r, r));
+}
+
+// The damped step (thread 0): (J^T J + lam diag(J^T J)) x = -J^T r by Cholesky.  false: the system is not
+// positive definite or the step is not finite.
+template <int NP>
+__device__ __forceinline__ bool lm_solve(const double* Js, double lam, double x[NP]) {
+  double A[NP][NP], Lc[NP][NP];
+  int q = 0;
+  for (int i = 0; i < NP; ++i)
+    for (int j = i; j < NP; ++j, ++q) A[i][j] = A[j][i] = Js[q];
+  for (int i = 0; i < NP; ++i) A[i][i] = dadd(A[i][i], dmul(lam, A[i][i]));
+  for (int j = 0; j < NP; ++j) {
+    double d = A[j][j];
+    for (int k = 0; k < j; ++k) d = dsub(d, dmul(Lc[j][k], Lc[j][k]));
+    if (!(d > 0.0)) return false;
+    Lc[j][j] = __dsqrt_rn(d);
+    for (int i = j + 1; i < NP; ++i) {
+      double s = A[i][j];
+      for (int k = 0; k < j; ++k) s = dsub(s, dmul(Lc[i][k], Lc[j][k]));
+      Lc[i][j] = __ddiv_rn(s, Lc[j][j]);
+    }
+  }
+  for (int i = 0; i < NP; ++i) {                        // L y = -J^T r
+    double s = -Js[NP * (NP + 1) / 2 + i];
+    for (int k = 0; k < i; ++k) s = dsub(s, dmul(Lc[i][k], x[k]));
+    x[i] = __ddiv_rn(s, Lc[i][i]);
+  }
+  for (int i = NP - 1; i >= 0; --i) {                   // L^T x = y
+    double s = x[i];
+    for (int k = i + 1; k < NP; ++k) s = dsub(s, dmul(Lc[k][i], x[k]));
+    x[i] = __ddiv_rn(s, Lc[i][i]);
+  }
+  bool ok = true;
+  for (int i = 0; i < NP; ++i) ok &= isfinite(x[i]);
+  return ok;
+}
+
+// Levenberg-Marquardt over the rows k < n, every thread of the block (GEO_THREADS) calls it.  Linearise
+// (acc_row(k, acc) adds row k's terms with lm_add, or skips the row), lam = 1e-3 mean diag(J^T J); then,
+// when `refine`, `iters` trials: step(Jsum, lam) forms the candidate on thread 0 (false: no step),
+// cost_row(k, c) adds row k's squared residual under it, a strictly lower cost is accepted (commit() on
+// thread 0, lam / 10, relinearise before the next trial), anything else sets lam * 10.  All sums are
+// fixed-order block sums (red, sum: block_sum scratch of lm_nj(NP) doubles per warp and in all).  Returns
+// (cost0, cost): r^T r at the start and at the end.
+template <int NP, class AccRow, class CostRow, class Step, class Commit>
+__device__ __forceinline__ double2 lm_refine(int n, bool refine, int iters, double* red, double* sum,
+                                             AccRow acc_row, CostRow cost_row, Step step, Commit commit) {
+  constexpr int NJ = lm_nj(NP);
+  __shared__ double Jsum[NJ];
+  __shared__ double s_cost, s_lam;
+  const int tid = threadIdx.x;
+  double cost0 = 0.0;
+  bool relin = true;
+  for (int it = -1; it < (refine ? iters : 0); ++it) {
+    if (relin) {                                        // J^T J, J^T r, r^T r at the current state
+      double acc[NJ];
+#pragma unroll
+      for (int i = 0; i < NJ; ++i) acc[i] = 0.0;
+      for (int k = tid; k < n; k += GEO_THREADS) acc_row(k, acc);
+      block_sum<NJ>(acc, red, sum);
+      if (tid == 0) {
+        for (int i = 0; i < NJ; ++i) Jsum[i] = sum[i];
+        if (it < 0) {
+          s_cost = sum[NJ - 1];
+          double d = 0.0;
+          int q = 0;
+          for (int i = 0; i < NP; q += NP - i, ++i) d = dadd(d, sum[q]);
+          s_lam = dmul(1e-3, __ddiv_rn(d, (double)NP));
+        }
+      }
+      __syncthreads();
+      if (it < 0) cost0 = s_cost;
+      relin = false;
+      if (it < 0) continue;
+    }
+    bool stepped = false;
+    if (tid == 0) stepped = step(Jsum, s_lam);
+    bool accept = false;
+    if (__syncthreads_or(stepped)) {
+      double c1[1] = {0.0};
+      for (int k = tid; k < n; k += GEO_THREADS) cost_row(k, c1[0]);
+      block_sum<1>(c1, red, sum);
+      accept = sum[0] < s_cost;
+    }
+    __syncthreads();
+    if (tid == 0) {
+      if (accept) {
+        s_cost = sum[0];
+        s_lam = __ddiv_rn(s_lam, 10.0);
+        commit();
+      } else {
+        s_lam = dmul(s_lam, 10.0);
+      }
+    }
+    __syncthreads();
+    relin = accept && it + 1 < iters;
+  }
+  return make_double2(cost0, s_cost);
 }
 
 // Cyclic Jacobi on a symmetric NxN (one thread, shared or local memory): on return the diagonal of A

@@ -1,4 +1,6 @@
-// Camera tracking from 2D-3D match lists: batched P3P RANSAC for P lists at once, three launches.
+// Camera tracking from 2D-3D match lists: batched P3P RANSAC for P lists at once, three launches.  The
+// hypothesis and scoring kernels are ransac.cuh's, ransac_hyp<PModel> and ransac_score<PModel>; the refit
+// is this file's.
 //
 //   pnp_hyp    one thread per (list, sample): 4 distinct rows by the splitmix64 sampler; rows 0-2 go to
 //              the Lambda Twist P3P solver (Persson & Nordberg, ECCV 2018) in double, row 3 picks among
@@ -14,57 +16,32 @@
 // atomics.  The hypothesis path uses correctly rounded operations only (__dmul_rn / __dadd_rn / __ddiv_rn
 // / __dsqrt_rn, __fmul_rn / __fadd_rn / __frcp_rn) in fixed orders with fixed iteration counts; oracle/pnp.py
 // restates it operation by operation, so counts, best sample and pre-refit mask agree bit for bit.
-#include "geometry.cuh"
+#include "ransac.cuh"
 
 namespace sslam {
 namespace {
 
-constexpr int MAX_L = 16384;          // list stride limit (refit flags live in shared memory)
-constexpr int MAX_ITERS = 65536;
-constexpr int MAX_REFINE = 100;
-constexpr int HYP_THREADS = 64;
-constexpr int SC_THREADS = 256;
-constexpr int SC_HYPS = 256;          // hypotheses per scoring CTA (32 per warp)
-constexpr int SC_TILE = 3072;         // rows staged per tile: 60 KB + 13 KB static, three CTAs per SM
 constexpr int HF = 12;                // floats per hypothesis: R row-major (9), t (3)
 constexpr int CUBIC_BISECT = 100;     // bisection steps for the root of the P3P cubic
 constexpr int GN_STEPS = 5;           // Gauss-Newton steps on the P3P depths
 constexpr double COLLINEAR_TOL = 1e-12;   // |d12 x d13|^2 <= tol |d12|^2 |d13|^2: collinear or coincident
 constexpr int MIN_REFINE_ROWS = 4;
 constexpr int NP = 6;                 // refinement parameters: w (3), d (3)
-constexpr int NJ = NP * (NP + 1) / 2 + NP + 1;   // J^T J upper triangle, J^T r, r^T r
+constexpr int NJ = lm_nj(NP);
 
-struct PnpParams {
-  const float* k1; const float* k2;          // points [F1,N,3], keypoints [F2,M,2]
-  int F1, F2;
-  const int32_t* pair_index;                 // [P,2] or null
-  int P, N, M;
-  const int32_t* pairs; const float* pair_scores; const int32_t* counts;   // [P,L,2], [P,L], [P]
-  int L, iters, refine_iters;
-  double fx, fy, cx, cy;
-  float t2;                                  // threshold^2 rounded to fp32
-  u64 seed;
-  double* R; double* t; double* rms;         // [P,9], [P,3], [P,2] or null
-  int32_t* out_pairs; float* out_scores; int32_t* out_counts; uint8_t* mask;
-  // workspace
-  int32_t* hyp_count;                        // [P,iters]  inliers per sample, -1 degenerate
-  int32_t* best;                             // [P]        best sample, -1 none
-  uint8_t* hyp_mask;                         // [P,L]      inliers of the best sample
-  float* hyp;                                // [P,iters,12]
-};
+struct PnpRow { float X, Y, Z, u, v; };
 
 // Row k as X, Y, Z (the 3-D point) and u, v (the keypoint); NaN (never an inlier, degenerate sample) when
 // an index is out of range.
-__device__ __forceinline__ void pnp_row(const PnpParams& r, int p, int a, int b, int k, float q[5]) {
+__device__ __forceinline__ PnpRow pnp_row(const RansacParams& r, int p, int a, int b, int k) {
   const int2 ij = reinterpret_cast<const int2*>(r.pairs)[(size_t)p * r.L + k];
   if (ij.x < 0 || ij.x >= r.N || ij.y < 0 || ij.y >= r.M) {
     const float nan = __int_as_float(0x7fc00000);
-    for (int i = 0; i < 5; ++i) q[i] = nan;
-    return;
+    return {nan, nan, nan, nan, nan};
   }
   const float* X = r.k1 + ((size_t)a * r.N + ij.x) * 3;
   const float2 v = reinterpret_cast<const float2*>(r.k2)[(size_t)b * r.M + ij.y];
-  q[0] = X[0]; q[1] = X[1]; q[2] = X[2]; q[3] = v.x; q[4] = v.y;
+  return {X[0], X[1], X[2], v.x, v.y};
 }
 
 // Roots of x^2 + b x + c (Lambda Twist's root2real, a negative discriminant clamped to 0).
@@ -229,19 +206,15 @@ __device__ __noinline__ int p3p(const double y[3][3], const double x[3][3], doub
   return nsol;
 }
 
-// Pose of sample s of list p (false: degenerate).  Rows 0-2 of the sample go to p3p; among its solutions
-// that are finite and put all four points at z > 0, row 3 picks the one with the least squared
+// Pose (R row-major, t) of the sample's rows q (false: degenerate).  Rows 0-2 go to p3p; among its
+// solutions that are finite and put all four points at z > 0, row 3 picks the one with the least squared
 // reprojection error (fx Xc / Zc + cx - u)^2 + (fy Yc / Zc + cy - v)^2, the lowest solution on ties.
-__device__ bool sample_pose(const PnpParams& r, int p, int a, int b, int n, int s, double R[9], double t[3]) {
-  int idx[4] = {-1, -1, -1, -1};
-  if (n < 4 || !sample_rows<4>(r.seed, s, n, idx)) return false;
+__device__ bool sample_pose(const PnpRow q[4], const RansacParams& r, double H[HF]) {
   double X[4][3], uv[4][2];
   bool fin = true;
   for (int k = 0; k < 4; ++k) {
-    float q[5];
-    pnp_row(r, p, a, b, idx[k], q);
-    for (int i = 0; i < 5; ++i) fin &= isfinite(q[i]);
-    X[k][0] = q[0]; X[k][1] = q[1]; X[k][2] = q[2]; uv[k][0] = q[3]; uv[k][1] = q[4];
+    fin &= isfinite(q[k].X) & isfinite(q[k].Y) & isfinite(q[k].Z) & isfinite(q[k].u) & isfinite(q[k].v);
+    X[k][0] = q[k].X; X[k][1] = q[k].Y; X[k][2] = q[k].Z; uv[k][0] = q[k].u; uv[k][1] = q[k].v;
   }
   if (!fin) return false;
   double y[3][3];
@@ -268,96 +241,55 @@ __device__ bool sample_pose(const PnpParams& r, int p, int a, int b, int n, int 
     if (best < 0 || e < be) { best = i; be = e; }
   }
   if (best < 0) return false;
-  for (int j = 0; j < 9; ++j) R[j] = Rs[best][j];
-  for (int j = 0; j < 3; ++j) t[j] = ts[best][j];
+  for (int j = 0; j < 9; ++j) H[j] = Rs[best][j];
+  for (int j = 0; j < 3; ++j) H[9 + j] = ts[best][j];
   return true;
 }
 
 // Inlier test in fp32, no contraction: Xc = ((R0 X + R1 Y) + R2 Z) + t0 (likewise Yc, Zc), iz = rcp(Zc),
 // du = (fx Xc) iz + cx - u, dv = (fy Yc) iz + cy - v; inlier iff Zc > 0 and du du + dv dv < t2.
-__device__ __forceinline__ bool pnp_inlier(const float h[HF], float X, float Y, float Z, float u, float v,
-                                           float fx, float fy, float cx, float cy, float t2) {
-  const float xc = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(h[0], X), __fmul_rn(h[1], Y)), __fmul_rn(h[2], Z)), h[9]);
-  const float yc = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(h[3], X), __fmul_rn(h[4], Y)), __fmul_rn(h[5], Z)), h[10]);
-  const float zc = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(h[6], X), __fmul_rn(h[7], Y)), __fmul_rn(h[8], Z)), h[11]);
-  const float iz = __frcp_rn(zc);
-  const float du = __fsub_rn(__fadd_rn(__fmul_rn(__fmul_rn(fx, xc), iz), cx), u);
-  const float dv = __fsub_rn(__fadd_rn(__fmul_rn(__fmul_rn(fy, yc), iz), cy), v);
-  return zc > 0.f && __fadd_rn(__fmul_rn(du, du), __fmul_rn(dv, dv)) < t2;
-}
-
-__global__ void __launch_bounds__(HYP_THREADS) pnp_hyp_kernel(PnpParams r) {
-  const int p = blockIdx.x;
-  const int s = blockIdx.y * HYP_THREADS + threadIdx.x;
-  if (s >= r.iters) return;
-  int a, b;
-  const int n = pair_rows(r, p, a, b);
-  double R[9], t[3];
-  const bool ok = sample_pose(r, p, a, b, n, s, R, t);
-  const size_t h = (size_t)p * r.iters + s;
-  float* o = r.hyp + h * HF;
-  for (int k = 0; k < 9; ++k) o[k] = ok ? __double2float_rn(R[k]) : 0.f;
-  for (int k = 0; k < 3; ++k) o[9 + k] = ok ? __double2float_rn(t[k]) : 0.f;
-  r.hyp_count[h] = ok ? 0 : -1;
-}
-
-__global__ void __launch_bounds__(SC_THREADS) pnp_score_kernel(PnpParams r, int tile) {
-  extern __shared__ float rows[];                    // [5][tile]: X, Y, Z, u, v
-  __shared__ float hs[SC_HYPS][HF];
-  __shared__ int cnt[SC_HYPS];
-  const int p = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int h0 = blockIdx.y * SC_HYPS;
-  const int nh = min(SC_HYPS, r.iters - h0);
-  int a, b;
-  const int n = pair_rows(r, p, a, b);
-  if (n < 4) return;                                  // every sample of the list is degenerate
+__device__ __forceinline__ bool pnp_inlier(const float h[HF], const PnpRow& q, const RansacParams& r) {
   const float fx = (float)r.fx, fy = (float)r.fy, cx = (float)r.cx, cy = (float)r.cy;
-  float* sX = rows;
-  float* sY = rows + tile;
-  float* sZ = rows + 2 * tile;
-  float* su = rows + 3 * tile;
-  float* sv = rows + 4 * tile;
-  const size_t base = (size_t)p * r.iters + h0;
-  for (int t = tid; t < nh * HF; t += SC_THREADS) hs[t / HF][t % HF] = r.hyp[base * HF + t];
-  for (int t = tid; t < nh; t += SC_THREADS) cnt[t] = r.hyp_count[base + t];
-  for (int k0 = 0; k0 < n; k0 += tile) {
-    const int nt = min(tile, n - k0);
-    __syncthreads();
-    for (int k = tid; k < nt; k += SC_THREADS) {
-      float q[5];
-      pnp_row(r, p, a, b, k0 + k, q);
-      sX[k] = q[0]; sY[k] = q[1]; sZ[k] = q[2]; su[k] = q[3]; sv[k] = q[4];
-    }
-    __syncthreads();
-    for (int hl = warp; hl < nh; hl += SC_THREADS / 32) {
-      if (cnt[hl] < 0) continue;
-      float h[HF];
-#pragma unroll
-      for (int k = 0; k < HF; ++k) h[k] = hs[hl][k];
-      int c = 0;
-      for (int kb = 0; kb < nt; kb += 32) {           // warp-uniform bound: every lane votes
-        const int k = kb + lane;
-        c += __popc(__ballot_sync(0xffffffffu, k < nt && pnp_inlier(h, sX[k], sY[k], sZ[k], su[k], sv[k], fx, fy,
-                                                                     cx, cy, r.t2)));
-      }
-      if (lane == 0) cnt[hl] += c;
-    }
-  }
-  __syncthreads();
-  for (int t = tid; t < nh; t += SC_THREADS) r.hyp_count[base + t] = cnt[t];
+  const float xc = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(h[0], q.X), __fmul_rn(h[1], q.Y)), __fmul_rn(h[2], q.Z)), h[9]);
+  const float yc = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(h[3], q.X), __fmul_rn(h[4], q.Y)), __fmul_rn(h[5], q.Z)), h[10]);
+  const float zc = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(h[6], q.X), __fmul_rn(h[7], q.Y)), __fmul_rn(h[8], q.Z)), h[11]);
+  const float iz = __frcp_rn(zc);
+  const float du = __fsub_rn(__fadd_rn(__fmul_rn(__fmul_rn(fx, xc), iz), cx), q.u);
+  const float dv = __fsub_rn(__fadd_rn(__fmul_rn(__fmul_rn(fy, yc), iz), cy), q.v);
+  return zc > 0.f && __fadd_rn(__fmul_rn(du, du), __fmul_rn(dv, dv)) < r.t2;
 }
 
-// Reprojection residual (px) of one row under (R, t) in double, and optionally its Jacobian along
+// The PnP model of ransac.cuh: 4-row samples, one pose per sample; rows staged as five float arrays
+// (X, Y, Z, u, v): 60 KB at 3072 rows plus 13 KB static, three scoring CTAs per SM.
+struct PModel {
+  static constexpr int SAMPLE = 4, SLOTS = 1, FLOATS = HF, TILE = 3072, ROW_FLOATS = 5;
+  using Row = PnpRow;
+  __device__ static PnpRow row(const RansacParams& r, int p, int a, int b, int k) { return pnp_row(r, p, a, b, k); }
+  __device__ static void stage(float* s, int tile, int k, const PnpRow& q) {
+    s[k] = q.X; s[tile + k] = q.Y; s[2 * tile + k] = q.Z; s[3 * tile + k] = q.u; s[4 * tile + k] = q.v;
+  }
+  __device__ static PnpRow staged(const float* s, int tile, int k) {
+    return {s[k], s[tile + k], s[2 * tile + k], s[3 * tile + k], s[4 * tile + k]};
+  }
+  __device__ static bool inlier(const float h[HF], const PnpRow& q, const RansacParams& r) { return pnp_inlier(h, q, r); }
+  __device__ static int solve(const PnpRow q[SAMPLE], const RansacParams& r, double H[SLOTS][HF]) {
+    return sample_pose(q, r, H[0]) ? 1 : 0;
+  }
+};
+
+// Reprojection residual (px) of one row under H = (R, t) in double, and optionally its Jacobian along
 // (w, d) for R <- Exp(w) R, t <- t + d: dXc/dw_j = e_j x (R X), dXc/dd = I.
-__device__ __forceinline__ void reproj(const double* R, const double* t, const float q[5], double fx, double fy,
-                                       double cx, double cy, double res[2], double (*J)[NP]) {
-  const double X[3] = {q[0], q[1], q[2]};
+__device__ __forceinline__ void reproj(const double* H, const PnpRow& q, double fx, double fy, double cx,
+                                       double cy, double res[2], double (*J)[NP]) {
+  const double* R = H;
+  const double* t = H + 9;
+  const double X[3] = {q.X, q.Y, q.Z};
   const double rx[3] = {dot3(R, X), dot3(R + 3, X), dot3(R + 6, X)};
   const double xc = dadd(rx[0], t[0]), yc = dadd(rx[1], t[1]), zc = dadd(rx[2], t[2]);
   const double iz = __ddiv_rn(1.0, zc);
   const double pu = dmul(xc, iz), pv = dmul(yc, iz);
-  res[0] = dsub(dadd(dmul(fx, pu), cx), (double)q[3]);
-  res[1] = dsub(dadd(dmul(fy, pv), cy), (double)q[4]);
+  res[0] = dsub(dadd(dmul(fx, pu), cx), (double)q.u);
+  res[1] = dsub(dadd(dmul(fy, pv), cy), (double)q.v);
   if (!J) return;
   const double gu[3] = {dmul(fx, iz), 0.0, -dmul(dmul(fx, pu), iz)};
   const double gv[3] = {0.0, dmul(fy, iz), -dmul(dmul(fy, pv), iz)};
@@ -370,235 +302,99 @@ __device__ __forceinline__ void reproj(const double* R, const double* t, const f
   }
 }
 
-// One LM trial (thread 0): solve (J^T J + lam diag(J^T J)) x = -J^T r by Cholesky, candidate
-// Rn = Exp(x_w) R, tn = t + x_d.  false: the system is not positive definite or the step is not finite.
-__device__ __noinline__ bool lm_step(const double* Js, double lam, const double* R, const double* t, double* Rn,
-                                     double* tn) {
-  double A[NP][NP], Lc[NP][NP], x[NP];
-  int q = 0;
-  for (int i = 0; i < NP; ++i)
-    for (int j = i; j < NP; ++j, ++q) A[i][j] = A[j][i] = Js[q];
-  for (int i = 0; i < NP; ++i) A[i][i] = dadd(A[i][i], dmul(lam, A[i][i]));
-  for (int j = 0; j < NP; ++j) {
-    double d = A[j][j];
-    for (int k = 0; k < j; ++k) d = dsub(d, dmul(Lc[j][k], Lc[j][k]));
-    if (!(d > 0.0)) return false;
-    Lc[j][j] = __dsqrt_rn(d);
-    for (int i = j + 1; i < NP; ++i) {
-      double s = A[i][j];
-      for (int k = 0; k < j; ++k) s = dsub(s, dmul(Lc[i][k], Lc[j][k]));
-      Lc[i][j] = __ddiv_rn(s, Lc[j][j]);
-    }
-  }
-  for (int i = 0; i < NP; ++i) {
-    double s = -Js[NP * (NP + 1) / 2 + i];
-    for (int k = 0; k < i; ++k) s = dsub(s, dmul(Lc[i][k], x[k]));
-    x[i] = __ddiv_rn(s, Lc[i][i]);
-  }
-  for (int i = NP - 1; i >= 0; --i) {
-    double s = x[i];
-    for (int k = i + 1; k < NP; ++k) s = dsub(s, dmul(Lc[k][i], x[k]));
-    x[i] = __ddiv_rn(s, Lc[i][i]);
-  }
-  bool ok = true;
-  for (int i = 0; i < NP; ++i) ok &= isfinite(x[i]);
-  if (!ok) return false;
+// One LM trial (thread 0): the damped step x, candidate Rn = Exp(x_w) R, tn = t + x_d (Hn = (Rn, tn)).
+// false: no step.
+__device__ __noinline__ bool lm_step(const double* Js, double lam, const double* H, double* Hn) {
+  double x[NP];
+  if (!lm_solve<NP>(Js, lam, x)) return false;
   double X[9];
   rodrigues(x, X);
-  mat3(X, R, Rn);
-  for (int i = 0; i < 3; ++i) tn[i] = dadd(t[i], x[3 + i]);
+  mat3(X, H, Hn);
+  for (int i = 0; i < 3; ++i) Hn[9 + i] = dadd(H[9 + i], x[3 + i]);
   return true;
 }
 
-// Best sample of list p in double on thread 0 (false: none); not inlined, so that the P3P solve stays out
+// Best sample of list p into H[0] on thread 0 (false: none); not inlined, so that the P3P solve stays out
 // of the row loops' registers.
-__device__ __noinline__ bool best_pose(const PnpParams& r, int p, int a, int b, int n, int best, double* R,
-                                       double* t) {
-  return best >= 0 && sample_pose(r, p, a, b, n, best, R, t);
+__device__ __noinline__ bool best_pose(const RansacParams& r, int p, int a, int b, int n, int best, double (*H)[HF]) {
+  return best >= 0 && sample_hyps<PModel>(r, p, a, b, n, best, H) != 0;
 }
 
 // One CTA per SM (minBlocksPerSM = 1): under the two-CTA register cap of 128, ptxas spills in p3p and
 // best_pose on thread 0's path.
-__global__ void __launch_bounds__(GEO_THREADS, 1) pnp_refit_kernel(PnpParams r) {
+__global__ void __launch_bounds__(GEO_THREADS, 1) pnp_refit_kernel(RansacParams r) {
   __shared__ uint8_t flag[MAX_L];
   __shared__ double red[(GEO_THREADS / 32) * NJ];
   __shared__ double sum[NJ];
-  __shared__ double Jsum[NJ];
-  __shared__ double sR[2][9], st[2][3];               // [0] best sample, [1] refined
-  __shared__ double nR[9], nt[3];                     // LM candidate
-  __shared__ double s_cost, s_lam;
+  __shared__ double sH[2][HF], nH[HF];                // [0] best sample, [1] refined; LM candidate
   __shared__ float hf[HF];
   __shared__ int scan[GEO_THREADS];
   __shared__ unsigned long long bkey[GEO_THREADS / 32];
-  __shared__ int s_best, s_ok, s_total, s_flag;
-  const int p = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  __shared__ int s_best, s_ok, s_total;
+  const int p = blockIdx.x, tid = threadIdx.x;
   int a, b;
   const int n = pair_rows(r, p, a, b);
   const double fx = r.fx, fy = r.fy, cx = r.cx, cy = r.cy;
-  const float fxf = (float)fx, fyf = (float)fy, cxf = (float)cx, cyf = (float)cy;
 
-  // ---- best sample: most inliers, lowest sample on ties
-  unsigned long long key = 0;
-  if (n >= 4)
-    for (int h = tid; h < r.iters; h += GEO_THREADS) {
-      const int c = r.hyp_count[(size_t)p * r.iters + h];
-      const unsigned long long k = ((unsigned long long)(unsigned)(c + 1) << 32) | (0xffffffffu - (unsigned)h);
-      key = k > key ? k : key;
-    }
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) {
-    const unsigned long long k = __shfl_xor_sync(0xffffffffu, key, o);
-    key = k > key ? k : key;
-  }
-  if (lane == 0) bkey[warp] = key;
-  __syncthreads();
+  // ---- best sample
+  best_keys<PModel>(r, p, n, bkey);
   if (tid == 0) {
-    unsigned long long k = 0;
-    for (int w = 0; w < GEO_THREADS / 32; ++w) k = bkey[w] > k ? bkey[w] : k;
-    const int best = (k >> 32) == 0 ? -1 : (int)(0xffffffffu - (unsigned)(k & 0xffffffffu));
-    s_ok = best_pose(r, p, a, b, n, best, sR[0], st[0]);
+    const int best = best_slot(bkey);
+    s_ok = best_pose(r, p, a, b, n, best, sH);
     s_best = s_ok ? best : -1;
-    if (s_ok) {
-      for (int k2 = 0; k2 < 9; ++k2) hf[k2] = __double2float_rn(sR[0][k2]);
-      for (int k2 = 0; k2 < 3; ++k2) hf[9 + k2] = __double2float_rn(st[0][k2]);
-    }
+    if (s_ok)
+      for (int k2 = 0; k2 < HF; ++k2) hf[k2] = __double2float_rn(sH[0][k2]);
   }
   __syncthreads();
   const bool have = s_ok;
-  uint8_t* hm = r.hyp_mask + (size_t)p * r.L;
-  int m = 0;                                          // inliers of the best sample (this thread's rows)
-  for (int k = tid; k < r.L; k += GEO_THREADS) {
-    bool in = false;
-    if (have && k < n) {
-      float q[5];
-      pnp_row(r, p, a, b, k, q);
-      in = pnp_inlier(hf, q[0], q[1], q[2], q[3], q[4], fxf, fyf, cxf, cyf, r.t2);
-    }
-    flag[k] = in;
-    hm[k] = in;
-    m += in;
-  }
-  m = block_reduce_sum(m, scan);                      // scan[] doubles as the reduction scratch (>= 33)
+  const int m = mask_pass<PModel>(r, p, a, b, n, have, hf, flag, scan);
 
   // ---- Levenberg-Marquardt over the best sample's inliers
-  double cost0 = 0.0, cost = 0.0;
+  double2 cost = make_double2(0.0, 0.0);              // r^T r before / after
   bool use_refit = false;
   if (have && m > 0) {
-    if (tid < 9) sR[1][tid] = sR[0][tid];
-    if (tid < 3) st[1][tid] = st[0][tid];
+    if (tid < HF) sH[1][tid] = sH[0][tid];
     __syncthreads();
     const bool refine = r.refine_iters > 0 && m >= MIN_REFINE_ROWS;
-    bool relin = true;
-    for (int it = -1; it < (refine ? r.refine_iters : 0); ++it) {
-      if (relin) {                                    // J^T J, J^T r, r^T r at the current pose
-        double acc[NJ];
+    auto acc_row = [&](int k, double (&acc)[NJ]) {
+      if (!flag[k]) return;
+      double res[2], J[2][NP];
+      reproj(sH[1], pnp_row(r, p, a, b, k), fx, fy, cx, cy, res, J);
 #pragma unroll
-        for (int i = 0; i < NJ; ++i) acc[i] = 0.0;
-        for (int k = tid; k < n; k += GEO_THREADS) {
-          if (!flag[k]) continue;
-          float q[5];
-          pnp_row(r, p, a, b, k, q);
-          double res[2], J[2][NP];
-          reproj(sR[1], st[1], q, fx, fy, cx, cy, res, J);
-#pragma unroll
-          for (int e = 0; e < 2; ++e) {
-            int c = 0;
-#pragma unroll
-            for (int i = 0; i < NP; ++i)
-#pragma unroll
-              for (int j = i; j < NP; ++j, ++c) acc[c] = dadd(acc[c], dmul(J[e][i], J[e][j]));
-#pragma unroll
-            for (int i = 0; i < NP; ++i) acc[c + i] = dadd(acc[c + i], dmul(J[e][i], res[e]));
-            acc[NJ - 1] = dadd(acc[NJ - 1], dmul(res[e], res[e]));
-          }
-        }
-        block_sum<NJ>(acc, red, sum);
-        if (tid == 0) {
-          for (int i = 0; i < NJ; ++i) Jsum[i] = sum[i];
-          if (it < 0) {
-            s_cost = sum[NJ - 1];
-            double d = 0.0;
-            int c = 0;
-            for (int i = 0; i < NP; c += NP - i, ++i) d = dadd(d, sum[c]);
-            s_lam = dmul(1e-3, __ddiv_rn(d, (double)NP));
-          }
-        }
-        __syncthreads();
-        if (it < 0) cost0 = s_cost;
-        relin = false;
-        if (it < 0) continue;
-      }
-      if (tid == 0) s_flag = lm_step(Jsum, s_lam, sR[1], st[1], nR, nt);
-      __syncthreads();
-      bool accept = false;
-      if (s_flag) {
-        double c1[1] = {0.0};
-        for (int k = tid; k < n; k += GEO_THREADS) {
-          if (!flag[k]) continue;
-          float q[5];
-          pnp_row(r, p, a, b, k, q);
-          double res[2];
-          reproj(nR, nt, q, fx, fy, cx, cy, res, nullptr);
-          c1[0] = dadd(c1[0], dadd(dmul(res[0], res[0]), dmul(res[1], res[1])));
-        }
-        block_sum<1>(c1, red, sum);
-        accept = sum[0] < s_cost;
-      }
-      __syncthreads();
-      if (tid == 0) {
-        if (accept) {
-          s_cost = sum[0];
-          s_lam = __ddiv_rn(s_lam, 10.0);
-          for (int i = 0; i < 9; ++i) sR[1][i] = nR[i];
-          for (int i = 0; i < 3; ++i) st[1][i] = nt[i];
-        } else {
-          s_lam = dmul(s_lam, 10.0);
-        }
-      }
-      __syncthreads();
-      relin = accept && it + 1 < r.refine_iters;
-    }
-    cost = s_cost;
+      for (int e = 0; e < 2; ++e) lm_add<NP>(acc, J[e], res[e]);
+    };
+    auto cost_row = [&](int k, double& c) {
+      if (!flag[k]) return;
+      double res[2];
+      reproj(nH, pnp_row(r, p, a, b, k), fx, fy, cx, cy, res, nullptr);
+      c = dadd(c, dadd(dmul(res[0], res[0]), dmul(res[1], res[1])));
+    };
+    auto step = [&](const double* J, double lam) { return lm_step(J, lam, sH[1], nH); };
+    auto commit = [&] {
+      for (int i = 0; i < HF; ++i) sH[1][i] = nH[i];
+    };
+    cost = lm_refine<NP>(n, refine, r.refine_iters, red, sum, acc_row, cost_row, step, commit);
     // ---- re-score with the refined pose: kept iff it has at least as many inliers
     if (refine) {
-      if (tid == 0) {
-        for (int k2 = 0; k2 < 9; ++k2) hf[k2] = __double2float_rn(sR[1][k2]);
-        for (int k2 = 0; k2 < 3; ++k2) hf[9 + k2] = __double2float_rn(st[1][k2]);
-      }
+      if (tid == 0)
+        for (int k2 = 0; k2 < HF; ++k2) hf[k2] = __double2float_rn(sH[1][k2]);
       __syncthreads();
-      int c = 0;
-      for (int k = tid; k < n; k += GEO_THREADS) {
-        float q[5];
-        pnp_row(r, p, a, b, k, q);
-        c += pnp_inlier(hf, q[0], q[1], q[2], q[3], q[4], fxf, fyf, cxf, cyf, r.t2);
-      }
-      c = block_reduce_sum(c, scan);
-      use_refit = c >= m;
+      use_refit = keep_refit<PModel>(r, p, a, b, n, hf, m, scan);
     }
   }
   __syncthreads();
   if (use_refit)
-    for (int k = tid; k < n; k += GEO_THREADS) {
-      float q[5];
-      pnp_row(r, p, a, b, k, q);
-      flag[k] = pnp_inlier(hf, q[0], q[1], q[2], q[3], q[4], fxf, fyf, cxf, cyf, r.t2);
-    }
+    for (int k = tid; k < n; k += GEO_THREADS) flag[k] = pnp_inlier(hf, pnp_row(r, p, a, b, k), r);
   if (tid == 0) r.best[p] = s_best;
   const int sel = use_refit ? 1 : 0;
   const bool model = have && m > 0;                   // a best sample without an inlier is no model
-  if (tid < 9) r.R[9 * (size_t)p + tid] = model ? sR[sel][tid] : 0.0;
-  if (tid < 3) r.t[3 * (size_t)p + tid] = model ? st[sel][tid] : 0.0;
+  if (tid < 9) r.R[9 * (size_t)p + tid] = model ? sH[sel][tid] : 0.0;
+  if (tid < 3) r.t[3 * (size_t)p + tid] = model ? sH[sel][9 + tid] : 0.0;
   if (r.rms && tid < 2) {
-    const double c = tid == 0 || !use_refit ? cost0 : cost;
+    const double c = tid == 0 || !use_refit ? cost.x : cost.y;
     r.rms[2 * (size_t)p + tid] = model ? __dsqrt_rn(__ddiv_rn(c, (double)m)) : 0.0;
   }
-
-  // ---- order-preserving compaction of the kept rows (matcher list format)
-  __syncthreads();
-  const int total = compact_rows(flag, n, r.L, p, r.pairs, r.pair_scores, r.out_pairs, r.out_scores, scan, &s_total);
-  if (r.mask)
-    for (int k = tid; k < r.L; k += GEO_THREADS) r.mask[(size_t)p * r.L + k] = k < n ? flag[k] : 0;
-  if (tid == 0) r.out_counts[p] = total;
+  finish_lists(r, p, n, flag, scan, &s_total);
 }
 
 }  // namespace
@@ -607,8 +403,7 @@ __global__ void __launch_bounds__(GEO_THREADS, 1) pnp_refit_kernel(PnpParams r) 
 using namespace sslam;
 
 extern "C" size_t sslam_ransac_pnp_workspace_bytes(int P, int L, int iters) {
-  if (P <= 0 || L < 0 || iters <= 0) return 0;
-  return ws_layout(P, L, iters, 1, HF).total;
+  return ransac_workspace_bytes<PModel>(P, L, iters);
 }
 
 extern "C" int sslam_ransac_pnp(const float* points, int F1, const float* kpts2, int F2, const int32_t* pair_index,
@@ -616,42 +411,18 @@ extern "C" int sslam_ransac_pnp(const float* points, int F1, const float* kpts2,
                                 const int32_t* counts, int L, double fx, double fy, double cx, double cy, int iters,
                                 double threshold, uint64_t seed, int refine_iters, double* R, double* t,
                                 double* rms, int32_t* out_pairs, float* out_scores, int32_t* out_counts,
-                                uint8_t* inlier_mask, void* ws, size_t ws_bytes, void* stream_) {
+                                uint8_t* inlier_mask, void* ws, size_t ws_bytes, void* stream) {
   int rc = check_device();
   if (rc) return rc;
-  cudaStream_t stream = (cudaStream_t)stream_;
-  SSLAM_REQUIRE(P >= 0 && N >= 0 && M >= 0 && L >= 0, SSLAM_EINVAL, "ransac_pnp: bad size");
-  SSLAM_REQUIRE(L <= MAX_L, SSLAM_EINVAL, "ransac_pnp: list stride %d > %d", L, MAX_L);
-  SSLAM_REQUIRE(iters >= 1 && iters <= MAX_ITERS, SSLAM_EINVAL, "ransac_pnp: iters=%d (need 1..%d)", iters,
-                MAX_ITERS);
-  SSLAM_REQUIRE(refine_iters >= 0 && refine_iters <= MAX_REFINE, SSLAM_EINVAL,
-                "ransac_pnp: refine_iters=%d (need 0..%d)", refine_iters, MAX_REFINE);
-  SSLAM_REQUIRE(threshold > 0.0 && isfinite(threshold), SSLAM_EINVAL, "ransac_pnp: threshold must be finite and > 0");
-  SSLAM_REQUIRE(fx > 0.0 && fy > 0.0 && isfinite(fx) && isfinite(fy) && isfinite(cx) && isfinite(cy),
-                SSLAM_EINVAL, "ransac_pnp: need fx, fy > 0 and finite intrinsics");
-  if (P == 0) return SSLAM_OK;
-  SSLAM_REQUIRE(points && kpts2 && pairs && pair_scores && counts && R && t && out_pairs && out_scores &&
-                out_counts && ws, SSLAM_EINVAL, "ransac_pnp: null pointer");
-  SSLAM_REQUIRE(F1 > 0 && F2 > 0 && (pair_index || (F1 >= P && F2 >= P)), SSLAM_EINVAL,
-                "ransac_pnp: banks hold %d / %d sets but %d implicit lists were requested", F1, F2, P);
-  const WsLayout w = ws_layout(P, L, iters, 1, HF);
-  SSLAM_REQUIRE(ws_bytes >= w.total, SSLAM_EWORKSPACE, "ransac_pnp: workspace %zu < %zu", ws_bytes, w.total);
-  char* base = static_cast<char*>(ws);
-  PnpParams r{points, kpts2, F1, F2, pair_index, P, N, M, pairs, pair_scores, counts, L, iters, refine_iters,
-              fx, fy, cx, cy, (float)(threshold * threshold), (u64)seed, R, t, rms,
-              out_pairs, out_scores, out_counts, inlier_mask,
-              reinterpret_cast<int32_t*>(base + w.count), reinterpret_cast<int32_t*>(base + w.best),
-              reinterpret_cast<uint8_t*>(base + w.mask), reinterpret_cast<float*>(base + w.hyp)};
-  const int tile = L < 1 ? 1 : (L < SC_TILE ? L : SC_TILE);
-  const size_t smem = (size_t)tile * 5 * sizeof(float);
-  static DeviceOnce once;
-  if (once.first_use())
-    SSLAM_CHECK_CUDA(cudaFuncSetAttribute(pnp_score_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                          (int)(SC_TILE * 5 * sizeof(float))));
-  SSLAM_LAUNCH(KK_PNP_HYP, stream,
-               pnp_hyp_kernel<<<dim3(P, (iters + HYP_THREADS - 1) / HYP_THREADS), HYP_THREADS, 0, stream>>>(r));
-  SSLAM_LAUNCH(KK_PNP_SCORE, stream,
-               pnp_score_kernel<<<dim3(P, (iters + SC_HYPS - 1) / SC_HYPS), SC_THREADS, smem, stream>>>(r, tile));
-  SSLAM_LAUNCH(KK_PNP_REFIT, stream, pnp_refit_kernel<<<P, GEO_THREADS, 0, stream>>>(r));
-  return SSLAM_OK;
+  const double K[4] = {fx, fy, cx, cy};
+  rc = check_list_args("ransac_pnp", P, N, M, L, F1, F2, pair_index,
+                       points && kpts2 && pairs && pair_scores && counts && R && t && out_pairs && out_scores &&
+                           out_counts && ws,
+                       &iters, &refine_iters, "threshold", threshold, K);
+  if (rc || P == 0) return rc;
+  RansacParams r{points, kpts2, F1, F2, pair_index, P, N, M, pairs, pair_scores, counts, L, iters,
+                 (float)(threshold * threshold), (u64)seed, nullptr, out_pairs, out_scores, out_counts, inlier_mask,
+                 nullptr, nullptr, nullptr, nullptr, fx, fy, cx, cy, refine_iters, R, t, rms};
+  return ransac_launch<PModel>("ransac_pnp", r, ws, ws_bytes, pnp_refit_kernel,
+                               {KK_PNP_HYP, KK_PNP_SCORE, KK_PNP_REFIT}, (cudaStream_t)stream);
 }

@@ -21,11 +21,9 @@
 namespace sslam {
 namespace {
 
-constexpr int MAX_L = 16384;          // list stride limit (row flags live in shared memory)
-constexpr int MAX_REFINE = 100;
 constexpr int MIN_REFINE_ROWS = 5;    // rows the 5-DOF refinement needs
 constexpr int NP = 5;                 // refinement parameters: w (3), d (2)
-constexpr int NJ = NP * (NP + 1) / 2 + NP + 1;   // J^T J upper triangle, J^T r, r^T r
+constexpr int NJ = lm_nj(NP);
 
 struct PoseParams {
   const float* k1; const float* k2;          // [F1,N,2], [F2,M,2]
@@ -173,40 +171,12 @@ __device__ __noinline__ void linearise(const double* R, const double* t, double*
   }
 }
 
-// One LM trial (thread 0): solve (J^T J + lam diag(J^T J)) x = -J^T r by Cholesky, candidate
-// Rn = Exp(x_w) R, tn = normalise(t + x_d1 b1 + x_d2 b2), En = [tn]x Rn.  false: the system is not positive
-// definite or the step is not finite.
+// One LM trial (thread 0): the damped step x, candidate Rn = Exp(x_w) R, tn = normalise(t + x_d1 b1 + x_d2 b2),
+// En = [tn]x Rn.  false: no step, or tn is zero.
 __device__ __noinline__ bool lm_candidate(const double* J, double lam, const double* R, const double* t,
                                           const double* B, double* Rn, double* tn, double* En) {
-  double A[NP][NP], Lc[NP][NP], x[NP];
-  int q = 0;
-  for (int i = 0; i < NP; ++i)
-    for (int j = i; j < NP; ++j, ++q) A[i][j] = A[j][i] = J[q];
-  for (int i = 0; i < NP; ++i) A[i][i] = dadd(A[i][i], dmul(lam, A[i][i]));
-  for (int j = 0; j < NP; ++j) {
-    double d = A[j][j];
-    for (int k = 0; k < j; ++k) d = dsub(d, dmul(Lc[j][k], Lc[j][k]));
-    if (!(d > 0.0)) return false;
-    Lc[j][j] = __dsqrt_rn(d);
-    for (int i = j + 1; i < NP; ++i) {
-      double s = A[i][j];
-      for (int k = 0; k < j; ++k) s = dsub(s, dmul(Lc[i][k], Lc[j][k]));
-      Lc[i][j] = __ddiv_rn(s, Lc[j][j]);
-    }
-  }
-  for (int i = 0; i < NP; ++i) {                        // L y = -J^T r
-    double s = -J[NP * (NP + 1) / 2 + i];
-    for (int k = 0; k < i; ++k) s = dsub(s, dmul(Lc[i][k], x[k]));
-    x[i] = __ddiv_rn(s, Lc[i][i]);
-  }
-  for (int i = NP - 1; i >= 0; --i) {                   // L^T x = y
-    double s = x[i];
-    for (int k = i + 1; k < NP; ++k) s = dsub(s, dmul(Lc[k][i], x[k]));
-    x[i] = __ddiv_rn(s, Lc[i][i]);
-  }
-  bool ok = true;
-  for (int i = 0; i < NP; ++i) ok &= isfinite(x[i]);
-  if (!ok) return false;
+  double x[NP];
+  if (!lm_solve<NP>(J, lam, x)) return false;
   double X[9];
   rodrigues(x, X);
   mat3(X, R, Rn);
@@ -222,13 +192,11 @@ __global__ void __launch_bounds__(GEO_THREADS) pose_kernel(PoseParams r) {
   __shared__ uint8_t flag[MAX_L];
   __shared__ double red[(GEO_THREADS / 32) * NJ];
   __shared__ double sum[NJ];
-  __shared__ double Jsum[NJ];
   __shared__ double Rc[2][9], tc[3];                   // decomposition
   __shared__ double sR[9], st[3], sE[9], sdE[NP * 9], sB[6];   // current pose and its linearisation
   __shared__ double nR[9], nt[3], nE[9];               // LM candidate
-  __shared__ double s_cost, s_lam;
   __shared__ int scan[GEO_THREADS];
-  __shared__ int s_total, s_have, s_flag;
+  __shared__ int s_total, s_have;
   const int p = blockIdx.x, tid = threadIdx.x;
   int a, b;
   const int n = pair_rows(r, p, a, b);
@@ -268,81 +236,35 @@ __global__ void __launch_bounds__(GEO_THREADS) pose_kernel(PoseParams r) {
   const bool have = s_have;
 
   // ---- refinement
-  double cost0 = 0.0, cost = 0.0;
+  double2 cost = make_double2(0.0, 0.0);                // r^T r before / after
   if (have) {
     const bool refine = r.iters > 0 && usable >= MIN_REFINE_ROWS;
-    bool relin = true;
-    for (int it = -1; it < (refine ? r.iters : 0); ++it) {
-      if (relin) {                                      // J^T J, J^T r, r^T r at the current pose
-        double acc[NJ];
+    auto acc_row = [&](int k, double (&acc)[NJ]) {
+      double f1[3], f2[3], l[4], s;
+      if (!rays(r, p, a, b, k, f1, f2)) return;
+      const double res = sampson(sE, f1, f2, fx, fy, l, s);
+      double jr[NP];
 #pragma unroll
-        for (int i = 0; i < NJ; ++i) acc[i] = 0.0;
-        for (int k = tid; k < n; k += GEO_THREADS) {
-          double f1[3], f2[3], l[4], s;
-          if (!rays(r, p, a, b, k, f1, f2)) continue;
-          const double res = sampson(sE, f1, f2, fx, fy, l, s);
-          double jr[NP];
-#pragma unroll
-          for (int j = 0; j < NP; ++j) {
-            double dl[4];
-            const double dnum = epi_terms(sdE + 9 * j, f1, f2, fx, fy, dl);
-            jr[j] = s > 0.0 ? __ddiv_rn(dsub(dnum, __ddiv_rn(dmul(res, dot4(l, dl)), s)), s) : 0.0;
-          }
-          int q = 0;
-#pragma unroll
-          for (int i = 0; i < NP; ++i)
-#pragma unroll
-            for (int j = i; j < NP; ++j, ++q) acc[q] = dadd(acc[q], dmul(jr[i], jr[j]));
-#pragma unroll
-          for (int i = 0; i < NP; ++i) acc[q + i] = dadd(acc[q + i], dmul(jr[i], res));
-          acc[NJ - 1] = dadd(acc[NJ - 1], dmul(res, res));
-        }
-        block_sum<NJ>(acc, red, sum);
-        if (tid == 0) {
-          for (int i = 0; i < NJ; ++i) Jsum[i] = sum[i];
-          if (it < 0) {
-            s_cost = sum[NJ - 1];
-            double d = 0.0;
-            int q = 0;
-            for (int i = 0; i < NP; q += NP - i, ++i) d = dadd(d, sum[q]);
-            s_lam = dmul(1e-3, __ddiv_rn(d, (double)NP));
-          }
-        }
-        __syncthreads();
-        if (it < 0) cost0 = s_cost;
-        relin = false;
-        if (it < 0) continue;
+      for (int j = 0; j < NP; ++j) {
+        double dl[4];
+        const double dnum = epi_terms(sdE + 9 * j, f1, f2, fx, fy, dl);
+        jr[j] = s > 0.0 ? __ddiv_rn(dsub(dnum, __ddiv_rn(dmul(res, dot4(l, dl)), s)), s) : 0.0;
       }
-      if (tid == 0) s_flag = lm_candidate(Jsum, s_lam, sR, st, sB, nR, nt, nE);
-      __syncthreads();
-      bool accept = false;
-      if (s_flag) {
-        double c1[1] = {0.0};
-        for (int k = tid; k < n; k += GEO_THREADS) {
-          double f1[3], f2[3], l[4], s;
-          if (!rays(r, p, a, b, k, f1, f2)) continue;
-          const double res = sampson(nE, f1, f2, fx, fy, l, s);
-          c1[0] = dadd(c1[0], dmul(res, res));
-        }
-        block_sum<1>(c1, red, sum);
-        accept = sum[0] < s_cost;
-      }
-      __syncthreads();
-      if (tid == 0) {
-        if (accept) {
-          s_cost = sum[0];
-          s_lam = __ddiv_rn(s_lam, 10.0);
-          for (int i = 0; i < 9; ++i) sR[i] = nR[i];
-          for (int i = 0; i < 3; ++i) st[i] = nt[i];
-          linearise(sR, st, sE, sdE, sB);
-        } else {
-          s_lam = dmul(s_lam, 10.0);
-        }
-      }
-      __syncthreads();
-      relin = accept && it + 1 < r.iters;
-    }
-    cost = s_cost;
+      lm_add<NP>(acc, jr, res);
+    };
+    auto cost_row = [&](int k, double& c) {
+      double f1[3], f2[3], l[4], s;
+      if (!rays(r, p, a, b, k, f1, f2)) return;
+      const double res = sampson(nE, f1, f2, fx, fy, l, s);
+      c = dadd(c, dmul(res, res));
+    };
+    auto step = [&](const double* J, double lam) { return lm_candidate(J, lam, sR, st, sB, nR, nt, nE); };
+    auto commit = [&] {
+      for (int i = 0; i < 9; ++i) sR[i] = nR[i];
+      for (int i = 0; i < 3; ++i) st[i] = nt[i];
+      linearise(sR, st, sE, sdE, sB);
+    };
+    cost = lm_refine<NP>(n, refine, r.iters, red, sum, acc_row, cost_row, step, commit);
   }
 
   // ---- final pass: cheirality of the refined pose, mask, points, compaction
@@ -362,7 +284,7 @@ __global__ void __launch_bounds__(GEO_THREADS) pose_kernel(PoseParams r) {
   if (tid < 9) r.R[9 * (size_t)p + tid] = have ? sR[tid] : 0.0;
   if (tid < 3) r.t[3 * (size_t)p + tid] = have ? st[tid] : 0.0;
   if (r.rms && tid < 2) {
-    const double c = tid == 0 ? cost0 : cost;
+    const double c = tid == 0 ? cost.x : cost.y;
     r.rms[2 * (size_t)p + tid] = have && usable > 0 ? __dsqrt_rn(__ddiv_rn(c, (double)usable)) : 0.0;
   }
   __syncthreads();
@@ -383,20 +305,13 @@ extern "C" int sslam_recover_pose(const float* kpts1, int F1, const float* kpts2
                                   float* out_scores, int32_t* out_counts, uint8_t* pose_mask, void* stream_) {
   int rc = check_device();
   if (rc) return rc;
+  const double K[4] = {fx, fy, cx, cy};
+  rc = check_list_args("recover_pose", P, N, M, L, F1, F2, pair_index,
+                       kpts1 && kpts2 && E && pairs && pair_scores && counts && R && t && out_pairs && out_scores &&
+                           out_counts,
+                       nullptr, &refine_iters, "distance_thresh", distance_thresh, K);
+  if (rc || P == 0) return rc;
   cudaStream_t stream = (cudaStream_t)stream_;
-  SSLAM_REQUIRE(P >= 0 && N >= 0 && M >= 0 && L >= 0, SSLAM_EINVAL, "recover_pose: bad size");
-  SSLAM_REQUIRE(L <= MAX_L, SSLAM_EINVAL, "recover_pose: list stride %d > %d", L, MAX_L);
-  SSLAM_REQUIRE(refine_iters >= 0 && refine_iters <= MAX_REFINE, SSLAM_EINVAL,
-                "recover_pose: refine_iters=%d (need 0..%d)", refine_iters, MAX_REFINE);
-  SSLAM_REQUIRE(distance_thresh > 0.0 && isfinite(distance_thresh), SSLAM_EINVAL,
-                "recover_pose: distance_thresh must be finite and > 0");
-  SSLAM_REQUIRE(fx > 0.0 && fy > 0.0 && isfinite(fx) && isfinite(fy) && isfinite(cx) && isfinite(cy),
-                SSLAM_EINVAL, "recover_pose: need fx, fy > 0 and finite intrinsics");
-  if (P == 0) return SSLAM_OK;
-  SSLAM_REQUIRE(kpts1 && kpts2 && E && pairs && pair_scores && counts && R && t && out_pairs && out_scores &&
-                out_counts, SSLAM_EINVAL, "recover_pose: null pointer");
-  SSLAM_REQUIRE(F1 > 0 && F2 > 0 && (pair_index || (F1 >= P && F2 >= P)), SSLAM_EINVAL,
-                "recover_pose: banks hold %d / %d sets but %d implicit pairs were requested", F1, F2, P);
   PoseParams r{kpts1, kpts2, F1, F2, pair_index, P, N, M, E, pairs, pair_scores, counts, L,
                fx, fy, cx, cy, distance_thresh, refine_iters, R, t, cand_good, rms, points,
                out_pairs, out_scores, out_counts, pose_mask};

@@ -1,11 +1,10 @@
 // Geometric verification of padded match lists: batched RANSAC for P pairs at once, against a
-// homography (HModel) or a fundamental matrix (FModel).  The three kernels are templates over the model;
-// only the minimal solve, the inlier test and the refit's normal rows and post-processing differ.
+// homography (HModel) or a fundamental matrix (FModel).  The hypothesis and scoring kernels are
+// ransac.cuh's, with the correspondences (x1, y1, x2, y2) staged as float4; the refit is this file's:
 //
 //   ransac_hyp     one thread per (pair, sample): SAMPLE distinct rows drawn by a counter-based
 //                  splitmix64 sampler, minimal solve in double -> SLOTS fp32 hypotheses
-//   ransac_score   the hot loop (P x SLOTS*iters x n error evaluations): the pair's correspondences are
-//                  staged in shared memory tile by tile, warps take hypotheses, lanes stride the points
+//   ransac_score   the hot loop (P x SLOTS*iters x n error evaluations)
 //   ransac_refit   one CTA per pair: best hypothesis slot (most inliers, lowest slot on ties), least-squares
 //                  normalised fit over its inliers (fixed-order double reductions, Jacobi on one
 //                  thread), re-score, order-preserving compaction into the matcher's list format
@@ -22,40 +21,14 @@
 // scoring operation by operation: the hypothesis path uses only correctly rounded operations
 // (__dmul_rn / __dadd_rn / __ddiv_rn / __dsqrt_rn, __fmul_rn / __fadd_rn / __frcp_rn) in fixed orders with
 // fixed iteration counts, so CUDA and NumPy agree bit for bit.
-#include "geometry.cuh"
+#include "ransac.cuh"
 
 namespace sslam {
 namespace {
 
-constexpr int MAX_L = 16384;          // list stride limit (refit flags live in shared memory)
-constexpr int MAX_ITERS = 65536;
-constexpr int HYP_THREADS = 64;
-constexpr int SC_THREADS = 256;
-constexpr int SC_HYPS = 256;          // hypotheses per scoring CTA (32 per warp)
-constexpr int SC_TILE = 4096;         // correspondences staged per tile: 64 KB, three CTAs per SM
-constexpr int RF_THREADS = GEO_THREADS;
 constexpr double PIVOT_TOL = 1e-8;    // |pivot| of the normalised 8x8 / 7x9 solves, |h33| before scaling
 constexpr int BISECT = 64;            // bisection steps per sign-changing bracket of the 7-point cubic
 constexpr double SQRT2 = 1.4142135623730951;
-
-// ---------------------------------------------------------------------------- shared pieces
-struct RansacParams {
-  const float* k1; const float* k2;          // [F1,N,2], [F2,M,2]
-  int F1, F2;
-  const int32_t* pair_index;                 // [P,2] or null
-  int P, N, M;
-  const int32_t* pairs; const float* pair_scores; const int32_t* counts;   // [P,L,2], [P,L], [P]
-  int L, iters;
-  float t2;                                  // threshold^2 rounded to fp32
-  u64 seed;
-  double* H;                                 // [P,9] or null: the model (H or F)
-  int32_t* out_pairs; float* out_scores; int32_t* out_counts; uint8_t* mask;
-  // workspace
-  int32_t* hyp_count;                        // [P,SLOTS*iters]  inliers per hypothesis slot, -1 degenerate
-  int32_t* best;                             // [P]              best slot, -1 none
-  uint8_t* hyp_mask;                         // [P,L]            inliers of the best slot
-  float* hyp;                                // [P,SLOTS*iters,9]
-};
 
 // H = T2^-1 . Hn . T1 with T = [[s,0,-s*cx],[0,s,-s*cy],[0,0,1]], then scaled to h33 = 1.
 // false when |h33| < PIVOT_TOL or a coefficient is not finite.
@@ -169,13 +142,25 @@ __device__ __forceinline__ bool is_inlier(const float h[9], float4 q, float t2) 
 }
 
 // ---------------------------------------------------------------------------- homography model
+// The row access of both models: correspondences as float4, staged as float4 (a 64 KB tile, three
+// scoring CTAs per SM).
+struct CorrRows {
+  static constexpr int FLOATS = 9, TILE = 4096, ROW_FLOATS = 4;
+  using Row = float4;
+  __device__ static float4 row(const RansacParams& r, int p, int a, int b, int k) { return corr(r, p, a, b, k); }
+  __device__ static void stage(float* s, int, int k, float4 q) { reinterpret_cast<float4*>(s)[k] = q; }
+  __device__ static float4 staged(const float* s, int, int k) { return reinterpret_cast<const float4*>(s)[k]; }
+};
+
 // Slots of sample s: bit k of solve()'s result marks slot k valid.  accumulate() adds one inlier's
 // normal-matrix terms (upper triangle, 45 sums); finish() turns the smallest eigenvector of the normal
 // matrix into the model (thread 0; A, V: 81-double shared scratch).
-struct HModel {
+struct HModel : CorrRows {
   static constexpr int SAMPLE = 4, SLOTS = 1, MIN_FIT = 4;
-  __device__ static int solve(const float4 q[SAMPLE], double H[SLOTS][9]) { return dlt4(q, H[0]) ? 1 : 0; }
-  __device__ static bool inlier(const float h[9], float4 q, float t2) { return is_inlier(h, q, t2); }
+  __device__ static int solve(const float4 q[SAMPLE], const RansacParams&, double H[SLOTS][FLOATS]) {
+    return dlt4(q, H[0]) ? 1 : 0;
+  }
+  __device__ static bool inlier(const float h[9], float4 q, const RansacParams& r) { return is_inlier(h, q, r.t2); }
   __device__ static void accumulate(double x, double y, double u, double v, double (&nm)[45]) {
     const double r0[9] = {x, y, 1.0, 0.0, 0.0, 0.0, -u * x, -u * y, -u};
     const double r1[9] = {0.0, 0.0, 0.0, x, y, 1.0, -v * x, -v * y, -v};
@@ -420,10 +405,12 @@ __device__ __forceinline__ bool epi_inlier(const float f[9], float4 q, float t2)
   return e1 < t2 && e2 < t2;
 }
 
-struct FModel {
+struct FModel : CorrRows {
   static constexpr int SAMPLE = 7, SLOTS = 3, MIN_FIT = 8;
-  __device__ static int solve(const float4 q[SAMPLE], double F[SLOTS][9]) { return seven_point(q, F); }
-  __device__ static bool inlier(const float f[9], float4 q, float t2) { return epi_inlier(f, q, t2); }
+  __device__ static int solve(const float4 q[SAMPLE], const RansacParams&, double F[SLOTS][FLOATS]) {
+    return seven_point(q, F);
+  }
+  __device__ static bool inlier(const float f[9], float4 q, const RansacParams& r) { return epi_inlier(f, q, r.t2); }
   __device__ static void accumulate(double x, double y, double u, double v, double (&nm)[45]) {
     const double r0[9] = {u * x, u * y, u, v * x, v * y, v, x, y, 1.0};
     int t = 0;
@@ -447,21 +434,7 @@ struct FModel {
   }
 };
 
-// ---------------------------------------------------------------------------- shared by both models
-// Slots of sample s of pair p as doubles: bit k set when slot k holds a model.
-template <class M>
-__device__ __forceinline__ int sample_hyps(const RansacParams& r, int p, int a, int b, int n, int s,
-                                           double Hs[M::SLOTS][9]) {
-  int idx[M::SAMPLE];
-#pragma unroll
-  for (int k = 0; k < M::SAMPLE; ++k) idx[k] = -1;
-  if (n < M::SAMPLE || !sample_rows<M::SAMPLE>(r.seed, s, n, idx)) return 0;
-  float4 q[M::SAMPLE];
-#pragma unroll
-  for (int k = 0; k < M::SAMPLE; ++k) q[k] = corr(r, p, a, b, idx[k]);
-  return M::solve(q, Hs);
-}
-
+// ---------------------------------------------------------------------------- refit
 // Hypothesis slot h of pair p as doubles (false: degenerate).
 template <class M>
 __device__ bool slot_hypothesis(const RansacParams& r, int p, int a, int b, int n, int h, double H[9]) {
@@ -472,99 +445,25 @@ __device__ bool slot_hypothesis(const RansacParams& r, int p, int a, int b, int 
   return true;
 }
 
-// ---------------------------------------------------------------------------- kernels
 template <class M>
-__global__ void __launch_bounds__(HYP_THREADS) ransac_hyp_kernel(RansacParams r) {
-  const int p = blockIdx.x;
-  const int s = blockIdx.y * HYP_THREADS + threadIdx.x;
-  if (s >= r.iters) return;
-  int a, b;
-  const int n = pair_rows(r, p, a, b);
-  double H[M::SLOTS][9];
-  const int ok = sample_hyps<M>(r, p, a, b, n, s, H);
-#pragma unroll
-  for (int j = 0; j < M::SLOTS; ++j) {
-    const size_t h = ((size_t)p * r.iters + s) * M::SLOTS + j;
-    const bool v = (ok >> j) & 1;
-    float* o = r.hyp + h * 9;
-#pragma unroll
-    for (int k = 0; k < 9; ++k) o[k] = v ? __double2float_rn(H[j][k]) : 0.f;
-    r.hyp_count[h] = v ? 0 : -1;
-  }
-}
-
-template <class M>
-__global__ void __launch_bounds__(SC_THREADS) ransac_score_kernel(RansacParams r, int tile) {
-  extern __shared__ float4 pts[];
-  __shared__ float hs[SC_HYPS][9];
-  __shared__ int cnt[SC_HYPS];
-  const int p = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int slots = M::SLOTS * r.iters;
-  const int h0 = blockIdx.y * SC_HYPS;
-  const int nh = min(SC_HYPS, slots - h0);
-  int a, b;
-  const int n = pair_rows(r, p, a, b);
-  if (n < M::SAMPLE) return;                           // every hypothesis of the pair is degenerate
-  const size_t base = (size_t)p * slots + h0;
-  for (int t = tid; t < nh * 9; t += SC_THREADS) hs[t / 9][t % 9] = r.hyp[base * 9 + t];
-  for (int t = tid; t < nh; t += SC_THREADS) cnt[t] = r.hyp_count[base + t];
-  for (int k0 = 0; k0 < n; k0 += tile) {
-    const int nt = min(tile, n - k0);
-    __syncthreads();
-    for (int k = tid; k < nt; k += SC_THREADS) pts[k] = corr(r, p, a, b, k0 + k);
-    __syncthreads();
-    for (int hl = warp; hl < nh; hl += SC_THREADS / 32) {
-      if (cnt[hl] < 0) continue;
-      float h[9];
-#pragma unroll
-      for (int k = 0; k < 9; ++k) h[k] = hs[hl][k];
-      int c = 0;
-      for (int k0 = 0; k0 < nt; k0 += 32) {              // warp-uniform bound: every lane votes
-        const int k = k0 + lane;
-        c += __popc(__ballot_sync(0xffffffffu, k < nt && M::inlier(h, pts[k], r.t2)));
-      }
-      if (lane == 0) cnt[hl] += c;
-    }
-  }
-  __syncthreads();
-  for (int t = tid; t < nh; t += SC_THREADS) r.hyp_count[base + t] = cnt[t];
-}
-
-template <class M>
-__global__ void __launch_bounds__(RF_THREADS) ransac_refit_kernel(RansacParams r) {
+__global__ void __launch_bounds__(GEO_THREADS) ransac_refit_kernel(RansacParams r) {
   __shared__ uint8_t flag[MAX_L];
-  __shared__ double red[(RF_THREADS / 32) * 45];
+  __shared__ double red[(GEO_THREADS / 32) * 45];
   __shared__ double sum[45];
   __shared__ double Aj[81], Vj[81];
   __shared__ double Hs[2][9];                       // [0] best hypothesis, [1] refit
   __shared__ float hf[9];
-  __shared__ int scan[RF_THREADS];
-  __shared__ unsigned long long bkey[RF_THREADS / 32];
+  __shared__ int scan[GEO_THREADS];
+  __shared__ unsigned long long bkey[GEO_THREADS / 32];
   __shared__ int s_best, s_ok, s_total;
-  const int p = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int p = blockIdx.x, tid = threadIdx.x;
   int a, b;
   const int n = pair_rows(r, p, a, b);
-  const int slots = M::SLOTS * r.iters;
 
-  // ---- best hypothesis: most inliers, lowest slot on ties
-  unsigned long long key = 0;
-  if (n >= M::SAMPLE)
-    for (int h = tid; h < slots; h += RF_THREADS) {
-      const int c = r.hyp_count[(size_t)p * slots + h];
-      const unsigned long long k = ((unsigned long long)(unsigned)(c + 1) << 32) | (0xffffffffu - (unsigned)h);
-      key = k > key ? k : key;
-    }
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) {
-    const unsigned long long k = __shfl_xor_sync(0xffffffffu, key, o);
-    key = k > key ? k : key;
-  }
-  if (lane == 0) bkey[warp] = key;
-  __syncthreads();
+  // ---- best hypothesis
+  best_keys<M>(r, p, n, bkey);
   if (tid == 0) {
-    unsigned long long k = 0;
-    for (int w = 0; w < RF_THREADS / 32; ++w) k = bkey[w] > k ? bkey[w] : k;
-    const int best = (k >> 32) == 0 ? -1 : (int)(0xffffffffu - (unsigned)(k & 0xffffffffu));
+    const int best = best_slot(bkey);
     s_ok = best >= 0 && slot_hypothesis<M>(r, p, a, b, n, best, Hs[0]);
     s_best = s_ok ? best : -1;
     if (s_ok)
@@ -572,21 +471,13 @@ __global__ void __launch_bounds__(RF_THREADS) ransac_refit_kernel(RansacParams r
   }
   __syncthreads();
   const bool have = s_ok;
-  uint8_t* hm = r.hyp_mask + (size_t)p * r.L;
-  int m = 0;                                        // inliers of the best hypothesis (this thread's rows)
-  for (int k = tid; k < r.L; k += RF_THREADS) {
-    const bool in = have && k < n && M::inlier(hf, corr(r, p, a, b, k), r.t2);
-    flag[k] = in;
-    hm[k] = in;
-    m += in;
-  }
-  m = block_reduce_sum(m, scan);                    // scan[] doubles as the reduction scratch (>= 33)
+  const int m = mask_pass<M>(r, p, a, b, n, have, hf, flag, scan);
 
   // ---- refit over the best hypothesis's inliers (normalised least squares)
   bool use_refit = false;
   if (have && m >= M::MIN_FIT) {
     double c4[4] = {0.0, 0.0, 0.0, 0.0};
-    for (int k = tid; k < n; k += RF_THREADS)
+    for (int k = tid; k < n; k += GEO_THREADS)
       if (flag[k]) {
         const float4 q = corr(r, p, a, b, k);
         c4[0] = dadd(c4[0], q.x); c4[1] = dadd(c4[1], q.y); c4[2] = dadd(c4[2], q.z); c4[3] = dadd(c4[3], q.w);
@@ -594,7 +485,7 @@ __global__ void __launch_bounds__(RF_THREADS) ransac_refit_kernel(RansacParams r
     block_sum<4>(c4, red, sum);
     const double cx1 = sum[0] / m, cy1 = sum[1] / m, cx2 = sum[2] / m, cy2 = sum[3] / m;
     double d2[2] = {0.0, 0.0};
-    for (int k = tid; k < n; k += RF_THREADS)
+    for (int k = tid; k < n; k += GEO_THREADS)
       if (flag[k]) {
         const float4 q = corr(r, p, a, b, k);
         d2[0] = dadd(d2[0], sqrt((q.x - cx1) * (q.x - cx1) + (q.y - cy1) * (q.y - cy1)));
@@ -607,7 +498,7 @@ __global__ void __launch_bounds__(RF_THREADS) ransac_refit_kernel(RansacParams r
       double nm[45];
 #pragma unroll
       for (int i = 0; i < 45; ++i) nm[i] = 0.0;
-      for (int k = tid; k < n; k += RF_THREADS)
+      for (int k = tid; k < n; k += GEO_THREADS)
         if (flag[k]) {
           const float4 q = corr(r, p, a, b, k);
           const double x = (q.x - cx1) * s1, y = (q.y - cy1) * s1;
@@ -626,72 +517,32 @@ __global__ void __launch_bounds__(RF_THREADS) ransac_refit_kernel(RansacParams r
           for (int k2 = 0; k2 < 9; ++k2) hf[k2] = __double2float_rn(Hs[1][k2]);
       }
       __syncthreads();
-      if (s_ok) {
-        int c = 0;
-        for (int k = tid; k < n; k += RF_THREADS) c += M::inlier(hf, corr(r, p, a, b, k), r.t2);
-        c = block_reduce_sum(c, scan);
-        use_refit = c >= m;
-      }
+      if (s_ok) use_refit = keep_refit<M>(r, p, a, b, n, hf, m, scan);
     }
   }
   __syncthreads();
   if (use_refit)
-    for (int k = tid; k < n; k += RF_THREADS) flag[k] = M::inlier(hf, corr(r, p, a, b, k), r.t2);
+    for (int k = tid; k < n; k += GEO_THREADS) flag[k] = M::inlier(hf, M::row(r, p, a, b, k), r);
   if (tid == 0) r.best[p] = s_best;
   if (r.H && tid < 9) r.H[9 * (size_t)p + tid] = have ? Hs[use_refit ? 1 : 0][tid] : 0.0;
-
-  // ---- order-preserving compaction of the kept rows (matcher list format)
-  __syncthreads();
-  const int total = compact_rows(flag, n, r.L, p, r.pairs, r.pair_scores, r.out_pairs, r.out_scores, scan, &s_total);
-  if (r.mask)
-    for (int k = tid; k < r.L; k += RF_THREADS) r.mask[(size_t)p * r.L + k] = k < n ? flag[k] : 0;
-  if (tid == 0) r.out_counts[p] = total;
-}
-
-template <class M>
-size_t workspace_bytes(int P, int L, int iters) {
-  if (P <= 0 || L < 0 || iters <= 0) return 0;
-  return ws_layout(P, L, iters, M::SLOTS, 9).total;
+  finish_lists(r, p, n, flag, scan, &s_total);
 }
 
 template <class Model>
 int ransac(const float* kpts1, int F1, const float* kpts2, int F2, const int32_t* pair_index, int P, int N, int M,
            const int32_t* pairs, const float* pair_scores, const int32_t* counts, int L, int iters, double threshold,
            uint64_t seed, double* H, int32_t* out_pairs, float* out_scores, int32_t* out_counts,
-           uint8_t* inlier_mask, void* ws, size_t ws_bytes, void* stream_) {
+           uint8_t* inlier_mask, void* ws, size_t ws_bytes, void* stream) {
   int rc = check_device();
   if (rc) return rc;
-  cudaStream_t stream = (cudaStream_t)stream_;
-  SSLAM_REQUIRE(P >= 0 && N >= 0 && M >= 0 && L >= 0, SSLAM_EINVAL, "ransac: bad size");
-  SSLAM_REQUIRE(L <= MAX_L, SSLAM_EINVAL, "ransac: list stride %d > %d", L, MAX_L);
-  SSLAM_REQUIRE(iters >= 1 && iters <= MAX_ITERS, SSLAM_EINVAL, "ransac: iters=%d (need 1..%d)", iters, MAX_ITERS);
-  SSLAM_REQUIRE(threshold > 0.0 && isfinite(threshold), SSLAM_EINVAL, "ransac: threshold must be > 0");
-  if (P == 0) return SSLAM_OK;
-  SSLAM_REQUIRE(kpts1 && kpts2 && pairs && pair_scores && counts && out_pairs && out_scores && out_counts && ws,
-                SSLAM_EINVAL, "ransac: null pointer");
-  SSLAM_REQUIRE(F1 > 0 && F2 > 0 && (pair_index || (F1 >= P && F2 >= P)), SSLAM_EINVAL,
-                "ransac: banks hold %d / %d sets but %d implicit pairs were requested", F1, F2, P);
-  const WsLayout w = ws_layout(P, L, iters, Model::SLOTS, 9);
-  SSLAM_REQUIRE(ws_bytes >= w.total, SSLAM_EWORKSPACE, "ransac: workspace %zu < %zu", ws_bytes, w.total);
-  char* base = static_cast<char*>(ws);
+  rc = check_list_args("ransac", P, N, M, L, F1, F2, pair_index,
+                       kpts1 && kpts2 && pairs && pair_scores && counts && out_pairs && out_scores && out_counts && ws,
+                       &iters, nullptr, "threshold", threshold, nullptr);
+  if (rc || P == 0) return rc;
   RansacParams r{kpts1, kpts2, F1, F2, pair_index, P, N, M, pairs, pair_scores, counts, L, iters,
-                 (float)(threshold * threshold), (u64)seed, H, out_pairs, out_scores, out_counts, inlier_mask,
-                 reinterpret_cast<int32_t*>(base + w.count), reinterpret_cast<int32_t*>(base + w.best),
-                 reinterpret_cast<uint8_t*>(base + w.mask), reinterpret_cast<float*>(base + w.hyp)};
-  const int tile = L < 1 ? 1 : (L < SC_TILE ? L : SC_TILE);
-  const size_t smem = (size_t)tile * sizeof(float4);
-  const int score_ctas = (Model::SLOTS * iters + SC_HYPS - 1) / SC_HYPS;
-  static DeviceOnce once;
-  if (once.first_use())
-    SSLAM_CHECK_CUDA(cudaFuncSetAttribute(ransac_score_kernel<Model>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                          (int)(SC_TILE * sizeof(float4))));
-  SSLAM_LAUNCH(KK_RANSAC_HYP, stream,
-               ransac_hyp_kernel<Model><<<dim3(P, (iters + HYP_THREADS - 1) / HYP_THREADS), HYP_THREADS, 0,
-                                          stream>>>(r));
-  SSLAM_LAUNCH(KK_RANSAC_SCORE, stream,
-               ransac_score_kernel<Model><<<dim3(P, score_ctas), SC_THREADS, smem, stream>>>(r, tile));
-  SSLAM_LAUNCH(KK_RANSAC_REFIT, stream, ransac_refit_kernel<Model><<<P, RF_THREADS, 0, stream>>>(r));
-  return SSLAM_OK;
+                 (float)(threshold * threshold), (u64)seed, H, out_pairs, out_scores, out_counts, inlier_mask};
+  return ransac_launch<Model>("ransac", r, ws, ws_bytes, ransac_refit_kernel<Model>,
+                              {KK_RANSAC_HYP, KK_RANSAC_SCORE, KK_RANSAC_REFIT}, (cudaStream_t)stream);
 }
 
 }  // namespace
@@ -700,11 +551,11 @@ int ransac(const float* kpts1, int F1, const float* kpts2, int F2, const int32_t
 using namespace sslam;
 
 extern "C" size_t sslam_ransac_workspace_bytes(int P, int L, int iters) {
-  return workspace_bytes<HModel>(P, L, iters);
+  return ransac_workspace_bytes<HModel>(P, L, iters);
 }
 
 extern "C" size_t sslam_ransac_fundamental_workspace_bytes(int P, int L, int iters) {
-  return workspace_bytes<FModel>(P, L, iters);
+  return ransac_workspace_bytes<FModel>(P, L, iters);
 }
 
 extern "C" int sslam_ransac_homography(const float* kpts1, int F1, const float* kpts2, int F2,

@@ -398,19 +398,16 @@ def ransac_workspace_bytes(P, L, iters, model="homography"):
     return getattr(_lib.load(), _RANSAC_SYMBOLS[model][1])(int(P), int(L), int(iters))
 
 
-def _ransac(model, kpts1, kpts2, pairs, pair_scores, counts, pair_index, num_pairs, threshold, iters, seed,
-            want_mask, workspace):
-    name = "ransac_" + model
-    lib = _lib.load()
-    _need_cuda(kpts1, kpts2, pairs, pair_scores, counts, pair_index)
-    k1, k2 = kpts1.contiguous(), kpts2.contiguous()
+def _match_lists(name, k1, k2, pairs, pair_scores, counts, pair_index, num_pairs):
+    """Checks and casts the padded match-list arguments of the geometry entries: returns k1, k2 (fp32,
+    contiguous), pairs, pair_scores, counts, pair_index as the C ABI takes them, and F1, N, F2, M, P, L."""
+    _need_cuda(k1, k2, pairs, pair_scores, counts, pair_index)
+    k1, k2 = k1.contiguous(), k2.contiguous()
     if k1.dtype != torch.float32 or k2.dtype != torch.float32:
         raise RuntimeError(f"{name} expects fp32 keypoints")
     pr = pairs.to(torch.int32).contiguous()
     ps = pair_scores.to(torch.float32).contiguous()
     cn = counts.to(torch.int32).contiguous()
-    F1, N = k1.shape[0], k1.shape[1]
-    F2, M = k2.shape[0], k2.shape[1]
     P, L = pr.shape[0], pr.shape[1]
     if pair_index is not None:
         pair_index = pair_index.to(torch.int32).contiguous()
@@ -418,20 +415,27 @@ def _ransac(model, kpts1, kpts2, pairs, pair_scores, counts, pair_index, num_pai
             raise RuntimeError(f"{name}: pair_index must hold one (a, b) row per match list")
     elif num_pairs is not None and int(num_pairs) != P:
         raise RuntimeError(f"{name}: num_pairs differs from the number of match lists")
+    return k1, k2, pr, ps, cn, pair_index, k1.shape[0], k1.shape[1], k2.shape[0], k2.shape[1], P, L
+
+
+def _ransac(model, kpts1, kpts2, pairs, pair_scores, counts, pair_index, num_pairs, threshold, iters, seed,
+            want_mask, workspace):
+    name = "ransac_" + model
+    lib = _lib.load()
+    k1, k2, pr, ps, cn, pair_index, F1, N, F2, M, P, L = _match_lists(name, kpts1, kpts2, pairs, pair_scores,
+                                                                      counts, pair_index, num_pairs)
     dev = pr.device
     G = torch.empty(P, 3, 3, dtype=torch.float64, device=dev)
     out_pairs = torch.empty(P, L, 2, dtype=torch.int32, device=dev)
     out_scores = torch.empty(P, L, dtype=torch.float32, device=dev)
     out_counts = torch.empty(P, dtype=torch.int32, device=dev)
     mask = torch.empty(P, L, dtype=torch.uint8, device=dev) if want_mask else None
-    fn, ws_fn, _ = _RANSAC_SYMBOLS[model]
-    need = getattr(lib, ws_fn)(P, L, int(iters))
+    need = ransac_workspace_bytes(P, L, iters, model)
     ws = workspace if workspace is not None else _ws("ransac", need, dev)
-    _lib.check(getattr(lib, fn)(_ptr(k1), F1, _ptr(k2), F2, _ptr(pair_index), P, N, M, _ptr(pr),
-                                _ptr(ps), _ptr(cn), L, int(iters), float(threshold),
-                                int(seed) & 0xFFFFFFFFFFFFFFFF, _ptr(G), _ptr(out_pairs),
-                                _ptr(out_scores), _ptr(out_counts), _ptr(mask), _ptr(ws), ws.numel(),
-                                _stream()))
+    fn = getattr(lib, _RANSAC_SYMBOLS[model][0])
+    _lib.check(fn(_ptr(k1), F1, _ptr(k2), F2, _ptr(pair_index), P, N, M, _ptr(pr), _ptr(ps), _ptr(cn), L,
+                  int(iters), float(threshold), int(seed) & 0xFFFFFFFFFFFFFFFF, _ptr(G), _ptr(out_pairs),
+                  _ptr(out_scores), _ptr(out_counts), _ptr(mask), _ptr(ws), ws.numel(), _stream()))
     return (G, out_pairs, out_scores, out_counts) + ((mask,) if want_mask else ())
 
 
@@ -465,25 +469,12 @@ def recover_pose(kpts1, kpts2, E, pairs, pair_scores, counts, fx, fy, cx, cy, pa
     mask (P,L) uint8][, points (P,L,3) fp32 in the camera-1 frame, |t| = 1, zero where a row is not
     good]).  A pair without a pose has R, t, rms all zeros and an empty list."""
     lib = _lib.load()
-    _need_cuda(kpts1, kpts2, E, pairs, pair_scores, counts, pair_index)
-    k1, k2 = kpts1.contiguous(), kpts2.contiguous()
-    if k1.dtype != torch.float32 or k2.dtype != torch.float32:
-        raise RuntimeError("recover_pose expects fp32 keypoints")
-    pr = pairs.to(torch.int32).contiguous()
-    ps = pair_scores.to(torch.float32).contiguous()
-    cn = counts.to(torch.int32).contiguous()
-    F1, N = k1.shape[0], k1.shape[1]
-    F2, M = k2.shape[0], k2.shape[1]
-    P, L = pr.shape[0], pr.shape[1]
+    _need_cuda(E)
+    k1, k2, pr, ps, cn, pair_index, F1, N, F2, M, P, L = _match_lists("recover_pose", kpts1, kpts2, pairs,
+                                                                      pair_scores, counts, pair_index, num_pairs)
     Ed = E.to(torch.float64).reshape(-1, 9).contiguous()
     if Ed.shape[0] != P:
         raise RuntimeError("recover_pose: E must hold one matrix per match list")
-    if pair_index is not None:
-        pair_index = pair_index.to(torch.int32).contiguous()
-        if pair_index.shape[0] != P:
-            raise RuntimeError("recover_pose: pair_index must hold one (a, b) row per match list")
-    elif num_pairs is not None and int(num_pairs) != P:
-        raise RuntimeError("recover_pose: num_pairs differs from the number of match lists")
     dev = pr.device
     R = torch.empty(P, 3, 3, dtype=torch.float64, device=dev)
     t = torch.empty(P, 3, dtype=torch.float64, device=dev)
@@ -517,22 +508,11 @@ def ransac_pnp(points, kpts2, pairs, pair_scores, counts, fx, fy, cx, cy, pair_i
     reprojection error in px over the best sample's inliers before / after the refinement —[, inlier mask
     (P,L) uint8]).  A list without a model has R, t, rms all zeros and an empty list."""
     lib = _lib.load()
-    _need_cuda(points, kpts2, pairs, pair_scores, counts, pair_index)
-    X, k2 = points.contiguous(), kpts2.contiguous()
-    if X.dtype != torch.float32 or k2.dtype != torch.float32 or X.dim() != 3 or X.shape[-1] != 3:
+    _need_cuda(points, kpts2)
+    if points.dtype != torch.float32 or kpts2.dtype != torch.float32 or points.dim() != 3 or points.shape[-1] != 3:
         raise RuntimeError("ransac_pnp expects fp32 points (F1,N,3) and fp32 keypoints (F2,M,2)")
-    pr = pairs.to(torch.int32).contiguous()
-    ps = pair_scores.to(torch.float32).contiguous()
-    cn = counts.to(torch.int32).contiguous()
-    F1, N = X.shape[0], X.shape[1]
-    F2, M = k2.shape[0], k2.shape[1]
-    P, L = pr.shape[0], pr.shape[1]
-    if pair_index is not None:
-        pair_index = pair_index.to(torch.int32).contiguous()
-        if pair_index.shape[0] != P:
-            raise RuntimeError("ransac_pnp: pair_index must hold one (a, b) row per match list")
-    elif num_pairs is not None and int(num_pairs) != P:
-        raise RuntimeError("ransac_pnp: num_pairs differs from the number of match lists")
+    X, k2, pr, ps, cn, pair_index, F1, N, F2, M, P, L = _match_lists("ransac_pnp", points, kpts2, pairs,
+                                                                     pair_scores, counts, pair_index, num_pairs)
     dev = pr.device
     R = torch.empty(P, 3, 3, dtype=torch.float64, device=dev)
     t = torch.empty(P, 3, dtype=torch.float64, device=dev)
@@ -541,7 +521,7 @@ def ransac_pnp(points, kpts2, pairs, pair_scores, counts, fx, fy, cx, cy, pair_i
     out_scores = torch.empty(P, L, dtype=torch.float32, device=dev)
     out_counts = torch.empty(P, dtype=torch.int32, device=dev)
     mask = torch.empty(P, L, dtype=torch.uint8, device=dev) if want_mask else None
-    need = lib.sslam_ransac_pnp_workspace_bytes(P, L, int(iters))
+    need = ransac_workspace_bytes(P, L, iters, "pnp")
     ws = workspace if workspace is not None else _ws("ransac", need, dev)
     _lib.check(lib.sslam_ransac_pnp(_ptr(X), F1, _ptr(k2), F2, _ptr(pair_index), P, N, M, _ptr(pr), _ptr(ps),
                                     _ptr(cn), L, float(fx), float(fy), float(cx), float(cy), int(iters),
