@@ -417,6 +417,39 @@ int sslam_ransac_pnp(const float* points, int F1, const float* kpts2, int F2, co
                      int32_t* out_counts, uint8_t* inlier_mask, void* ws, size_t ws_bytes, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
+ * Triangulation of match lists under a known relative pose (map growth): the 3-D point of every row of P
+ * lists, x_b ~ R x_a + t, in the units of t.  One launch (one CTA per list), no workspace, no atomics, no
+ * host synchronisation (capturable in a CUDA graph); a list's result does not depend on its position in
+ * the batch.  The banks, pair_index and the padded lists are those of sslam_recover_pose; rows k <
+ * min(counts[p], L) are used, and a row whose keypoint indices are out of range or whose coordinates are
+ * not finite is never kept.  R [P,9] double row-major and t [P,3] double are each list's relative pose
+ * (typically sslam_ransac_pnp's); a list whose R or t has a non-finite entry, or whose R is all zero (the
+ * "no model" of every geometry entry), keeps no row.  One pinhole camera K = [[fx,0,cx],[0,fy,cy],[0,0,1]]
+ * for both images.  Per row, on one thread, in double with correctly rounded operations only:
+ *   Midpoint: the rays and midpoint of sslam_recover_pose's cheirality (f1 = K^-1 x1, f2 = K^-1 x2,
+ *   X = z1 f1), which also gives the "rays not parallel" test den > 1e-12 a c.
+ *   Refinement (refine_iters Levenberg-Marquardt trials on X, 0 keeps the midpoint): the residual is the
+ *   4-vector of pixel errors pi(X) - x1, pi(R X + t) - x2 with an analytic Jacobian; lambda starts at 1e-3
+ *   times the mean of diag(J^T J); each trial solves (J^T J + lambda diag(J^T J)) x = -J^T r by Cholesky,
+ *   and the candidate X + x is accepted iff its depth is > 0 in both cameras and the cost strictly
+ *   decreases (lambda /= 10, relinearise), otherwise lambda *= 10.
+ *   Gates on the final X: the row is kept iff the rays are not parallel, 0 < z_a < distance_thresh and
+ *   0 < z_b < distance_thresh, the parallax cosine X.(X - C_b) / (|X| |X - C_b|) with C_b = -R^T t is
+ *   <= max_parallax_cos, and the squared reprojection error is < threshold^2 in both views.
+ *   Outputs: points [P,L,3] fp32 X in the camera-a frame, 0 where a row is not kept (may be NULL); mask
+ *   [P,L] uint8 (may be NULL); the kept rows in input order as out_pairs [P,L,2] (-1 padded), out_scores
+ *   [P,L] (0 padded), out_counts [P] -- the matcher's list format.
+ * Limits: L <= 16384, 0 <= refine_iters <= 100, threshold > 0 and finite, 0 <= max_parallax_cos <= 1,
+ * distance_thresh > 0, fx, fy > 0 and finite, cx, cy finite.
+ */
+int sslam_triangulate(const float* kpts1, int F1, const float* kpts2, int F2, const int32_t* pair_index,
+                      int P, int N, int M, const int32_t* pairs, const float* pair_scores,
+                      const int32_t* counts, int L, const double* R, const double* t, double fx, double fy,
+                      double cx, double cy, double threshold, double max_parallax_cos,
+                      double distance_thresh, int refine_iters, float* points, int32_t* out_pairs,
+                      float* out_scores, int32_t* out_counts, uint8_t* mask, void* stream);
+
+/* ---------------------------------------------------------------------------------------------
  * Optional cell-softmax front stage of the decode (north_star "softmax/depth-to-space ... border
  * mask"; OFF by default — the reference code has no such mode, keypoint_selector.py:61-62 is a
  * sigmoid; the vocabulary is papers/pdfs/SuperPoint_DeTone.md:49-58):

@@ -1,8 +1,8 @@
-// Helpers shared by the per-pair geometry kernels (ransac.cu, pose.cu, pnp.cu): the argument checks of
-// the list entries, the padded match-list accessors, the splitmix64 row sampler, correctly rounded double
-// arithmetic, 3x3 helpers and Rodrigues, the fixed-order block reductions, cyclic Jacobi, the
-// Levenberg-Marquardt loop, the order-preserving compaction into the matcher's list format and the RANSAC
-// workspace layout.
+// Helpers shared by the per-pair geometry kernels (ransac.cu, pose.cu, pnp.cu, triangulate.cu): the
+// argument checks of the list entries, the padded match-list accessors, the splitmix64 row sampler,
+// correctly rounded double arithmetic, 3x3 helpers and Rodrigues, calibrated rays and midpoint
+// triangulation, the fixed-order block reductions, cyclic Jacobi, the Levenberg-Marquardt loop, the
+// order-preserving compaction into the matcher's list format and the RANSAC workspace layout.
 #pragma once
 
 #include "common.cuh"
@@ -15,6 +15,10 @@ constexpr int MAX_L = 16384;          // list stride limit (row flags live in sh
 constexpr int MAX_ITERS = 65536;      // RANSAC samples per list
 constexpr int MAX_REFINE = 100;       // Levenberg-Marquardt trials
 constexpr int MAX_DRAWS = 32;         // sampler draws per sample (redraws included)
+// Levenberg-Marquardt damping schedule: lambda starts at LM_LAMBDA0 times the mean of diag(J^T J); an
+// accepted trial divides it by LM_LAMBDA_STEP, a rejected one multiplies it by LM_LAMBDA_STEP.
+constexpr double LM_LAMBDA0 = 1e-3;
+constexpr double LM_LAMBDA_STEP = 10.0;
 
 // Checks shared by the match-list entries; SSLAM_OK or the code to return, the message prefixed by fn.
 // iters, refine_iters and the intrinsics K = {fx, fy, cx, cy} are checked where the entry takes them (not
@@ -131,6 +135,39 @@ __device__ __forceinline__ void rodrigues(const double* w, double* X) {
   }
 }
 
+// Normalised rays (K^-1 x) of row k; false when the row is not usable (a keypoint index out of range, or
+// a coordinate that is not finite).  Pm: the list fields of pair_rows / corr and fx, fy, cx, cy.
+template <class Pm>
+__device__ __forceinline__ bool rays(const Pm& r, int p, int a, int b, int k, double f1[3], double f2[3]) {
+  const float4 q = corr(r, p, a, b, k);
+  if (!(isfinite(q.x) && isfinite(q.y) && isfinite(q.z) && isfinite(q.w))) return false;
+  f1[0] = __ddiv_rn(dsub(q.x, r.cx), r.fx); f1[1] = __ddiv_rn(dsub(q.y, r.cy), r.fy); f1[2] = 1.0;
+  f2[0] = __ddiv_rn(dsub(q.z, r.cx), r.fx); f2[1] = __ddiv_rn(dsub(q.w, r.cy), r.fy); f2[2] = 1.0;
+  return true;
+}
+
+// Midpoint of the rays f1, f2 under (R, t), x2 ~ R x1 + t: the depths z1, z2 minimising |z1 u + t - z2 f2|
+// with u = R f1, X = z1 f1 (camera-1 frame).  Returns whether the rays are not parallel, den > 1e-12 a c.
+__device__ __forceinline__ bool midpoint(const double* R, const double* t, const double f1[3], const double f2[3],
+                                         double X[3]) {
+  const double u[3] = {dot3(R, f1), dot3(R + 3, f1), dot3(R + 6, f1)};
+  const double a = dot3(u, u), b = dot3(u, f2), c = dot3(f2, f2), d = dot3(u, t), e = dot3(f2, t);
+  const double den = dsub(dmul(a, c), dmul(b, b));
+  const double z1 = __ddiv_rn(dsub(dmul(b, e), dmul(c, d)), den);
+  X[0] = dmul(z1, f1[0]); X[1] = dmul(z1, f1[1]); X[2] = z1;
+  return den > dmul(dmul(1e-12, a), c);
+}
+
+// Triangulation of one row under (R, t) with cv2.recoverPose's cheirality: good iff the rays are not
+// parallel, 0 < z1 < dist and 0 < (R X + t)_z < dist.
+__device__ __forceinline__ bool triangulate(const double* R, const double* t, const double f1[3],
+                                            const double f2[3], double dist, double X[3]) {
+  const bool apart = midpoint(R, t, f1, f2, X);
+  const double z1 = X[2];
+  const double z2 = dadd(dot3(R + 6, X), t[2]);
+  return apart && z1 > 0.0 && z1 < dist && z2 > 0.0 && z2 < dist;
+}
+
 // Fixed-order block sum of R doubles per thread over GEO_THREADS threads: warp butterflies, then warps
 // in order.
 template <int R>
@@ -156,6 +193,15 @@ __device__ __forceinline__ void block_sum(double (&v)[R], double* red /* [GEO_TH
 // ---------------------------------------------------------------------------- Levenberg-Marquardt
 // Accumulators of an NP-parameter refinement: J^T J upper triangle, J^T r, r^T r.
 constexpr int lm_nj(int np) { return np * (np + 1) / 2 + np + 1; }
+
+// The starting damping of the accumulators Js: LM_LAMBDA0 times the mean of diag(J^T J).
+template <int NP>
+__device__ __forceinline__ double lm_lambda0(const double* Js) {
+  double d = 0.0;
+  int q = 0;
+  for (int i = 0; i < NP; q += NP - i, ++i) d = dadd(d, Js[q]);
+  return dmul(LM_LAMBDA0, __ddiv_rn(d, (double)NP));
+}
 
 // Adds one residual r with Jacobian row j to the accumulators.
 template <int NP>
@@ -206,12 +252,12 @@ __device__ __forceinline__ bool lm_solve(const double* Js, double lam, double x[
 }
 
 // Levenberg-Marquardt over the rows k < n, every thread of the block (GEO_THREADS) calls it.  Linearise
-// (acc_row(k, acc) adds row k's terms with lm_add, or skips the row), lam = 1e-3 mean diag(J^T J); then,
-// when `refine`, `iters` trials: step(Jsum, lam) forms the candidate on thread 0 (false: no step),
-// cost_row(k, c) adds row k's squared residual under it, a strictly lower cost is accepted (commit() on
-// thread 0, lam / 10, relinearise before the next trial), anything else sets lam * 10.  All sums are
-// fixed-order block sums (red, sum: block_sum scratch of lm_nj(NP) doubles per warp and in all).  Returns
-// (cost0, cost): r^T r at the start and at the end.
+// (acc_row(k, acc) adds row k's terms with lm_add, or skips the row), lam = lm_lambda0; then, when
+// `refine`, `iters` trials: step(Jsum, lam) forms the candidate on thread 0 (false: no step), cost_row(k, c)
+// adds row k's squared residual under it, a strictly lower cost is accepted (commit() on thread 0,
+// lam / LM_LAMBDA_STEP, relinearise before the next trial), anything else sets lam * LM_LAMBDA_STEP.  All
+// sums are fixed-order block sums (red, sum: block_sum scratch of lm_nj(NP) doubles per warp and in all).
+// Returns (cost0, cost): r^T r at the start and at the end.
 template <int NP, class AccRow, class CostRow, class Step, class Commit>
 __device__ __forceinline__ double2 lm_refine(int n, bool refine, int iters, double* red, double* sum,
                                              AccRow acc_row, CostRow cost_row, Step step, Commit commit) {
@@ -232,10 +278,7 @@ __device__ __forceinline__ double2 lm_refine(int n, bool refine, int iters, doub
         for (int i = 0; i < NJ; ++i) Jsum[i] = sum[i];
         if (it < 0) {
           s_cost = sum[NJ - 1];
-          double d = 0.0;
-          int q = 0;
-          for (int i = 0; i < NP; q += NP - i, ++i) d = dadd(d, sum[q]);
-          s_lam = dmul(1e-3, __ddiv_rn(d, (double)NP));
+          s_lam = lm_lambda0<NP>(sum);
         }
       }
       __syncthreads();
@@ -256,10 +299,10 @@ __device__ __forceinline__ double2 lm_refine(int n, bool refine, int iters, doub
     if (tid == 0) {
       if (accept) {
         s_cost = sum[0];
-        s_lam = __ddiv_rn(s_lam, 10.0);
+        s_lam = __ddiv_rn(s_lam, LM_LAMBDA_STEP);
         commit();
       } else {
-        s_lam = dmul(s_lam, 10.0);
+        s_lam = dmul(s_lam, LM_LAMBDA_STEP);
       }
     }
     __syncthreads();

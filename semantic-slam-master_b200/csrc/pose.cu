@@ -42,30 +42,6 @@ struct PoseParams {
   int32_t* out_pairs; float* out_scores; int32_t* out_counts; uint8_t* mask;
 };
 
-// Normalised rays (K^-1 x) of row k; false when the row is not usable (a keypoint index out of range, or
-// a coordinate that is not finite).
-__device__ __forceinline__ bool rays(const PoseParams& r, int p, int a, int b, int k, double f1[3], double f2[3]) {
-  const float4 q = corr(r, p, a, b, k);
-  if (!(isfinite(q.x) && isfinite(q.y) && isfinite(q.z) && isfinite(q.w))) return false;
-  f1[0] = __ddiv_rn(dsub(q.x, r.cx), r.fx); f1[1] = __ddiv_rn(dsub(q.y, r.cy), r.fy); f1[2] = 1.0;
-  f2[0] = __ddiv_rn(dsub(q.z, r.cx), r.fx); f2[1] = __ddiv_rn(dsub(q.w, r.cy), r.fy); f2[2] = 1.0;
-  return true;
-}
-
-// Triangulation of one row under (R, t), x2 ~ R x1 + t: the depths z1, z2 minimising |z1 u + t - z2 f2|
-// with u = R f1, X = z1 f1 (camera-1 frame).  Good iff den > 1e-12 a c, 0 < z1 < dist and
-// 0 < (R X + t)_z < dist.
-__device__ __forceinline__ bool triangulate(const double* R, const double* t, const double f1[3],
-                                            const double f2[3], double dist, double X[3]) {
-  const double u[3] = {dot3(R, f1), dot3(R + 3, f1), dot3(R + 6, f1)};
-  const double a = dot3(u, u), b = dot3(u, f2), c = dot3(f2, f2), d = dot3(u, t), e = dot3(f2, t);
-  const double den = dsub(dmul(a, c), dmul(b, b));
-  const double z1 = __ddiv_rn(dsub(dmul(b, e), dmul(c, d)), den);
-  X[0] = dmul(z1, f1[0]); X[1] = dmul(z1, f1[1]); X[2] = z1;
-  const double z2 = dadd(dot3(R + 6, X), t[2]);
-  return den > dmul(dmul(1e-12, a), c) && z1 > 0.0 && z1 < dist && z2 > 0.0 && z2 < dist;
-}
-
 // f2^T E f1, and the first two entries of F x1 = K^-T E f1 and F^T x2 = K^-T E^T f2 (pixel units).
 __device__ __forceinline__ double epi_terms(const double* E, const double f1[3], const double f2[3], double fx,
                                             double fy, double l[4]) {

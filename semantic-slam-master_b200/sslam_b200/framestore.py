@@ -16,6 +16,10 @@ slots through ``pair_index`` (slot ids), so nothing leaves the device until the 
                         camera, from the resident keypoints.
 ``track_poses``         the pose of each list's second frame against 3-D points attached to its first
                         frame's keypoints (geometry.point_map), by RANSAC P3P on the resident keypoints.
+``triangulate_pairs``   the 3-D points of the rows of lists under known relative poses, on the resident
+                        keypoints.
+``track_and_map``       one step of sequence tracking with map growth: track_poses, then the points carried
+                        onto each list's second frame and new points triangulated for its other keypoints.
 ``TrackingCounters``    the counters of track_frame_sequence (:166-199) accumulated on the device.
 """
 
@@ -174,6 +178,37 @@ class FrameStore:
                                         pair_index=idx, threshold=threshold, iters=iters, seed=seed,
                                         refine_iters=refine_iters)
         return out[:5]
+
+
+    def _pixel_keypoints(self):
+        kp = self.bank["keypoints"]
+        return kp * self.fe.patch + self.fe.patch / 2 if self.fe.grid != "pixel" else kp
+
+    @torch.no_grad()
+    def triangulate_pairs(self, frame_pairs, pairs, scores, counts, R, t, camera, threshold=3.0, min_parallax_deg=1.0,
+                          distance_thresh=50.0, refine_iters=10, want_mask=False):
+        """The 3-D points of the rows of the lists match_pairs / match_spacings returned for ``frame_pairs``
+        (a, b), under the relative pose (R, t) of each pair (x_b ~ R x_a + t), on the resident keypoints:
+        geometry.triangulate_device's (points (P,L,3) in frame a's camera frame, kept pairs, scores,
+        counts[, mask])."""
+        kp = self._pixel_keypoints()
+        return geometry.triangulate_device(kp, kp, pairs, scores, counts, R, t, camera,
+                                           pair_index=self.pair_index(frame_pairs), threshold=threshold,
+                                           min_parallax_deg=min_parallax_deg, distance_thresh=distance_thresh,
+                                           refine_iters=refine_iters, want_mask=want_mask)
+
+    @torch.no_grad()
+    def track_and_map(self, frame_pairs, pairs, scores, counts, point_maps, camera, **kw):
+        """One step of sequence tracking with map growth for the lists match_pairs / match_spacings returned
+        for ``frame_pairs`` (a, b): point_maps (P, Ka, 3) as for track_poses.  The pose of frame b by RANSAC
+        P3P against the points of frame a, then the next point maps (P, Kb, 3) of frame b: the PnP inliers'
+        points carried over, and points triangulated under that pose for the keypoints that have none
+        (geometry.track_and_map, whose keyword arguments ``kw`` takes).  Returns (R (P,3,3), t (P,3), pairs,
+        scores, counts, next point maps); a list without a model has R, t all zeros, an empty list and an
+        all-NaN map."""
+        kp = self._pixel_keypoints()
+        return geometry.track_and_map(point_maps, kp, kp, pairs, scores, counts, camera, self.pair_index(frame_pairs),
+                                      **kw)
 
 
 class TrackingCounters:

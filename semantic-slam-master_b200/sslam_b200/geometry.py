@@ -9,7 +9,10 @@ Tracking chain — ``recover_pose_device(..., want_mask=True, want_points=True)`
 |t|); ``point_map`` moves its points onto the keypoints of the second frame; the next frame's lists from that
 frame then pair points with keypoints, and ``solve_pnp_device`` gives that frame's pose in the same units,
 so chained poses share one scale (``rows_with_points`` first drops the rows without a point).  ``point_map``
-with the PnP's mask and (R, t) carries the points on.
+with the PnP's mask and (R, t) carries the points on.  Carrying alone loses points at every frame (a point
+survives only while its keypoint stays a PnP inlier), so ``track_and_map`` also triangulates every row of the
+step's lists under the PnP pose (``triangulate_device``, csrc/triangulate.cu) and fills the keypoints that
+have no carried point with the new points: one batched step of a sequence, in the map's units.
 
 Device API — ``verify_homography_device`` / ``verify_fundamental_device`` take banks of keypoint sets and
 the padded lists the matcher produced (``pairs [P,N,2]``, ``pair_scores [P,N]``, ``counts [P]``) and
@@ -24,6 +27,8 @@ of ``cv2.findFundamentalMat(pts1, pts2, cv2.FM_RANSAC, thresh)``; ``recover_pose
 ``cv2.recoverPose(E, pts1, pts2, K, distanceThresh)``; ``solve_pnp_ransac`` those of
 ``cv2.solvePnPRansac(X, uv, K, None, flags=cv2.SOLVEPNP_P3P)``.
 """
+
+import math
 
 import numpy as np
 import torch
@@ -186,6 +191,22 @@ def solve_pnp_device(points, kpts, pairs, scores, counts, camera, pair_index=Non
                           want_mask=want_mask, workspace=workspace)
 
 
+def triangulate_device(kpts1, kpts2, pairs, scores, counts, R, t, camera, pair_index=None, threshold=3.0,
+                       min_parallax_deg=1.0, distance_thresh=50.0, refine_iters=10, want_mask=False):
+    """The 3-D point of every row of the lists under a known relative pose per list (x2 ~ R x1 + t, R (P,3,3),
+    t (P,3), e.g. solve_pnp_device's), in the units of t: midpoint of the rays, then refine_iters
+    Levenberg-Marquardt trials on the pixel error in both views.  A row is kept iff its rays are not parallel,
+    its point lies in front of both cameras closer than distance_thresh, the angle between its two rays is at
+    least min_parallax_deg and its reprojection error is below threshold px in both views.  camera: (fx, fy,
+    cx, cy) or a 3x3 matrix, shared by both images.  -> ops.triangulate's (points (P,L,3) fp32 in the
+    camera-1 frame, zero where not kept, kept pairs, scores, counts[, mask (P,L)]) on device.  A list whose
+    R is all zero (no model) or not finite keeps no row."""
+    fx, fy, cx, cy = _intrinsics(camera)
+    return ops.triangulate(kpts1, kpts2, pairs, scores, counts, R, t, fx, fy, cx, cy, pair_index=pair_index,
+                           threshold=threshold, max_parallax_cos=math.cos(math.radians(min_parallax_deg)),
+                           distance_thresh=distance_thresh, refine_iters=refine_iters, want_mask=want_mask)
+
+
 def _log_so3(R):
     """Rotation matrix -> axis-angle vector (3,) (NumPy; the angle in [0, pi])."""
     c = np.clip((np.trace(R) - 1.0) / 2.0, -1.0, 1.0)
@@ -237,14 +258,16 @@ def solve_pnp_ransac(object_points, image_points, camera_matrix, dist_coeffs=Non
     return True, _log_so3(R).reshape(3, 1), t.reshape(3, 1), inl
 
 
-def point_map(pairs, counts, points, mask, num_keypoints, R=None, t=None):
+def point_map(pairs, counts, points, mask, num_keypoints, R=None, t=None, into=None):
     """Carry one step's 3-D points to the keypoints of the next: for list p, every row k < counts[p] with
     mask[p, k] set and 0 <= j = pairs[p, k, 1] < num_keypoints gives map[p, j] = R[p] points[p, k] + t[p]
     (points[p, k] without R, t).  A keypoint in several such rows takes the lowest row (a scatter-min of row
     indices: deterministic).  -> (P, num_keypoints, 3) fp32 on device, NaN where a keypoint has no point.
+    With ``into`` (P, num_keypoints, 3), its finite entries are kept and the rows fill only the others.
     pairs (P,L,2), counts (P,), points (P,L,3) and mask (P,L) index the same rows — for recover_pose_device,
     its input lists with want_mask / want_points; for solve_pnp_device, its input lists with its mask and
-    its (R, t).  Device-only, no synchronisation, capturable in a CUDA graph."""
+    its (R, t); for triangulate_device, its input lists with its mask and points and the (R, t) it was given.
+    Device-only, no synchronisation, capturable in a CUDA graph."""
     P, L = pairs.shape[0], pairs.shape[1]
     K = int(num_keypoints)
     dev = pairs.device
@@ -257,12 +280,17 @@ def point_map(pairs, counts, points, mask, num_keypoints, R=None, t=None):
     first = first[:, :K]
     has = first < L
     if L == 0:
-        return torch.full((P, K, 3), float("nan"), dtype=torch.float32, device=dev)
-    X = points.to(torch.float64).gather(1, first.clamp(max=L - 1)[..., None].expand(P, K, 3))
-    if R is not None:
-        X = torch.einsum("pij,pkj->pki", R.to(torch.float64).reshape(P, 3, 3), X) + \
-            t.to(torch.float64).reshape(P, 1, 3)
-    return torch.where(has[..., None], X, torch.full_like(X, float("nan"))).to(torch.float32)
+        out = torch.full((P, K, 3), float("nan"), dtype=torch.float32, device=dev)
+    else:
+        X = points.to(torch.float64).gather(1, first.clamp(max=L - 1)[..., None].expand(P, K, 3))
+        if R is not None:
+            X = torch.einsum("pij,pkj->pki", R.to(torch.float64).reshape(P, 3, 3), X) + \
+                t.to(torch.float64).reshape(P, 1, 3)
+        out = torch.where(has[..., None], X, torch.full_like(X, float("nan"))).to(torch.float32)
+    if into is None:
+        return out
+    into = into.to(torch.float32)
+    return torch.where(torch.isfinite(into).all(-1, keepdim=True), into, out)
 
 
 def rows_with_points(pairs, scores, counts, point_maps):
@@ -285,3 +313,39 @@ def rows_with_points(pairs, scores, counts, point_maps):
     sc = torch.zeros(P, L + 1, dtype=torch.float32, device=dev)
     sc.scatter_(1, pos, scores.to(torch.float32))
     return rows[:, :L].contiguous(), sc[:, :L].contiguous(), keep.sum(1).to(torch.int32)
+
+
+def track_and_map(point_maps, kpts_a, kpts_b, pairs, scores, counts, camera, pair_index, threshold=3.0, iters=1024,
+                  seed=0, refine_iters=10, min_parallax_deg=1.0, distance_thresh=50.0, tri_refine_iters=10):
+    """One batched step of sequence tracking with map growth.  List p pairs keypoints i of frame a with
+    keypoints j of frame b, (a, b) = pair_index[p] into the banks kpts_a (Fa,Ka,2) and kpts_b (Fb,Kb,2);
+    point_maps (P,Ka,3) holds the 3-D point of each keypoint of list p's frame a (NaN where there is none).
+
+      1. rows_with_points, then solve_pnp_device: the pose (R, t) of frame b in the map's units;
+      2. the PnP inliers' points are carried onto frame b's keypoints with (R, t) (point_map);
+      3. every row of the input lists is triangulated under (R, t) (triangulate_device);
+      4. the new points fill the keypoints of frame b that have no carried point (point_map(into=...)).
+
+    threshold (px) is the PnP's inlier threshold and the triangulation's reprojection gate; iters, seed and
+    refine_iters go to the PnP, min_parallax_deg, distance_thresh and tri_refine_iters to the triangulation.
+    -> (R (P,3,3), t (P,3), PnP pairs, scores, counts, next point maps (P,Kb,3) fp32) on device.  A list
+    without a PnP model has R, t all zeros and an all-NaN next map.  No synchronisation, capturable in a CUDA
+    graph."""
+    maps = point_maps.to(torch.float32).contiguous()
+    P, Kb = pairs.shape[0], kpts_b.shape[1]
+    dev = pairs.device
+    rows, sc, n = rows_with_points(pairs, scores, counts, maps)
+    idx = pair_index.to(torch.int32)
+    pnp_idx = torch.stack([torch.arange(P, dtype=torch.int32, device=dev), idx[:, 1]], 1)
+    R, t, pp, ps, pc, _, mask = solve_pnp_device(maps, kpts_b, rows, sc, n, camera, pair_index=pnp_idx,
+                                                 threshold=threshold, iters=iters, seed=seed,
+                                                 refine_iters=refine_iters, want_mask=True)
+    Na = maps.shape[1]
+    X = maps.gather(1, rows[..., 0].to(torch.int64).clamp(0, max(Na - 1, 0))[..., None].expand(P, -1, 3)) \
+        if Na else torch.zeros(P, rows.shape[1], 3, device=dev)
+    carried = point_map(rows, n, X, mask, Kb, R, t)
+    pts, _, _, _, tmask = triangulate_device(kpts_a, kpts_b, pairs, scores, counts, R, t, camera, pair_index=idx,
+                                             threshold=threshold, min_parallax_deg=min_parallax_deg,
+                                             distance_thresh=distance_thresh, refine_iters=tri_refine_iters,
+                                             want_mask=True)
+    return R, t, pp, ps, pc, point_map(pairs, counts, pts, tmask, Kb, R, t, into=carried)

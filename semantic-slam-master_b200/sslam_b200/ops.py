@@ -2,6 +2,7 @@
 work is enqueued on torch's current stream; nothing here synchronises."""
 
 import ctypes
+import math
 
 import torch
 
@@ -529,6 +530,41 @@ def ransac_pnp(points, kpts2, pairs, pair_scores, counts, fx, fy, cx, cy, pair_i
                                     _ptr(t), _ptr(rms), _ptr(out_pairs), _ptr(out_scores), _ptr(out_counts),
                                     _ptr(mask), _ptr(ws), ws.numel(), _stream()))
     return (R, t, out_pairs, out_scores, out_counts, rms) + ((mask,) if want_mask else ())
+
+
+def triangulate(kpts1, kpts2, pairs, pair_scores, counts, R, t, fx, fy, cx, cy, pair_index=None, num_pairs=None,
+                threshold=3.0, max_parallax_cos=math.cos(math.radians(1.0)), distance_thresh=50.0, refine_iters=10,
+                want_mask=False):
+    """Triangulation of every row of P match lists under a known relative pose per list (sslam_triangulate).
+
+    kpts1 (F1,N,2), kpts2 (F2,M,2) fp32, pairs (P,L,2) int32, pair_scores (P,L), counts (P,) and pair_index
+    as for recover_pose; R (P,3,3) or (P,9) and t (P,3) float64 with x2 ~ R x1 + t (R all zero: no pose);
+    one pinhole camera (fx, fy, cx, cy) for both images.  A row is kept iff its rays are not parallel, its
+    refined point lies at depths in (0, distance_thresh) in both cameras, the cosine of its parallax angle
+    is <= max_parallax_cos (default: cos 1 deg) and its squared reprojection error is < threshold^2 in both
+    views.  Returns (points (P,L,3) fp32 in the camera-1 frame, in the units of t, zero where a row is not
+    kept; kept pairs (P,L,2) int32 in input order -1 padded, their scores (P,L), counts (P,) int32[, mask
+    (P,L) uint8])."""
+    lib = _lib.load()
+    _need_cuda(R, t)
+    k1, k2, pr, ps, cn, pair_index, F1, N, F2, M, P, L = _match_lists("triangulate", kpts1, kpts2, pairs,
+                                                                      pair_scores, counts, pair_index, num_pairs)
+    Rd = R.to(torch.float64).reshape(-1, 9).contiguous()
+    td = t.to(torch.float64).reshape(-1, 3).contiguous()
+    if Rd.shape[0] != P or td.shape[0] != P:
+        raise RuntimeError("triangulate: R and t must hold one pose per match list")
+    dev = pr.device
+    points = torch.empty(P, L, 3, dtype=torch.float32, device=dev)
+    out_pairs = torch.empty(P, L, 2, dtype=torch.int32, device=dev)
+    out_scores = torch.empty(P, L, dtype=torch.float32, device=dev)
+    out_counts = torch.empty(P, dtype=torch.int32, device=dev)
+    mask = torch.empty(P, L, dtype=torch.uint8, device=dev) if want_mask else None
+    _lib.check(lib.sslam_triangulate(_ptr(k1), F1, _ptr(k2), F2, _ptr(pair_index), P, N, M, _ptr(pr), _ptr(ps),
+                                     _ptr(cn), L, _ptr(Rd), _ptr(td), float(fx), float(fy), float(cx), float(cy),
+                                     float(threshold), float(max_parallax_cos), float(distance_thresh),
+                                     int(refine_iters), _ptr(points), _ptr(out_pairs), _ptr(out_scores),
+                                     _ptr(out_counts), _ptr(mask), _stream()))
+    return (points, out_pairs, out_scores, out_counts) + ((mask,) if want_mask else ())
 
 
 # ---------------------------------------------------------------------------------- optional decode front stage (J1)
