@@ -450,6 +450,43 @@ int sslam_triangulate(const float* kpts1, int F1, const float* kpts2, int F2, co
                       float* out_scores, int32_t* out_counts, uint8_t* mask, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
+ * Sliding-window bundle adjustment: for each of P windows of W posed frames, the poses of the last
+ * W - fixed frames and the points of the window's tracks are refined jointly on the pixel error of every
+ * observation, in one launch (one CTA per window), without host synchronisation (capturable in a CUDA
+ * graph), without atomics; a window's result does not depend on its position in the batch.
+ *   kpts [F,K,2] fp32 pixel bank; frame_index [P,W] int32 slot of each window frame; obs [P,N,W] int32
+ *   keypoint of track n in window frame w (-1: none); points [P,N,3] fp32 track points in the world frame;
+ *   counts [P] int32 tracks per window; R [P,W,9] row-major, t [P,W,3] double, x_w ~ R_w X + t_w; one
+ *   pinhole camera.  The first `fixed` frames of every window are held (2 pins the monocular scale).
+ *   Used set, fixed at the start: observation (n, w) is used when its slot and keypoint index are in range,
+ *   its keypoint and the point are finite and the depth is > 0; a track is used when n < counts[p] and it
+ *   has at least 2 such observations.  Cost: sum of rho(|r|^2) over used observations, r = pi(R_w X + t_w)
+ *   - x, rho Huber with threshold `huber` px (inf: least squares), IRLS weight min(1, huber / |r|) at the
+ *   linearisation point.  Levenberg-Marquardt (R_w <- Exp(w) R_w, t_w <- t_w + d, X <- X + dX), damping
+ *   H_ii (1 + lambda), lambda0 = 1e-3 mean diag(J^T W J) over all free parameters, /10 on an accepted
+ *   trial, x10 otherwise; each trial solves the Schur complement on the poses by a dense Cholesky (not
+ *   positive definite or a step that is not finite: rejected) and back-substitutes per track; a candidate
+ *   with a used observation at depth <= 0 is rejected, a strictly lower cost accepted.  All arithmetic is
+ *   double and correctly rounded except Rodrigues' sin / cos; sums run in ascending track, then frame order.
+ *   Outputs: R_out, t_out (held frames copied bit for bit); points_out [P,N,3] fp32 (refined for used
+ *   tracks, copied otherwise); rms [P,2] double, the RMS pixel error over the used observations before /
+ *   after; accepted [P] int32 accepted trials (may be NULL); mask [P,N,W] uint8, used and squared error
+ *   < threshold^2 at the end (may be NULL).  A window with a pose that is not finite or an all-zero R, or
+ *   without a used track, is returned unchanged with zero rms, accepted and mask.
+ *   The workspace (sslam_bundle_adjust_workspace_bytes) holds 49 bytes per track and window.
+ * Limits: 2 <= W <= 8 (SSLAM_EUNSUPPORTED above), 1 <= fixed <= W, N <= 65536 (SSLAM_EUNSUPPORTED
+ * above), 0 <= refine_iters <= 100, huber > 0, threshold > 0 and finite, fx, fy > 0 and finite, cx, cy
+ * finite.
+ */
+size_t sslam_bundle_adjust_workspace_bytes(int P, int N);
+int sslam_bundle_adjust(const float* kpts, int F, int K, const int32_t* frame_index, int P, int W, int N,
+                        const int32_t* obs, const float* points, const int32_t* counts, const double* R,
+                        const double* t, double fx, double fy, double cx, double cy, int fixed, double huber,
+                        double threshold, int refine_iters, double* R_out, double* t_out, float* points_out,
+                        double* rms, int32_t* accepted, uint8_t* mask, void* ws, size_t ws_bytes,
+                        void* stream);
+
+/* ---------------------------------------------------------------------------------------------
  * Optional cell-softmax front stage of the decode (north_star "softmax/depth-to-space ... border
  * mask"; OFF by default — the reference code has no such mode, keypoint_selector.py:61-62 is a
  * sigmoid; the vocabulary is papers/pdfs/SuperPoint_DeTone.md:49-58):

@@ -59,7 +59,7 @@ enum KernelKind {
   KK_DECODE_SCAN = 0, KK_DECODE_TOPK, KK_DECODE_COUNT, KK_DECODE_RESOLVE, KK_NMS, KK_GATHER, KK_L2NORM,
   KK_MATCH_F32, KK_MATCH_TC, KK_SPLIT, KK_UNPACK, KK_FINALIZE, KK_GEMM, KK_LAYERNORM, KK_EVAL, KK_HEATMAP,
   KK_CONV_HEAD, KK_RANSAC_HYP, KK_RANSAC_SCORE, KK_RANSAC_REFIT, KK_POSE,
-  KK_PNP_HYP, KK_PNP_SCORE, KK_PNP_REFIT, KK_TRIANGULATE, KK_COUNT
+  KK_PNP_HYP, KK_PNP_SCORE, KK_PNP_REFIT, KK_TRIANGULATE, KK_BUNDLE_ADJUST, KK_COUNT
 };
 extern std::atomic<int> g_profile_on;
 void prof_mark(int kind, cudaStream_t stream, bool begin);

@@ -81,6 +81,12 @@ SIGNATURES = {
                                   ctypes.c_double, ctypes.c_double, ctypes.c_double, ctypes.c_double,
                                   ctypes.c_double, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                   c_void_p]),
+    "sslam_bundle_adjust_workspace_bytes": (c_size_t, [c_int, c_int]),
+    "sslam_bundle_adjust": (c_int, [c_void_p, c_int, c_int, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p,
+                                    c_void_p, c_void_p, c_void_p, ctypes.c_double, ctypes.c_double, ctypes.c_double,
+                                    ctypes.c_double, c_int, ctypes.c_double, ctypes.c_double, c_int, c_void_p,
+                                    c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t,
+                                    c_void_p]),
 }
 
 # include/sslam_b200_debug.h (tools only)

@@ -210,6 +210,20 @@ class FrameStore:
         return geometry.track_and_map(point_maps, kp, kp, pairs, scores, counts, camera, self.pair_index(frame_pairs),
                                       **kw)
 
+    @torch.no_grad()
+    def bundle_adjust(self, windows, obs, points, counts, R, t, camera, **kw):
+        """Sliding-window bundle adjustment on the resident keypoints: ``windows`` holds P lists of W resident
+        frame ids; obs (P,N,W), points (P,N,3), counts (P,) as geometry.window_tracks returns them, R (P,W,3,3),
+        t (P,W,3) the frames' absolute poses.  -> geometry.bundle_adjust_device's (R, t, points, rms,
+        accepted[, mask]), whose keyword arguments ``kw`` takes."""
+        for frames in windows:
+            for f in frames:
+                if not self.holds(f):
+                    raise KeyError(f"window frame {f} is not resident")
+        kp = self._pixel_keypoints()
+        fi = torch.tensor([[self.slot_of(f) for f in frames] for frames in windows], dtype=torch.int32)
+        return geometry.bundle_adjust_device(kp, fi.to(kp.device), obs, points, counts, R, t, camera, **kw)
+
 
 class TrackingCounters:
     """Device-side accumulators of TrackingTester.track_frame_sequence (test/test_tracking.py:139-199):

@@ -258,6 +258,20 @@ def solve_pnp_ransac(object_points, image_points, camera_matrix, dist_coeffs=Non
     return True, _log_so3(R).reshape(3, 1), t.reshape(3, 1), inl
 
 
+def _first_row(pairs, counts, mask, K):
+    """The lowest row k < counts[p] with mask[p, k] set and 0 <= j = pairs[p, k, 1] < K of each keypoint j of
+    list p, by a scatter-min of row indices (deterministic) -> (P, K) int64, L where there is none."""
+    P, L = pairs.shape[0], pairs.shape[1]
+    dev = pairs.device
+    k = torch.arange(L, device=dev)
+    j = pairs[..., 1].to(torch.int64)
+    keep = (k[None] < counts.to(torch.int64)[:, None]) & mask.to(torch.bool) & (j >= 0) & (j < K)
+    col = torch.where(keep, j, torch.full_like(j, K))             # dropped rows go to a spare column
+    first = torch.full((P, K + 1), L, dtype=torch.int64, device=dev)
+    first.scatter_reduce_(1, col, k[None].expand(P, L), reduce="amin", include_self=True)
+    return first[:, :K]
+
+
 def point_map(pairs, counts, points, mask, num_keypoints, R=None, t=None, into=None):
     """Carry one step's 3-D points to the keypoints of the next: for list p, every row k < counts[p] with
     mask[p, k] set and 0 <= j = pairs[p, k, 1] < num_keypoints gives map[p, j] = R[p] points[p, k] + t[p]
@@ -271,13 +285,7 @@ def point_map(pairs, counts, points, mask, num_keypoints, R=None, t=None, into=N
     P, L = pairs.shape[0], pairs.shape[1]
     K = int(num_keypoints)
     dev = pairs.device
-    k = torch.arange(L, device=dev)
-    j = pairs[..., 1].to(torch.int64)
-    keep = (k[None] < counts.to(torch.int64)[:, None]) & mask.to(torch.bool) & (j >= 0) & (j < K)
-    col = torch.where(keep, j, torch.full_like(j, K))             # dropped rows go to a spare column
-    first = torch.full((P, K + 1), L, dtype=torch.int64, device=dev)
-    first.scatter_reduce_(1, col, k[None].expand(P, L), reduce="amin", include_self=True)
-    first = first[:, :K]
+    first = _first_row(pairs, counts, mask, K)
     has = first < L
     if L == 0:
         out = torch.full((P, K, 3), float("nan"), dtype=torch.float32, device=dev)
@@ -316,7 +324,8 @@ def rows_with_points(pairs, scores, counts, point_maps):
 
 
 def track_and_map(point_maps, kpts_a, kpts_b, pairs, scores, counts, camera, pair_index, threshold=3.0, iters=1024,
-                  seed=0, refine_iters=10, min_parallax_deg=1.0, distance_thresh=50.0, tri_refine_iters=10):
+                  seed=0, refine_iters=10, min_parallax_deg=1.0, distance_thresh=50.0, tri_refine_iters=10,
+                  want_links=False):
     """One batched step of sequence tracking with map growth.  List p pairs keypoints i of frame a with
     keypoints j of frame b, (a, b) = pair_index[p] into the banks kpts_a (Fa,Ka,2) and kpts_b (Fb,Kb,2);
     point_maps (P,Ka,3) holds the 3-D point of each keypoint of list p's frame a (NaN where there is none).
@@ -330,7 +339,13 @@ def track_and_map(point_maps, kpts_a, kpts_b, pairs, scores, counts, camera, pai
     refine_iters go to the PnP, min_parallax_deg, distance_thresh and tri_refine_iters to the triangulation.
     -> (R (P,3,3), t (P,3), PnP pairs, scores, counts, next point maps (P,Kb,3) fp32) on device.  A list
     without a PnP model has R, t all zeros and an all-NaN next map.  No synchronisation, capturable in a CUDA
-    graph."""
+    graph.
+
+    With ``want_links`` also (link (P,Kb) int32, born (P,Kb) bool), the provenance window_tracks chains into
+    multi-frame tracks: for each keypoint j of frame b with a point, link[j] is the keypoint i of frame a of
+    the row that gave j its point — the lowest PnP-inlier row with that j when the point was carried (born
+    0), the lowest kept triangulation row with that j when it was triangulated (born 1); -1 and 0 where j
+    has no point."""
     maps = point_maps.to(torch.float32).contiguous()
     P, Kb = pairs.shape[0], kpts_b.shape[1]
     dev = pairs.device
@@ -348,4 +363,111 @@ def track_and_map(point_maps, kpts_a, kpts_b, pairs, scores, counts, camera, pai
                                              threshold=threshold, min_parallax_deg=min_parallax_deg,
                                              distance_thresh=distance_thresh, refine_iters=tri_refine_iters,
                                              want_mask=True)
-    return R, t, pp, ps, pc, point_map(pairs, counts, pts, tmask, Kb, R, t, into=carried)
+    nxt = point_map(pairs, counts, pts, tmask, Kb, R, t, into=carried)
+    if not want_links:
+        return R, t, pp, ps, pc, nxt
+    fc = _first_row(rows, n, mask, Kb)
+    ft = _first_row(pairs, counts, tmask, Kb)
+    L = pairs.shape[1]
+    has_c, has_t = fc < L, ft < L
+    ic = rows[..., 0].to(torch.int64).gather(1, fc.clamp(max=max(L - 1, 0))) if L else fc
+    it = pairs[..., 0].to(torch.int64).gather(1, ft.clamp(max=max(L - 1, 0))) if L else ft
+    fin = torch.isfinite(nxt).all(-1)
+    link = torch.where(fin & has_c, ic, torch.where(fin & has_t, it, torch.full_like(ic, -1)))
+    return R, t, pp, ps, pc, nxt, link.to(torch.int32), fin & ~has_c & has_t
+
+
+def window_tracks(maps, links, born, R, t):
+    """Multi-frame tracks of a window of W frames from the provenance of its W-1 tracking steps.
+
+    maps (P,W,K,3) point map of each window frame (NaN where a keypoint has none); links, born (P,W-1,K)
+    track_and_map's link / born of the step into frame w (index w-1); R (P,W,3,3), t (P,W,3) absolute poses,
+    x_w ~ R_w X + t_w, in any world frame.  Every keypoint of frame 0 with a point roots a track; a keypoint
+    j of frame w >= 1 with a point inherits the track of keypoint link[j] of frame w-1 when it is not born
+    and that keypoint has a track, and roots a new track at (w, j) otherwise.  A born track also observes
+    (w-1, link[j]) when that keypoint has no track (the lowest such j claims it).  A track observes at most
+    one keypoint per frame, the lowest j.  Its point is R_w^T (M_w[j] - t_w) of its root (w, j), in double.
+    -> (obs (P,N,W) int32 keypoint of track n in frame w, -1 none; points (P,N,3) fp32 world, NaN padded;
+    counts (P,) int32; track_of (P,W,K) int32, -1 none), N = W*K, tracks in ascending root order (w-major,
+    then j).  Device-only, no synchronisation, capturable in a CUDA graph."""
+    P, W, K = maps.shape[0], maps.shape[1], maps.shape[2]
+    N = W * K
+    dev = maps.device
+    fin = torch.isfinite(maps).all(-1)
+    j = torch.arange(K, device=dev)[None].expand(P, K)
+    none = torch.full((P, K), -1, dtype=torch.int64, device=dev)
+    rid, claims = [torch.where(fin[:, 0], j, none)], [none]      # root (w*K + j) of each keypoint's track
+    for w in range(1, W):
+        lk = links[:, w - 1].to(torch.int64)
+        bn = born[:, w - 1].to(torch.bool)
+        ok = (lk >= 0) & (lk < K)
+        lc = lk.clamp(0, K - 1)
+        prev = rid[w - 1].gather(1, lc)
+        inherit = fin[:, w] & ~bn & ok & (prev >= 0)
+        rid.append(torch.where(inherit, prev, torch.where(fin[:, w], w * K + j, none)))
+        cand = fin[:, w] & bn & ok & (prev < 0)
+        first = torch.full((P, K + 1), K, dtype=torch.int64, device=dev)
+        first.scatter_reduce_(1, torch.where(cand, lc, K), j, reduce="amin", include_self=True)
+        claims.append(torch.where(cand & (first.gather(1, lc) == j), lk, none))
+    rid = torch.stack(rid, 1).reshape(P, N)
+    flat = torch.arange(N, device=dev)[None]
+    is_root = rid == flat
+    pos = is_root.to(torch.int64).cumsum(1) - 1
+    track_of = torch.where(rid >= 0, pos.gather(1, rid.clamp(min=0)), -1).reshape(P, W, K)
+    counts = is_root.sum(1).to(torch.int32)
+    obs = []
+    for w in range(W):
+        tw = track_of[:, w]
+        m = torch.full((P, N + 1), K, dtype=torch.int64, device=dev)
+        m.scatter_reduce_(1, torch.where(tw >= 0, tw, N), j, reduce="amin", include_self=True)
+        obs.append(torch.where(m[:, :N] < K, m[:, :N], -1))
+    for w in range(1, W):                                           # born tracks claim (w-1, link)
+        cl = claims[w]
+        tgt = torch.full((P, N + 1), -1, dtype=torch.int64, device=dev)
+        tgt.scatter_(1, torch.where(cl >= 0, track_of[:, w], N), cl)
+        obs[w - 1] = torch.where(tgt[:, :N] >= 0, tgt[:, :N], obs[w - 1])
+    obs = torch.stack(obs, 2).to(torch.int32)
+    Rd = R.to(torch.float64).reshape(P, W, 3, 3)
+    X = torch.einsum("pwji,pwkj->pwki", Rd, maps.to(torch.float64) - t.to(torch.float64).reshape(P, W, 1, 3))
+    pts = torch.full((P, N + 1, 3), float("nan"), dtype=torch.float32, device=dev)
+    pts.scatter_(1, torch.where(is_root, pos, N)[..., None].expand(P, N, 3), X.reshape(P, N, 3).to(torch.float32))
+    return obs.contiguous(), pts[:, :N].contiguous(), counts, track_of.to(torch.int32).contiguous()
+
+
+def window_map(track_of, points, R, t, obs=None, mask=None):
+    """The point maps (P,W,K,3) fp32 of the window frames from the tracks' points (P,N,3) (usually refined by
+    bundle_adjust_device): M_w[j] = R_w X + t_w in double for the track of (w, j) (window_tracks' track_of),
+    NaN where there is none.  With bundle_adjust_device's ``mask`` (P,N,W) and the ``obs`` it was given, a
+    keypoint that is an observation of a track with at least two observations and whose mask entry is 0
+    (an outlier, or not used) gets NaN; tracks of a single observation cannot be judged and keep their
+    points.  The newest frame's slice feeds the next track_and_map.  Device-only, capturable."""
+    P, W, K = track_of.shape
+    N = points.shape[1]
+    dev = track_of.device
+    tr = track_of.to(torch.int64)
+    keep = tr >= 0
+    X = points.to(torch.float64).gather(1, tr.clamp(0, max(N - 1, 0)).reshape(P, W * K, 1).expand(P, W * K, 3))
+    M = torch.einsum("pwij,pwkj->pwki", R.to(torch.float64).reshape(P, W, 3, 3), X.reshape(P, W, K, 3)) + \
+        t.to(torch.float64).reshape(P, W, 1, 3)
+    if mask is not None:
+        ob = obs.to(torch.int64)
+        seen = ob >= 0
+        bad = seen & (mask == 0) & (seen.sum(2, keepdim=True) >= 2)
+        drop = torch.zeros(P, W, K + 1, dtype=torch.bool, device=dev)
+        drop.scatter_(2, torch.where(bad, ob, K).permute(0, 2, 1), True)
+        keep = keep & ~drop[..., :K]
+    return torch.where(keep[..., None], M, torch.full_like(M, float("nan"))).to(torch.float32)
+
+
+def bundle_adjust_device(kpts, frame_index, obs, points, counts, R, t, camera, fixed=2, huber=3.0, threshold=3.0,
+                         refine_iters=10, want_mask=False):
+    """Sliding-window bundle adjustment (csrc/bundle_adjust.cu) of P windows: the poses of the last W - fixed
+    frames and the tracks' points refined jointly on the pixel error of every observation, Huber-robust at
+    ``huber`` px (inf: least squares), by Levenberg-Marquardt on the Schur complement.  kpts (F,K,2) pixel
+    bank, frame_index (P,W) its slots, obs / points / counts as window_tracks returns them, R (P,W,3,3), t
+    (P,W,3) absolute poses; camera (fx, fy, cx, cy) or a 3x3 matrix.  The default fixed = 2 pins the
+    monocular scale.  -> ops.bundle_adjust's (R, t, points, rms (P,2), accepted (P,)[, mask (P,N,W)]) on
+    device."""
+    fx, fy, cx, cy = _intrinsics(camera)
+    return ops.bundle_adjust(kpts, frame_index, obs, points, counts, R, t, fx, fy, cx, cy, fixed=fixed, huber=huber,
+                             threshold=threshold, refine_iters=refine_iters, want_mask=want_mask)

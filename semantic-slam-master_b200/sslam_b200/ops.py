@@ -567,6 +567,61 @@ def triangulate(kpts1, kpts2, pairs, pair_scores, counts, R, t, fx, fy, cx, cy, 
     return (points, out_pairs, out_scores, out_counts) + ((mask,) if want_mask else ())
 
 
+
+def bundle_adjust_workspace_bytes(P, N):
+    """Workspace bytes bundle_adjust needs for P windows of N tracks."""
+    return int(_lib.load().sslam_bundle_adjust_workspace_bytes(int(P), int(N)))
+
+
+def bundle_adjust(kpts, frame_index, obs, points, counts, R, t, fx, fy, cx, cy, fixed=2, huber=3.0, threshold=3.0,
+                  refine_iters=10, want_mask=False, workspace=None):
+    """Sliding-window bundle adjustment of P windows of W frames (sslam_bundle_adjust).
+
+    kpts (F,K,2) fp32 pixel bank; frame_index (P,W) slot of each window frame; obs (P,N,W) keypoint of track n
+    in frame w (-1: none), points (P,N,3) fp32 in the world frame, counts (P,) tracks per window (usually
+    geometry.window_tracks'); R (P,W,3,3) or (P,W,9), t (P,W,3) float64 absolute poses, x_w ~ R_w X + t_w; one
+    pinhole camera.  The first ``fixed`` frames are held; ``huber`` px is the robust threshold (inf: least
+    squares), ``threshold`` px the inlier test of the mask.  2 <= W <= 8, N <= 65536.
+    Returns (R (P,W,3,3), t (P,W,3) float64, points (P,N,3) fp32, rms (P,2) float64 — RMS pixel error over the
+    used observations before / after —, accepted (P,) int32 trials[, mask (P,N,W) uint8 — used and below
+    threshold at the end]).  A window without a model (a pose not finite or an all-zero R) or without a used
+    track comes back unchanged with zero rms."""
+    lib = _lib.load()
+    _need_cuda(kpts, frame_index, obs, points, counts, R, t)
+    kp = kpts.contiguous()
+    if kp.dtype != torch.float32 or kp.dim() != 3 or kp.shape[-1] != 2:
+        raise RuntimeError("bundle_adjust expects fp32 keypoints (F,K,2)")
+    if points.dtype != torch.float32 or points.dim() != 3 or points.shape[-1] != 3:
+        raise RuntimeError("bundle_adjust expects fp32 points (P,N,3)")
+    fi = frame_index.to(torch.int32).contiguous()
+    ob = obs.to(torch.int32).contiguous()
+    X = points.contiguous()
+    cn = counts.to(torch.int32).contiguous()
+    if fi.dim() != 2 or ob.dim() != 3:
+        raise RuntimeError("bundle_adjust expects frame_index (P,W) and obs (P,N,W)")
+    P, W = fi.shape
+    N = ob.shape[1]
+    Rd = R.to(torch.float64).reshape(P, W, 9).contiguous() if R.numel() == P * W * 9 else None
+    td = t.to(torch.float64).reshape(P, W, 3).contiguous() if t.numel() == P * W * 3 else None
+    if ob.shape != (P, N, W) or X.shape != (P, N, 3) or cn.shape != (P,) or Rd is None or td is None:
+        raise RuntimeError("bundle_adjust: frame_index (P,W), obs (P,N,W), points (P,N,3), counts (P,), "
+                           "R (P,W,3,3) and t (P,W,3) must agree")
+    dev = fi.device
+    R_out = torch.empty(P, W, 3, 3, dtype=torch.float64, device=dev)
+    t_out = torch.empty(P, W, 3, dtype=torch.float64, device=dev)
+    X_out = torch.empty(P, N, 3, dtype=torch.float32, device=dev)
+    rms = torch.empty(P, 2, dtype=torch.float64, device=dev)
+    acc = torch.empty(P, dtype=torch.int32, device=dev)
+    mask = torch.empty(P, N, W, dtype=torch.uint8, device=dev) if want_mask else None
+    need = bundle_adjust_workspace_bytes(P, N)
+    ws = workspace if workspace is not None else _ws("bundle_adjust", need, dev)
+    _lib.check(lib.sslam_bundle_adjust(_ptr(kp), kp.shape[0], kp.shape[1], _ptr(fi), P, W, N, _ptr(ob), _ptr(X),
+                                       _ptr(cn), _ptr(Rd), _ptr(td), float(fx), float(fy), float(cx), float(cy),
+                                       int(fixed), float(huber), float(threshold), int(refine_iters), _ptr(R_out),
+                                       _ptr(t_out), _ptr(X_out), _ptr(rms), _ptr(acc), _ptr(mask), _ptr(ws),
+                                       ws.numel(), _stream()))
+    return (R_out, t_out, X_out, rms, acc) + ((mask,) if want_mask else ())
+
 # ---------------------------------------------------------------------------------- optional decode front stage (J1)
 def heatmap_from_cells(logits, cell=8, border=0):
     """(B, cell*cell+1, Hc, Wc) fp32 cell logits -> (B, Hc*cell, Wc*cell) heatmap: channel softmax,
